@@ -9,6 +9,8 @@
                                                 C3; the table is hash-sharded over the N GPUs
   python bench.py --impl reference ...          the CPU restatement of the reference path on this box's
                                                 host cores, same config, bounded sample
+  python bench.py ... --dump-outputs DIR        also write what the last timed step computed, as .npy
+                                                files (one GPU or the reference arm)
 
 A step = build the count table for the whole read set from scratch (clear, consume every read).
 One JSON line (rank 0): `value` device-timed with the reads resident in HBM; `e2e` the same job
@@ -65,7 +67,12 @@ def parse_args():
     ap.add_argument("--round-mw", type=int, default=256, help="sharded table: Mi windows per round of a device-resident batch "
                     "(the library's default is 64: see DESIGN.md section 6)")
     ap.add_argument("--table-hint", type=int, default=-1, help="expected distinct k-mers (-1: genome length for c2, none for c3)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64), see dump_outputs()")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def workload(a, world: int) -> dict:
@@ -161,6 +168,26 @@ def measured_traffic(name: str):
         return None
 
 
+DUMP_PAIRS = 1 << 20  # (hash, count) pairs --dump-outputs keeps: 24 MiB of float64
+
+
+def dump_outputs(out_dir: str, keys: np.ndarray, vals: np.ndarray, histo: list, counted: int) -> None:
+    """What a caller of the timed path receives -- the k-mers counted, the (hash, count) table
+    sorted by hash, its histogram -- as float64 .npy files, so that two builds can be compared
+    output for output.  A table larger than DUMP_PAIRS is sampled at evenly spaced ranks; each
+    hash is split into 32-bit halves, which float64 holds exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(keys)
+    pick = np.arange(min(n, DUMP_PAIRS), dtype=np.int64) * n // max(min(n, DUMP_PAIRS), 1)
+    k, v = keys[pick], vals[pick]
+    freq, distinct = np.array(histo, dtype=np.uint64).reshape(-1, 2).T
+    arrays = {"kmers_counted": np.array([counted], dtype=np.uint64), "table_size": np.array([n], dtype=np.uint64),
+              "table_hash_hi32": k >> np.uint64(32), "table_hash_lo32": k & np.uint64(0xFFFFFFFF), "table_count": v,
+              "histo_count": freq, "histo_kmers": distinct}
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x.astype(np.float64))
+
+
 def alg_bytes_per_kmer(read_len: int, k: int, world: int = 1) -> float:
     # SURVEY.md 8(d): every base read once (1 B) + 16-B slot read + 8-B count write,
     # + remote 8-B write and read of the routed hash on (N-1)/N of the k-mers
@@ -195,6 +222,8 @@ def run_reference(a, rank: int, world: int):
         dt = time.perf_counter() - t0
         if i >= a.warmup:
             times.append(dt)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *t.items_sorted(), t.histo(zero=False), total)
     ms = 1e3 * float(np.mean(times))
     v = total / (ms / 1e3)
     sample = f"first {n} reads of the workload ({total} k-mers) per step, table rebuilt each step"
@@ -337,6 +366,8 @@ def run_single(a, local: int):
     value = counted / (ms_per_step / 1e3)
     distinct = len(table)
     cap = table.capacity
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *table.export(1), table.histo(), counted)
 
     # roofline of the dominant kernels: algorithmic bytes / their own duration, CUDA events on the
     # launch stream.  Partitioned pipeline: scatter_kernel + aggregate_kernel together do what
@@ -639,6 +670,8 @@ def main():
     if a.impl == "reference":
         return run_reference(a, rank, world)
     if world > 1:
+        if a.dump_outputs:
+            sys.exit("--dump-outputs: one GPU only (a sharded table's outputs are spread over the ranks)")
         return run_sharded(a, rank, world, local)
     return run_single(a, local)
 

@@ -66,8 +66,8 @@ def test_specialised_k_list_is_sane():
 
 
 def test_reference_suite_is_vendored_unmodified():
-    """tests/reference_suite holds the reference's own tests byte for byte (compared here, where
-    /root/reference exists; on the GPU box the comparison has nothing to compare with)."""
+    """tests/reference_suite holds the reference's own tests byte for byte (their SHA-256 against
+    tests/golden/reference_suite_sha256.json)."""
     import importlib.util
     import os
 
