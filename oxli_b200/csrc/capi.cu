@@ -112,20 +112,120 @@ static std::atomic<uint32_t> g_accumulate{(uint32_t)std::max(1, std::min(16, env
 static std::atomic<uint32_t> g_groups_override{(uint32_t)env_int("OXLI_B200_GROUPS", 0)};  // 0 = default
 constexpr int kStageBufs = 4;  // host batches: chunks in flight between the copy stream and the kernels
 
+// A host batch as the staging ring reads it: read boundaries offsets[0..n_reads] (positions in
+// `bases`; the batch's own positions count from offsets[0]) and whether `bases` is pinned.
+struct HostBatch {
+    const uint8_t *bases;
+    const uint64_t *offsets;
+    uint64_t n_reads;
+    bool pinned;
+};
+
+// Ring of kStageBufs staging buffers through which host batches reach the device: chunk ci goes
+// to buffer ci % kStageBufs.  A buffer holds the chunk's bases (through pinned memory when the
+// source is pageable) and its batch-relative read boundaries; ev_ready[b] marks its copies
+// landed, ev_free[b] (recorded by whoever launches the kernels) the kernels done reading it.
+struct StageRing {
+    cudaStream_t copy = nullptr;  // the H2D copies
+    uint8_t *d_bases[kStageBufs] = {}, *h_bases[kStageBufs] = {};
+    uint64_t d_cap[kStageBufs] = {}, h_cap[kStageBufs] = {};
+    uint64_t *d_offs[kStageBufs] = {}, *h_offs[kStageBufs] = {};
+    uint64_t offs_cap[kStageBufs] = {};
+    uint64_t n_off[kStageBufs] = {};  // boundaries of the chunk staged in buffer b, sentinel included
+    cudaEvent_t ev_ready[kStageBufs] = {}, ev_free[kStageBufs] = {};
+
+    oxg_status init() {
+        CU(cudaStreamCreateWithFlags(&copy, cudaStreamNonBlocking));
+        for (int b = 0; b < kStageBufs; ++b) {
+            CU(cudaEventCreateWithFlags(&ev_ready[b], cudaEventDisableTiming));
+            CU(cudaEventCreateWithFlags(&ev_free[b], cudaEventDisableTiming));
+        }
+        return OXG_OK;
+    }
+
+    void release() {
+        cudaStreamSynchronize(copy);
+        for (int b = 0; b < kStageBufs; ++b) {
+            cudaEventDestroy(ev_ready[b]); cudaEventDestroy(ev_free[b]);
+            cudaFree(d_bases[b]); cudaFreeHost(h_bases[b]); cudaFree(d_offs[b]); cudaFreeHost(h_offs[b]);
+        }
+        cudaStreamDestroy(copy);
+    }
+
+    // Buffers 0..n_bufs-1 take chunks of `bytes`.  A device buffer is replaced once `kernels` has
+    // drained, a pinned one (needed for pageable sources only) once the copy stream has.
+    oxg_status reserve(int n_bufs, uint64_t bytes, bool src_pinned, cudaStream_t kernels) {
+        for (int b = 0; b < n_bufs; ++b) {
+            if (d_cap[b] < bytes) {
+                CU(cudaStreamSynchronize(kernels));
+                if (d_bases[b]) CU(cudaFree(d_bases[b]));
+                d_bases[b] = nullptr; d_cap[b] = 0;
+                CU(cudaMalloc(&d_bases[b], bytes));
+                d_cap[b] = bytes;
+            }
+            if (!src_pinned && h_cap[b] < bytes) {
+                CU(cudaStreamSynchronize(copy));
+                if (h_bases[b]) CU(cudaFreeHost(h_bases[b]));
+                h_bases[b] = nullptr; h_cap[b] = 0;
+                CU(cudaMallocHost(&h_bases[b], bytes));
+                h_cap[b] = bytes;
+            }
+        }
+        return OXG_OK;
+    }
+
+    // room for n boundaries in buffer b; `kernels` (if any) is drained too before the old ones go
+    oxg_status reserve_offs(int b, uint64_t n, cudaStream_t kernels) {
+        if (offs_cap[b] >= n) return OXG_OK;
+        CU(cudaStreamSynchronize(copy));
+        if (kernels) CU(cudaStreamSynchronize(kernels));
+        if (d_offs[b]) CU(cudaFree(d_offs[b]));
+        if (h_offs[b]) CU(cudaFreeHost(h_offs[b]));
+        d_offs[b] = nullptr; h_offs[b] = nullptr; offs_cap[b] = 0;
+        const uint64_t ncap = std::max<uint64_t>(n, 1 << 16);
+        CU(cudaMalloc(&d_offs[b], ncap * 8));
+        CU(cudaMallocHost(&h_offs[b], ncap * 8));
+        offs_cap[b] = ncap;
+        return OXG_OK;
+    }
+
+    // Stage bytes [lo, hi) of batch h (batch-relative) as chunk ci of n_chunks: queue the copies
+    // of the bases and of the read boundaries that can fall inside [lo, hi + 1] on the copy
+    // stream.  The caller makes its kernels wait for ev_ready[b] and records ev_free[b] after them.
+    oxg_status stage(const HostBatch &h, uint64_t ci, uint64_t n_chunks, uint64_t lo, uint64_t hi, cudaStream_t kernels) {
+        const int b = (int)(ci % kStageBufs);
+        const uint64_t base0 = h.offsets[0];
+        // every chunk also validates its share of the offsets (all pairs are seen once per call),
+        // so the O(n_reads) pass runs next to the copies instead of in front of the first one
+        for (uint64_t r = h.n_reads * ci / n_chunks, e = h.n_reads * (ci + 1) / n_chunks; r < e; ++r)
+            if (h.offsets[r + 1] < h.offsets[r]) return fail(OXG_ERR_INVALID, "offsets must be non-decreasing");
+        const uint64_t *ob = std::lower_bound(h.offsets, h.offsets + h.n_reads + 1, base0 + lo + 1);
+        const uint64_t n = (uint64_t)(std::upper_bound(h.offsets, h.offsets + h.n_reads + 1, base0 + hi + 1) - ob);
+        if (ci >= (uint64_t)kStageBufs) {
+            // the buffer's previous chunk: its copy out of the pinned staging has finished (host
+            // side may be refilled) and its kernels have read the device side
+            CU(cudaEventSynchronize(ev_ready[b]));
+            CU(cudaStreamWaitEvent(copy, ev_free[b], 0));
+        }
+        TRY(reserve_offs(b, n + 1, kernels));
+        for (uint64_t i = 0; i < n; ++i) h_offs[b][i] = ob[i] - base0;
+        h_offs[b][n] = ~0ULL >> 1;  // sentinel keeps n_off >= 1
+        n_off[b] = n + 1;
+        const uint8_t *src = h.bases + base0 + lo;
+        if (!h.pinned) { memcpy(h_bases[b], src, hi - lo); src = h_bases[b]; }
+        CU(cudaMemcpyAsync(d_bases[b], src, hi - lo, cudaMemcpyHostToDevice, copy));
+        CU(cudaMemcpyAsync(d_offs[b], h_offs[b], n_off[b] * 8, cudaMemcpyHostToDevice, copy));
+        CU(cudaEventRecord(ev_ready[b], copy));
+        return OXG_OK;
+    }
+};
+
 struct DeviceCtx {
     int dev = -1;
     int sms = 0;
-    cudaStream_t stream = nullptr, copy = nullptr;
+    cudaStream_t stream = nullptr;
     std::mutex mu;
-    // ring of staging buffers for host batches
-    uint8_t *d_stage[kStageBufs] = {};
-    uint8_t *h_stage[kStageBufs] = {};
-    uint64_t d_stage_cap[kStageBufs] = {}, h_stage_cap[kStageBufs] = {};
-    uint64_t *d_offs[kStageBufs] = {};
-    uint64_t *h_offs[kStageBufs] = {};
-    uint64_t offs_cap[kStageBufs] = {};
-    cudaEvent_t ev_ready[kStageBufs] = {};
-    cudaEvent_t ev_stage_free[kStageBufs] = {};  // the kernels reading staging buffer b have finished
+    StageRing ring;  // host batches
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_mid = nullptr;
     cudaEvent_t ev_user0 = nullptr, ev_user1 = nullptr;
     // scratch
@@ -143,7 +243,6 @@ struct DeviceCtx {
     uint32_t *d_frag_cnt = nullptr;   uint64_t frag_cnt_cap = 0;
     uint64_t *d_spill = nullptr;      uint64_t spill_cap = 0;
     unsigned long long *d_spill_n = nullptr;
-    bool agg_attr_done = false;
     // export: compacted pairs, the second pair of arrays of the radix sort, its histogram, pinned bounce buffers
     uint64_t *d_exp_k[2] = {}, *d_exp_v[2] = {};
     uint64_t exp_cap[2] = {};
@@ -176,11 +275,7 @@ oxg_status get_ctx(int dev, DeviceCtx **out) {
                         dev, prop.major, prop.minor);
         c->sms = prop.multiProcessorCount;
         CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&c->copy, cudaStreamNonBlocking));
-        for (int i = 0; i < kStageBufs; ++i) {
-            CU(cudaEventCreateWithFlags(&c->ev_ready[i], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&c->ev_stage_free[i], cudaEventDisableTiming));
-        }
+        TRY(c->ring.init());
         CU(cudaEventCreate(&c->ev_t0));
         CU(cudaEventCreate(&c->ev_t1));
         CU(cudaEventCreate(&c->ev_mid));
@@ -412,6 +507,18 @@ const void *specialised_entry(uint32_t k, int mode) {
 bool specialised_k(uint32_t k) { return specialised_entry(k, kModeCount) != nullptr; }
 uint32_t tile_width(uint32_t k) { return specialised_k(k) ? kWarpTile : kTileW; }
 
+// Static + dynamic shared memory of fn may pass 48 KB: opt in, once per function and device.
+oxg_status max_dyn_smem(const void *fn, int dev, size_t bytes) {
+    static std::mutex mu;
+    static std::vector<std::pair<const void *, int>> done;
+    std::lock_guard<std::mutex> lk(mu);
+    const std::pair<const void *, int> key{fn, dev};
+    if (std::find(done.begin(), done.end(), key) != done.end()) return OXG_OK;
+    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    done.push_back(key);
+    return OXG_OK;
+}
+
 template <int MODE>
 oxg_status launch_consume(oxg_table *t, const ConsumeParams &p) {
     DeviceCtx *c = t->ctx;
@@ -425,16 +532,7 @@ oxg_status launch_consume(oxg_table *t, const ConsumeParams &p) {
     };
     if (const void *fn = specialised_entry(t->k, MODE)) {
         const size_t dyn = consume_dyn_smem(MODE);
-        if (dyn) {  // static + dynamic shared memory may pass 48 KB: opt in once per function and device
-            static std::mutex attr_mu;
-            static std::vector<std::pair<const void *, int>> attr_done;
-            std::lock_guard<std::mutex> lk(attr_mu);
-            const std::pair<const void *, int> key{fn, c->dev};
-            if (std::find(attr_done.begin(), attr_done.end(), key) == attr_done.end()) {
-                CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-                attr_done.push_back(key);
-            }
-        }
+        if (dyn) TRY(max_dyn_smem(fn, c->dev, dyn));
         void *args[] = {const_cast<ConsumeParams *>(&p)};
         CU(cudaLaunchKernel(fn, dim3(grid_of(fn, dyn)), dim3(kThreads), args, dyn, c->stream));
     } else {
@@ -529,17 +627,8 @@ oxg_status plan_partitioned(oxg_table *t, uint64_t span, uint64_t n_tiles, int n
     return OXG_OK;
 }
 
-// scatter_kernel needs more than 48 KB of dynamic shared memory: opt in once per k and device
-oxg_status scatter_attr(DeviceCtx *c, uint32_t k) {
-    static std::mutex mu;
-    static std::vector<std::pair<uint32_t, int>> done;
-    std::lock_guard<std::mutex> lk(mu);
-    const std::pair<uint32_t, int> key{k, c->dev};
-    if (std::find(done.begin(), done.end(), key) != done.end()) return OXG_OK;
-    CU(cudaFuncSetAttribute(specialised_entry(k, kModePart), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    done.push_back(key);
-    return OXG_OK;
-}
+// scatter_kernel needs more than 48 KB of dynamic shared memory
+oxg_status scatter_attr(DeviceCtx *c, uint32_t k) { return max_dyn_smem(specialised_entry(k, kModePart), c->dev, 227 * 1024); }
 
 oxg_status ensure_part_buffers(DeviceCtx *c, const PartPlan &pl) {
     TRY(ensure_dev(&c->d_frag, &c->frag_cap, pl.frag_entries()));
@@ -569,42 +658,19 @@ oxg_status launch_part_a(oxg_table *t, ConsumeParams p, const PartPlan &pl, uint
     return OXG_OK;
 }
 
-// the aggregation kernel is built for three CTA sizes (one CTA per SM each); OXLI_B200_AGG_THREADS picks
-static const int g_agg_threads = [] { const int v = env_int("OXLI_B200_AGG_THREADS", kAggThreadsDefault); return v == 512 || v == 768 || v == 1024 ? v : kAggThreadsDefault; }();
-// ... and OXLI_B200_AGG_THREADS_DIRECT for the variant without the cache, which is bound by the latency
-// of its table loads and wants every thread it can get (C3-shaped input, pass B per step:
-// 512 / 768 / 1024 threads = 46.2 / 35.3 / 32.4 ms)
-static const int g_agg_threads_direct = [] { const int v = env_int("OXLI_B200_AGG_THREADS_DIRECT", 1024); return v == 512 || v == 768 || v == 1024 ? v : 1024; }();
-int agg_threads(bool cache = true) { return cache ? g_agg_threads : g_agg_threads_direct; }
-const void *agg_fn(bool cache = true) {
-    if (!cache) return g_agg_threads_direct == 512 ? (const void *)aggregate_kernel<512, false> : g_agg_threads_direct == 768 ? (const void *)aggregate_kernel<768, false> : (const void *)aggregate_kernel<1024, false>;
-    return g_agg_threads == 512 ? (const void *)aggregate_kernel<512, true> : g_agg_threads == 1024 ? (const void *)aggregate_kernel<1024, true> : (const void *)aggregate_kernel<768, true>;
-}
-// grid: one CTA per SM and item at most (the cached kernel fills an SM's shared memory; the direct
-// one is held to one CTA per SM by its registers)
-oxg_status launch_aggregate(DeviceCtx *c, const AggParams &a, cudaStream_t stream) {
-    const bool cache = a.use_cache != 0;
-    const size_t smem = aggregate_smem_bytes(cache);
-    if (cache && !c->agg_attr_done) {
-        CU(cudaFuncSetAttribute(agg_fn(true), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        c->agg_attr_done = true;
-    }
-    int per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, agg_fn(cache), agg_threads(cache), smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    const uint64_t items = (uint64_t)a.n_parts * a.groups;
-    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(items, (uint64_t)c->sms * per_sm));
-    void *args[] = {const_cast<AggParams *>(&a)};
-    CU(cudaLaunchKernel(agg_fn(cache), dim3(grid), dim3(agg_threads(cache)), args, smem, stream));
-    return OXG_OK;
-}
+// The aggregation kernel in two variants, one CTA per SM each.  With the shared-memory cache:
+// kAggThreadsDefault threads.  Without it, the kernel is bound by the latency of its table loads
+// and wants every thread it can get (C3-shaped input, pass B per step: 512 / 768 / 1024 threads =
+// 46.2 / 35.3 / 32.4 ms).
+constexpr int kAggThreadsDirect = 1024;
+const void *const kAggCached = (const void *)aggregate_kernel<kAggThreadsDefault, true>;
+const void *const kAggDirect = (const void *)aggregate_kernel<kAggThreadsDirect, false>;
 
 // The shared-memory table of pass B pays when keys repeat inside what it is given -- at least two
 // occurrences per key the table holds, is hinted to hold or (sketch) is about to hold -- and a
 // partition's keys fit it: 16 Ki slots took 4.9 K keys per partition at 9.2 ms per C2 step and
 // 9.8 K at 19.6.  Nothing known at all (no hint, no sketch yet): on.
-static const int g_cache_override = env_int("OXLI_B200_AGG_CACHE", -1);  // experiments: 0 / 1 force it off / on
 uint32_t use_cache_for(const oxg_table *t, const PartPlan &pl, uint64_t windows) {
-    if (g_cache_override >= 0) return g_cache_override ? 1u : 0u;
     const uint64_t keys = std::max(std::max(t->size, t->hint_keys), t->est_keys);
     return keys == 0 || (windows >= 2 * keys && keys <= 8192ull * pl.n_parts) ? 1u : 0u;
 }
@@ -621,20 +687,39 @@ uint32_t aggregate_groups(const PartPlan &pl, uint32_t use_cache, uint64_t hashe
     return (uint32_t)std::max<uint64_t>(pl.groups, std::min<uint64_t>(64, (items + pl.n_parts - 1) / pl.n_parts));
 }
 
-// pass B over n_src sources (one, this device's own pass A output, without sharding)
-oxg_status launch_part_b(oxg_table *t, const PartPlan &pl, const AggSource *src, int n_src, uint64_t windows) {
-    DeviceCtx *c = t->ctx;
+// what pass B (and the sketch) of plan pl's rank reads: n_src sources of pass A output -- one,
+// this device's own, without sharding -- into table view v
+AggParams agg_params(const TableView &v, const PartPlan &pl, const AggSource *src, int n_src) {
     AggParams a{};
-    a.table = view_of(t, true);
+    a.table = v;
     for (int s = 0; s < n_src; ++s) a.src[s] = src[s];
     a.n_src = n_src;
     a.n_parts = pl.n_parts; a.dest0 = (uint32_t)pl.self_rank * pl.n_parts; a.n_ctas = pl.grid_a;
     a.frag_cap = pl.frag_cap; a.part_bits = pl.part_bits; a.spill_cap = pl.spill_cap;
     a.owner_shift = pl.owner_shift; a.self_rank = pl.self_rank; a.n_ranks = pl.n_ranks;
+    return a;
+}
+
+// pass B over `windows` hashes of n_src sources.  Grid: one CTA per SM and item at most (the
+// cached kernel fills an SM's shared memory; the direct one is held to one CTA per SM by its
+// registers).
+oxg_status launch_part_b(oxg_table *t, const TableView &v, const PartPlan &pl, const AggSource *src, int n_src,
+                         uint64_t windows, cudaStream_t stream) {
+    DeviceCtx *c = t->ctx;
+    AggParams a = agg_params(v, pl, src, n_src);
     a.work_counter = (unsigned long long *)&t->d_ctrl->absorb_counter;
     a.use_cache = use_cache_for(t, pl, windows);
     a.groups = aggregate_groups(pl, a.use_cache, windows);
-    TRY(launch_aggregate(c, a, c->stream));
+    const void *fn = a.use_cache ? kAggCached : kAggDirect;
+    const int threads = a.use_cache ? kAggThreadsDefault : kAggThreadsDirect;
+    const size_t smem = aggregate_smem_bytes(a.use_cache != 0);
+    if (a.use_cache) TRY(max_dyn_smem(fn, c->dev, smem));
+    int per_sm = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+    const uint64_t items = (uint64_t)a.n_parts * a.groups;
+    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>(items, (uint64_t)c->sms * per_sm));
+    void *args[] = {&a};
+    CU(cudaLaunchKernel(fn, dim3(grid), dim3(threads), args, smem, stream));
     LAUNCHED();
     CU(cudaGetLastError());
     return OXG_OK;
@@ -662,13 +747,7 @@ oxg_status presize_for_group(oxg_table *t, const PartPlan &pl, const AggSource *
         CU(cudaMallocHost(&t->h_sketch, kSketchRegs * 4));
         CU(cudaMemsetAsync(t->d_sketch, 0, kSketchRegs * 4, stream));
     }
-    AggParams a{};
-    for (int s = 0; s < n_src; ++s) a.src[s] = src[s];
-    a.n_src = n_src;
-    a.n_parts = pl.n_parts; a.dest0 = (uint32_t)pl.self_rank * pl.n_parts; a.n_ctas = pl.grid_a;
-    a.frag_cap = pl.frag_cap; a.part_bits = pl.part_bits; a.spill_cap = pl.spill_cap;
-    a.owner_shift = pl.owner_shift; a.self_rank = pl.self_rank; a.n_ranks = pl.n_ranks;
-    sketch_kernel<<<c->sms * 2, 512, 0, stream>>>(a, t->d_sketch);
+    sketch_kernel<<<c->sms * 2, 512, 0, stream>>>(agg_params(TableView{}, pl, src, n_src), t->d_sketch);
     LAUNCHED();
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(t->h_sketch, t->d_sketch, kSketchRegs * 4, cudaMemcpyDeviceToHost, stream));
@@ -710,7 +789,7 @@ oxg_status flush_pending(oxg_table *t, uint64_t *counted) {
     const bool roomy = t->size != 0 && (t->size + 2 * t->last_made) * 10 <= t->cap * 7;
     const bool sketched = !hint_holds && !roomy;
     if (sketched) TRY(presize_for_group(t, t->pend.pl, &own, 1, c->stream));
-    TRY(launch_part_b(t, t->pend.pl, &own, 1, t->pend.windows));
+    TRY(launch_part_b(t, view_of(t, true), t->pend.pl, &own, 1, t->pend.windows, c->stream));
     CU(cudaEventRecord(c->ev_t1, c->stream));
     const uint64_t size_before = t->size;
     TRY(pull_ctrl(t));
@@ -841,56 +920,82 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
     return OXG_OK;
 }
 
-// error-mode driver on a device-resident batch (src/lib.rs:586-600 semantics)
-oxg_status consume_resident(oxg_table *t, const uint8_t *d_bases, const uint64_t *d_offsets,
-                            const uint64_t *h_offsets /*nullable*/, uint64_t n_reads,
-                            uint64_t total, int skip_bad, uint64_t *total_counted,
-                            int64_t *err_read, uint64_t *err_pos) {
-    DeviceCtx *c = t->ctx;
+// ---- error mode (src/lib.rs:586-600): count up to the first window holding a bad byte ---------
+
+// Pre-scan: prime ctrl->first_bad, run kModeFirstBad over the batch's n_win windows through
+// `span` (see consume_batch), and return the first bad window (~0: none).
+template <class Span>
+oxg_status first_bad_window(oxg_table *t, const Span &span, uint64_t n_win, uint64_t total, uint64_t *fb) {
+    t->h_ctrl->first_bad = ~0ULL;
+    CU(cudaMemcpyAsync(&t->d_ctrl->first_bad, &t->h_ctrl->first_bad, 8, cudaMemcpyHostToDevice, t->ctx->stream));
+    TRY(span(kModeFirstBad, 0, n_win, total, nullptr));
+    TRY(pull_ctrl(t));
+    *fb = t->h_ctrl->first_bad;
+    return OXG_OK;
+}
+
+// The read r holding window fb -- the last r with offsets[r] <= fb -- and where it starts.  A host
+// batch (h_offsets given) counts positions from h_offsets[0]; a device-resident one from the
+// start of its buffer, and its boundaries are read back from d_offsets.
+oxg_status read_of(DeviceCtx *c, const uint64_t *h_offsets, const uint64_t *d_offsets, uint64_t n_reads, uint64_t fb,
+                   uint64_t *r, uint64_t *r_start) {
+    std::vector<uint64_t> tmp;
+    uint64_t base0 = 0;
+    if (h_offsets) {
+        base0 = h_offsets[0];
+    } else {
+        tmp.resize(n_reads + 1);
+        CU(cudaMemcpyAsync(tmp.data(), d_offsets, (n_reads + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        h_offsets = tmp.data();
+    }
+    *r = (uint64_t)(std::upper_bound(h_offsets, h_offsets + n_reads + 1, base0 + fb) - h_offsets) - 1;
+    *r_start = h_offsets[*r] - base0;
+    return OXG_OK;
+}
+
+oxg_status bad_kmer(uint64_t r, uint64_t pos, int64_t *err_read, uint64_t *err_pos) {
+    if (err_read) *err_read = (int64_t)r;
+    if (err_pos) *err_pos = pos;
+    return fail(OXG_ERR_BAD_KMER, "bad k-mer encountered at position %llu", (unsigned long long)pos);
+}
+
+// Consume a batch of n_reads reads, `total` bases, into one table.  span(mode, w_lo, w_hi,
+// data_end, counted) runs one mode over window starts [w_lo, w_hi) of the batch: run_span over a
+// device-resident batch, stream_span over a host one.  Offsets as for read_of.  group_cap: see
+// oxg_table::group_cap.
+template <class Span>
+oxg_status consume_batch(oxg_table *t, const Span &span, const uint64_t *h_offsets, const uint64_t *d_offsets,
+                         uint64_t n_reads, uint64_t total, int skip_bad, uint32_t group_cap,
+                         uint64_t *total_counted, int64_t *err_read, uint64_t *err_pos) {
     const uint64_t k = t->k;
-    uint64_t counted = 0;
+    if (total_counted) *total_counted = 0;
     if (err_read) *err_read = -1;
     if (err_pos) *err_pos = 0;
     t->last_ms = 0.f; t->last_ms_a = 0.f; t->last_ms_b = 0.f; t->last_launches = 0;
     const uint64_t n_win = total >= k ? total - k + 1 : 0;
+    if (n_win == 0) return OXG_OK;
     t->part_budget = n_win;
-    t->group_cap = 0;
+    t->group_cap = group_cap;
+    uint64_t counted = 0, fb = ~0ULL;
     oxg_status ret = OXG_OK;
-    if (skip_bad || n_win == 0) {
-        TRY(run_span(t, kModeCount, d_bases, 0, 0, n_win, total, d_offsets, n_reads + 1, nullptr, &counted));
+    if (!skip_bad) TRY(first_bad_window(t, span, n_win, total, &fb));
+    if (fb == ~0ULL) {
+        TRY(span(kModeCount, 0, n_win, total, &counted));
     } else {
-        t->h_ctrl->first_bad = ~0ULL;
-        CU(cudaMemcpyAsync(&t->d_ctrl->first_bad, &t->h_ctrl->first_bad, 8, cudaMemcpyHostToDevice, c->stream));
-        TRY(run_span(t, kModeFirstBad, d_bases, 0, 0, n_win, total, d_offsets, n_reads + 1, nullptr, nullptr));
-        TRY(pull_ctrl(t));
-        const uint64_t fb = t->h_ctrl->first_bad;
-        if (fb == ~0ULL) {
-            TRY(run_span(t, kModeCount, d_bases, 0, 0, n_win, total, d_offsets, n_reads + 1, nullptr, &counted));
-        } else {
-            // read holding position fb: last r with offsets[r] <= fb
-            std::vector<uint64_t> tmp;
-            if (!h_offsets) {
-                tmp.resize(n_reads + 1);
-                CU(cudaMemcpyAsync(tmp.data(), d_offsets, (n_reads + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
-                CU(cudaStreamSynchronize(c->stream));
-                h_offsets = tmp.data();
-            }
-            const uint64_t r = (uint64_t)(std::upper_bound(h_offsets, h_offsets + n_reads + 1, fb) - h_offsets) - 1;
-            const uint64_t r_start = h_offsets[r];
-            uint64_t in_read = 0;
-            // everything before that read, then the clean prefix of the read itself
-            TRY(run_span(t, kModeCount, d_bases, 0, 0, r_start >= k ? r_start - k + 1 : 0, r_start, d_offsets, n_reads + 1, nullptr, &counted));
-            TRY(flush_pending(t, &counted));  // the position reported below counts the windows of the bad read only
-            TRY(run_span(t, kModeCount, d_bases, 0, r_start, fb, fb + k - 1, d_offsets, n_reads + 1, nullptr, &in_read));
-            TRY(flush_pending(t, &in_read));
-            counted += in_read;
-            if (err_read) *err_read = (int64_t)r;
-            if (err_pos) *err_pos = in_read;
-            ret = fail(OXG_ERR_BAD_KMER, "bad k-mer encountered at position %llu", (unsigned long long)in_read);
-        }
+        uint64_t r = 0, r_start = 0, in_read = 0;
+        TRY(read_of(t->ctx, h_offsets, d_offsets, n_reads, fb, &r, &r_start));
+        // everything before that read, then the clean prefix of the read itself
+        TRY(span(kModeCount, 0, r_start >= k ? r_start - k + 1 : 0, r_start, &counted));
+        TRY(flush_pending(t, &counted));  // the position reported below counts the windows of the bad read only
+        TRY(span(kModeCount, r_start, fb, fb + k - 1, &in_read));
+        TRY(flush_pending(t, &in_read));
+        counted += in_read;
+        ret = bad_kmer(r, in_read, err_read, err_pos);
     }
     if (ret == OXG_OK) TRY(flush_pending(t, &counted));
     t->part_budget = 0;
+    t->group_cap = 0;
     if (total_counted) *total_counted = counted;
     return ret;
 }
@@ -988,7 +1093,7 @@ oxg_status oxg_table_capacity(const oxg_table *t, uint64_t *slots) {
 oxg_status oxg_sync(oxg_table *t) {
     ENTER(t);
     CU(cudaStreamSynchronize(c->stream));
-    CU(cudaStreamSynchronize(c->copy));
+    CU(cudaStreamSynchronize(c->ring.copy));
     return OXG_OK;
 }
 
@@ -1067,7 +1172,10 @@ oxg_status oxg_consume_batch_device(oxg_table *t, const uint8_t *d_bases, const 
     if (total_counted) *total_counted = 0;
     if (n_reads == 0 || total_bases == 0) { if (err_read) *err_read = -1; if (err_pos) *err_pos = 0; return OXG_OK; }
     if (!d_bases || !d_offsets) return fail(OXG_ERR_INVALID, "null argument");
-    return consume_resident(t, d_bases, d_offsets, nullptr, n_reads, total_bases, skip_bad, total_counted, err_read, err_pos);
+    auto span = [&](int mode, uint64_t w_lo, uint64_t w_hi, uint64_t data_end, uint64_t *counted) {
+        return run_span(t, mode, d_bases, 0, w_lo, w_hi, data_end, d_offsets, n_reads + 1, nullptr, counted);
+    };
+    return consume_batch(t, span, nullptr, d_offsets, n_reads, total_bases, skip_bad, 0, total_counted, err_read, err_pos);
 }
 
 oxg_status oxg_hash_batch_device(oxg_table *t, const uint8_t *d_bases, const uint64_t *d_offsets,
@@ -1081,95 +1189,39 @@ oxg_status oxg_hash_batch_device(oxg_table *t, const uint8_t *d_bases, const uin
     return OXG_OK;
 }
 
-// Host batch: stream [w_lo, w_hi) through a ring of kStageBufs staging buffers.  A producer
-// thread slices the read boundaries, stages pageable sources into pinned memory and queues the
-// H2D copies back to back on the copy stream, up to kStageBufs chunks ahead of the kernels; the
-// calling thread launches each chunk's kernels as its copy lands (run_span blocks until they
-// are done, which is also what frees the chunk's buffer).  With only one chunk in flight ahead
-// the copy engine idled between chunks and the step was 19 ms longer than its kernels.
-static oxg_status stream_span(oxg_table *t, int mode, const uint8_t *bases, const uint64_t *offsets,
-                              uint64_t n_reads, uint64_t w_lo, uint64_t w_hi, uint64_t data_end,
-                              bool src_pinned, uint64_t *counted, const uint8_t *mapped = nullptr) {
-    // mapped != nullptr: device-usable alias of `bases` (pinned, mapped host memory); the kernels
-    // then read the bases in place over PCIe and only the read boundaries are copied
+// Host batch: stream [w_lo, w_hi) through the context's staging ring.  A producer thread slices
+// the read boundaries, stages pageable sources into pinned memory and queues the H2D copies back
+// to back on the copy stream, up to kStageBufs chunks ahead of the kernels; the calling thread
+// launches each chunk's kernels as its copy lands (run_span blocks until they are done, which is
+// also what frees the chunk's buffer).  With only one chunk in flight ahead the copy engine idled
+// between chunks and the step was 19 ms longer than its kernels.
+static oxg_status stream_span(oxg_table *t, int mode, const HostBatch &h, uint64_t w_lo, uint64_t w_hi,
+                              uint64_t data_end, uint64_t *counted) {
     DeviceCtx *c = t->ctx;
+    StageRing &ring = c->ring;
     const uint64_t k = t->k;
     if (w_hi <= w_lo) return OXG_OK;
-    const uint64_t base0 = offsets[0];
     const uint64_t first = w_lo & ~(uint64_t)(kTileW - 1);
     const uint64_t n_chunks = (w_hi - first + kChunkBytes - 1) / kChunkBytes;
     // staging sized to the batch (pinning full chunks costs a third of a second; a caller
     // that hands over a few thousand reads should not pay it), full chunks once one is needed
     const uint64_t stage_bytes = std::min(pow2_at_least(std::max<uint64_t>(data_end - first, 1 << 20)), kChunkBytes) + 256 + 16;
-    for (int b = 0; b < (int)std::min<uint64_t>(n_chunks, kStageBufs) && !mapped; ++b) {
-        if (c->d_stage_cap[b] < stage_bytes) {
-            CU(cudaStreamSynchronize(c->stream));
-            if (c->d_stage[b]) CU(cudaFree(c->d_stage[b]));
-            c->d_stage[b] = nullptr; c->d_stage_cap[b] = 0;
-            CU(cudaMalloc(&c->d_stage[b], stage_bytes));
-            c->d_stage_cap[b] = stage_bytes;
-        }
-        if (!src_pinned && c->h_stage_cap[b] < stage_bytes) {
-            CU(cudaStreamSynchronize(c->copy));
-            if (c->h_stage[b]) CU(cudaFreeHost(c->h_stage[b]));
-            c->h_stage[b] = nullptr; c->h_stage_cap[b] = 0;
-            CU(cudaMallocHost(&c->h_stage[b], stage_bytes));
-            c->h_stage_cap[b] = stage_bytes;
-        }
-    }
-    struct Slice { uint64_t lo, hi; const uint64_t *ob; uint64_t n_off; };
-    auto slice_of = [&](uint64_t ci) {
-        Slice s;
-        s.lo = first + ci * kChunkBytes;
-        s.hi = std::min(data_end, s.lo + kChunkBytes + k - 1);
-        // reads whose boundaries can fall inside [lo, hi + 1]
-        s.ob = std::lower_bound(offsets, offsets + n_reads + 1, base0 + s.lo + 1);
-        s.n_off = (uint64_t)(std::upper_bound(offsets, offsets + n_reads + 1, base0 + s.hi + 1) - s.ob);
-        return s;
-    };
+    TRY(ring.reserve((int)std::min<uint64_t>(n_chunks, kStageBufs), stage_bytes, h.pinned, c->stream));
+    auto chunk_lo = [&](uint64_t ci) { return first + ci * kChunkBytes; };
+    auto chunk_hi = [&](uint64_t ci) { return std::min(data_end, chunk_lo(ci) + kChunkBytes + k - 1); };
     // the previous use of buffer b (chunk ci - kStageBufs) is over: its kernels were waited for
+    // (a partitioned launch is only queued when run_span returns)
     auto issue_copy = [&](uint64_t ci) -> oxg_status {
         NvtxRange range("oxg:stage + H2D copy");
-        const int b = (int)(ci % kStageBufs);
-        // every chunk also validates its share of the offsets (all pairs are seen once per call),
-        // so the O(n_reads) pass runs on the producer thread next to the copies instead of in
-        // front of the first one
-        for (uint64_t r = n_reads * ci / n_chunks, e = n_reads * (ci + 1) / n_chunks; r < e; ++r)
-            if (offsets[r + 1] < offsets[r]) return fail(OXG_ERR_INVALID, "offsets must be non-decreasing");
-        const Slice s = slice_of(ci);
-        if (ci >= (uint64_t)kStageBufs) {
-            // the buffer's previous chunk: its copy out of the pinned staging has finished (host
-            // side may be refilled) and its kernels have read the device side (a partitioned
-            // launch is only queued when run_span returns)
-            CU(cudaEventSynchronize(c->ev_ready[b]));
-            CU(cudaStreamWaitEvent(c->copy, c->ev_stage_free[b], 0));
-        }
-        if (c->offs_cap[b] < s.n_off + 1) {
-            CU(cudaStreamSynchronize(c->copy));
-            if (c->d_offs[b]) CU(cudaFree(c->d_offs[b]));
-            if (c->h_offs[b]) CU(cudaFreeHost(c->h_offs[b]));
-            c->d_offs[b] = nullptr; c->h_offs[b] = nullptr; c->offs_cap[b] = 0;
-            const uint64_t ncap = std::max<uint64_t>(s.n_off + 1, 1 << 16);
-            CU(cudaMalloc(&c->d_offs[b], ncap * 8));
-            CU(cudaMallocHost(&c->h_offs[b], ncap * 8));
-            c->offs_cap[b] = ncap;
-        }
-        for (uint64_t i = 0; i < s.n_off; ++i) c->h_offs[b][i] = s.ob[i] - base0;  // batch-relative positions
-        c->h_offs[b][s.n_off] = ~0ULL >> 1;  // sentinel keeps n_off >= 1
-        const uint8_t *src = bases + base0 + s.lo;
-        if (!src_pinned) { memcpy(c->h_stage[b], src, s.hi - s.lo); src = c->h_stage[b]; }
-        if (!mapped) CU(cudaMemcpyAsync(c->d_stage[b], src, s.hi - s.lo, cudaMemcpyHostToDevice, c->copy));
-        CU(cudaMemcpyAsync(c->d_offs[b], c->h_offs[b], (s.n_off + 1) * 8, cudaMemcpyHostToDevice, c->copy));
-        CU(cudaEventRecord(c->ev_ready[b], c->copy));
-        return OXG_OK;
+        return ring.stage(h, ci, n_chunks, chunk_lo(ci), chunk_hi(ci), nullptr);
     };
     auto run_chunk = [&](uint64_t ci) -> oxg_status {
         const int b = (int)(ci % kStageBufs);
-        const Slice s = slice_of(ci);
-        CU(cudaStreamWaitEvent(c->stream, c->ev_ready[b], 0));
-        TRY(run_span(t, mode, mapped ? mapped + base0 + s.lo : c->d_stage[b], s.lo, std::max(s.lo, w_lo),
-                     std::min(w_hi, s.lo + kChunkBytes), s.hi, c->d_offs[b], s.n_off + 1, nullptr, counted));
-        CU(cudaEventRecord(c->ev_stage_free[b], c->stream));
+        const uint64_t lo = chunk_lo(ci);
+        CU(cudaStreamWaitEvent(c->stream, ring.ev_ready[b], 0));
+        TRY(run_span(t, mode, ring.d_bases[b], lo, std::max(lo, w_lo), std::min(w_hi, lo + kChunkBytes), chunk_hi(ci),
+                     ring.d_offs[b], ring.n_off[b], nullptr, counted));
+        CU(cudaEventRecord(ring.ev_free[b], c->stream));
         return OXG_OK;
     };
     if (n_chunks == 1) {
@@ -1243,7 +1295,7 @@ static oxg_status stream_span(oxg_table *t, int mode, const uint8_t *bases, cons
     producer.join();
     // a call that stopped early (error, or pre-scan hit) may have copies queued that nobody will
     // wait for: drain them before the staging buffers are used again
-    if (st != OXG_OK || mode != kModeCount) cudaStreamSynchronize(c->copy);
+    if (st != OXG_OK || mode != kModeCount) cudaStreamSynchronize(ring.copy);
     return st;
 }
 
@@ -1256,54 +1308,18 @@ oxg_status oxg_consume_batch(oxg_table *t, const uint8_t *bases, const uint64_t 
     if (err_pos) *err_pos = 0;
     if (n_reads == 0) return OXG_OK;
     if (!bases || !offsets) return fail(OXG_ERR_INVALID, "null argument");
-    // (monotonicity of the offsets is checked chunk by chunk while they are staged: stream_span)
+    // (monotonicity of the offsets is checked chunk by chunk while they are staged: StageRing::stage)
     if (offsets[n_reads] < offsets[0]) return fail(OXG_ERR_INVALID, "offsets must be non-decreasing");
-    const uint64_t k = t->k;
-    const uint64_t total = offsets[n_reads] - offsets[0];
-    const uint64_t n_win = total >= k ? total - k + 1 : 0;
-    t->last_ms = 0.f; t->last_ms_a = 0.f; t->last_ms_b = 0.f; t->last_launches = 0;
-    if (n_win == 0) return OXG_OK;
-    t->part_budget = n_win;
-    t->group_cap = 4;
     cudaPointerAttributes attr{};
-    bool pinned = cudaPointerGetAttributes(&attr, bases) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+    const bool pinned = cudaPointerGetAttributes(&attr, bases) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     cudaGetLastError();
-    static const bool zero_copy = [] { const char *e = getenv("OXLI_B200_ZEROCOPY"); return e && *e && strcmp(e, "0") != 0; }();
-    const uint8_t *mapped = pinned && zero_copy && attr.devicePointer ? static_cast<const uint8_t *>(attr.devicePointer) : nullptr;
-    if (mapped && ((reinterpret_cast<uintptr_t>(mapped) + offsets[0]) & 15)) mapped = nullptr;  // the kernels copy 16-byte units
-    uint64_t counted = 0;
-    oxg_status ret = OXG_OK;
-    if (skip_bad) {
-        TRY(stream_span(t, kModeCount, bases, offsets, n_reads, 0, n_win, total, pinned, &counted, mapped));
-    } else {
-        t->h_ctrl->first_bad = ~0ULL;
-        CU(cudaMemcpyAsync(&t->d_ctrl->first_bad, &t->h_ctrl->first_bad, 8, cudaMemcpyHostToDevice, c->stream));
-        TRY(stream_span(t, kModeFirstBad, bases, offsets, n_reads, 0, n_win, total, pinned, nullptr));
-        TRY(pull_ctrl(t));
-        const uint64_t fb = t->h_ctrl->first_bad;
-        if (fb == ~0ULL) {
-            TRY(stream_span(t, kModeCount, bases, offsets, n_reads, 0, n_win, total, pinned, &counted));
-        } else {
-            const uint64_t base0 = offsets[0];
-            const uint64_t r = (uint64_t)(std::upper_bound(offsets, offsets + n_reads + 1, base0 + fb) - offsets) - 1;
-            const uint64_t r_start = offsets[r] - base0;
-            uint64_t in_read = 0;
-            TRY(stream_span(t, kModeCount, bases, offsets, n_reads, 0, r_start >= k ? r_start - k + 1 : 0, r_start, pinned, &counted));
-            TRY(flush_pending(t, &counted));  // the position reported below counts the windows of the bad read only
-            TRY(stream_span(t, kModeCount, bases, offsets, n_reads, r_start, fb, fb + k - 1, pinned, &in_read));
-            TRY(flush_pending(t, &in_read));
-            counted += in_read;
-            if (err_read) *err_read = (int64_t)r;
-            if (err_pos) *err_pos = in_read;
-            ret = fail(OXG_ERR_BAD_KMER, "bad k-mer encountered at position %llu", (unsigned long long)in_read);
-        }
-    }
-    if (ret == OXG_OK) TRY(flush_pending(t, &counted));
-    t->part_budget = 0;
-    t->group_cap = 0;
-    if (total_counted) *total_counted = counted;
-    return ret;
+    const HostBatch h{bases, offsets, n_reads, pinned};
+    auto span = [&](int mode, uint64_t w_lo, uint64_t w_hi, uint64_t data_end, uint64_t *counted) {
+        return stream_span(t, mode, h, w_lo, w_hi, data_end, counted);
+    };
+    return consume_batch(t, span, offsets, nullptr, n_reads, offsets[n_reads] - offsets[0], skip_bad, 4, total_counted, err_read, err_pos);
 }
+
 
 // ---- by-hash operations ----------------------------------------------------
 

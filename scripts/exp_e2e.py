@@ -13,7 +13,7 @@ for rep in range(4):
     t.clear()
     t0 = time.perf_counter(); st, total, _, _ = t.consume_batch(h, offs); dt = time.perf_counter() - t0
     ms, nl = t.last_consume_kernel_ms()
-    print(f"chunk {os.environ.get('OXLI_B200_CHUNK_MB', '64')} MiB zero_copy={os.environ.get('OXLI_B200_ZEROCOPY', '0')}: wall {dt*1e3:.1f} ms, kernels {ms:.1f} ms in {nl} launches, {total/dt/1e9:.1f} G k-mers/s", flush=True)
+    print(f"chunk {os.environ.get('OXLI_B200_CHUNK_MB', '64')} MiB: wall {dt*1e3:.1f} ms, kernels {ms:.1f} ms in {nl} launches, {total/dt/1e9:.1f} G k-mers/s", flush=True)
 # error mode = a pre-scan pass (same copies, kernels of ~0.2 ms per chunk) + the counting pass:
 # the difference to the skip-mode wall time is what the copies cost when nothing competes
 for rep in range(2):
