@@ -220,6 +220,15 @@ struct StageRing {
     }
 };
 
+// Deferred (key, increment) pairs of a table that ran into its load limit (drain_deferred): the
+// list launches defer into, and the one a replay of it defers into.  Fixed lists are allocated
+// once and never enlarged (a shard's: see oxg_table::pooled).
+struct DeferLists {
+    ulonglong2 *d_pairs = nullptr;   uint64_t cap = 0;
+    ulonglong2 *d_pairs2 = nullptr;  uint64_t cap2 = 0;
+    bool fixed = false;
+};
+
 struct DeviceCtx {
     int dev = -1;
     int sms = 0;
@@ -230,8 +239,7 @@ struct DeviceCtx {
     cudaEvent_t ev_user0 = nullptr, ev_user1 = nullptr;
     // scratch
     uint64_t *d_tile_first = nullptr; uint64_t tile_first_cap = 0;
-    ulonglong2 *d_overflow = nullptr;   uint64_t overflow_cap = 0;   // deferred (key, increment) pairs
-    ulonglong2 *d_overflow2 = nullptr;  uint64_t overflow2_cap = 0;  // replay target when a replay defers again
+    DeferLists defer;                 // tables of this context that are not shards
     uint64_t *d_dense = nullptr;      // kHistDense bins
     uint64_t *d_big = nullptr;        uint64_t big_cap = 0;
     uint64_t *d_io = nullptr;         uint64_t io_cap = 0;   // generic u64 in/out scratch (device)
@@ -341,6 +349,30 @@ uint64_t capacity_for_keys(uint64_t keys) {
     return cap;
 }
 
+// the slots of a table grown for `keys` distinct keys: <= 50 % load, and sparse while small
+uint64_t slots_for(uint64_t keys) { return std::max(capacity_for_keys(keys), pow2_at_least(keys * 2)); }
+
+// Device memory free now.  A slow driver call, and at times a very slow one (10-150 ms measured
+// with two ranks on one box; asked in every round of the last third of a C3 step, it made steps of
+// 95 ms take 100-260 ms at random): ask it only when there is a question.
+oxg_status free_device_bytes(size_t *free_b) {
+    size_t total = 0;
+    CU(cudaMemGetInfo(free_b, &total));
+    return OXG_OK;
+}
+
+// *yes: a table grown for `keys` would be larger than `cap` slots and take less than half of the
+// free device memory (asked only when it would be larger)
+oxg_status larger_and_fits(uint64_t keys, uint64_t cap, bool *yes) {
+    *yes = false;
+    const uint64_t want = slots_for(keys);
+    if (want <= cap) return OXG_OK;
+    size_t free_b = 0;
+    TRY(free_device_bytes(&free_b));
+    *yes = want * 16 < free_b / 2;
+    return OXG_OK;
+}
+
 
 }  // namespace
 
@@ -394,7 +426,8 @@ struct oxg_table {
 
 namespace {
 
-TableView view_of(const oxg_table *t, bool with_overflow) {
+// the table as its kernels see it; `defer` (nullptr: none) takes what runs into the load limit
+TableView view_of(const oxg_table *t, const DeferLists *defer = nullptr) {
     TableView v;
     v.slots = t->slots;
     v.cap = t->cap;
@@ -403,8 +436,8 @@ TableView view_of(const oxg_table *t, bool with_overflow) {
     v.shift = 64 - lg;
     v.limit = t->cap - t->cap / 5;  // stop creating keys at 80 % load
     v.ctrl = t->d_ctrl;
-    v.overflow = with_overflow ? t->ctx->d_overflow : nullptr;
-    v.overflow_cap = with_overflow ? t->ctx->overflow_cap : 0;
+    v.overflow = defer ? defer->d_pairs : nullptr;
+    v.overflow_cap = defer ? defer->cap : 0;
     return v;
 }
 
@@ -426,8 +459,9 @@ constexpr size_t kFieldTile = offsetof(Ctrl, tile_counter) / 8;
 constexpr size_t kLaunchFields = (offsetof(Ctrl, scratch) - offsetof(Ctrl, counted)) / 8;
 constexpr size_t kFieldScratch = offsetof(Ctrl, scratch) / 8;
 
-oxg_status alloc_slots(DeviceCtx *c, uint64_t cap, ulonglong2 **out, bool pooled = false) {
-    if (pooled) CU(cudaMallocAsync(out, cap * sizeof(ulonglong2), c->stream));
+oxg_status alloc_slots(const oxg_table *t, uint64_t cap, ulonglong2 **out) {
+    DeviceCtx *c = t->ctx;
+    if (t->pooled) CU(cudaMallocAsync(out, cap * sizeof(ulonglong2), c->stream));
     else CU(cudaMalloc(out, cap * sizeof(ulonglong2)));  // (cudaMallocAsync pools were 2x slower for growing multi-GB tables)
     init_slots_kernel<<<grid_for(c, cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(*out, cap);
     LAUNCHED();
@@ -435,37 +469,67 @@ oxg_status alloc_slots(DeviceCtx *c, uint64_t cap, ulonglong2 **out, bool pooled
     return OXG_OK;
 }
 
-// grow (or rebuild at the same size) so that `keys` distinct keys sit at <= 50 % load
+oxg_status free_slots(const oxg_table *t, ulonglong2 *p) {
+    if (t->pooled) CU(cudaFreeAsync(p, t->ctx->stream)); else CU(cudaFree(p));
+    return OXG_OK;
+}
+
+// grow so that `keys` distinct keys sit at <= 50 % load
 oxg_status grow_to_fit(oxg_table *t, uint64_t keys) {
-    uint64_t want = std::max(capacity_for_keys(keys), pow2_at_least(keys * 2));
+    const uint64_t want = slots_for(keys);
     if (want <= t->cap) return OXG_OK;
     DeviceCtx *c = t->ctx;
     ulonglong2 *fresh = nullptr;
-    TRY(alloc_slots(c, want, &fresh, t->pooled));
+    TRY(alloc_slots(t, want, &fresh));
     ulonglong2 *old = t->slots;
     const uint64_t old_cap = t->cap;
     t->slots = fresh;
     t->cap = want;
     if (t->size) {
-        rehash_kernel<<<grid_for(c, old_cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, old_cap, view_of(t, false));
+        rehash_kernel<<<grid_for(c, old_cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, old_cap, view_of(t));
         LAUNCHED();
         CU(cudaGetLastError());
     }
     CU(cudaStreamSynchronize(c->stream));
-    if (t->pooled) CU(cudaFreeAsync(old, c->stream)); else CU(cudaFree(old));
-    return OXG_OK;
+    return free_slots(t, old);
 }
 
 oxg_status reserve_keys(oxg_table *t, uint64_t extra) { return grow_to_fit(t, t->size + extra); }
 
+// Rebuild the table into a fresh slot array of the same size (erase, cut).  rebuild(old) queues
+// the kernel that moves what stays from the old array into view_of(t) and adds what it drops to
+// ctrl->scratch[0], which the caller has zeroed; side_drops(count) says whether the out-of-band
+// key goes too.  *removed (if given): the keys dropped, the out-of-band one included.
+template <class Rebuild, class SideDrops>
+oxg_status rebuild_slots(oxg_table *t, const Rebuild &rebuild, const SideDrops &side_drops, uint64_t *removed) {
+    ulonglong2 *fresh = nullptr;
+    TRY(alloc_slots(t, t->cap, &fresh));
+    ulonglong2 *old = t->slots;
+    t->slots = fresh;
+    rebuild(old);
+    LAUNCHED();
+    CU(cudaGetLastError());
+    TRY(pull_ctrl(t));
+    TRY(free_slots(t, old));
+    Ctrl *h = t->h_ctrl;
+    uint64_t n = h->scratch[0];
+    h->size -= n;
+    if (h->side_present && side_drops(h->side_count)) { h->side_present = 0; h->side_count = 0; ++n; }
+    t->size = h->size;
+    CU(cudaMemcpyAsync(t->d_ctrl, h, offsetof(Ctrl, counted), cudaMemcpyHostToDevice, t->ctx->stream));
+    CU(cudaStreamSynchronize(t->ctx->stream));
+    if (removed) *removed = n;
+    return OXG_OK;
+}
+
 // A launch ran into the load limit and deferred `ov` hash OCCURRENCES (not distinct keys: on
 // high-coverage input every new key is deferred many times).  Grow geometrically -- room for
 // at most as many new keys as the table already holds -- and replay; a replay that runs into
-// the limit again defers into the second list and the loop goes round once more.
-oxg_status drain_deferred(oxg_table *t, uint64_t ov, bool may_allocate = true) {
+// the limit again defers into the second list, the two swap and the loop goes round once more.
+oxg_status drain_deferred(oxg_table *t, DeferLists &d, uint64_t ov) {
     NvtxRange range("oxg:replay deferred");
     DeviceCtx *c = t->ctx;
-    if (ov > c->overflow_cap) return fail(OXG_ERR_CUDA, "internal: overflow list overrun");
+    if (ov > d.cap) return fail(OXG_ERR_CUDA, "internal: overflow list overrun");
     uint64_t prev = ~0ULL;
     while (ov) {
         const uint64_t room = std::min<uint64_t>(ov, std::max<uint64_t>(t->size, 1ull << 20));
@@ -474,19 +538,36 @@ oxg_status drain_deferred(oxg_table *t, uint64_t ov, bool may_allocate = true) {
         // deferred for a probe run that would not end rather than for load: double regardless
         if (t->cap == cap_before && ov >= prev) TRY(grow_to_fit(t, t->cap));
         prev = ov;
-        if (may_allocate) TRY(ensure_dev(&c->d_overflow2, &c->overflow2_cap, ov));
-        else if (c->overflow2_cap < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
+        if (!d.fixed) TRY(ensure_dev(&d.d_pairs2, &d.cap2, ov));
+        else if (d.cap2 < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
         TRY(zero_ctrl_fields(t, offsetof(Ctrl, overflow) / 8, 1));
-        TableView v = view_of(t, false);
-        v.overflow = c->d_overflow2; v.overflow_cap = c->overflow2_cap;
-        replay_pairs_kernel<<<grid_for(c, (ov + 3) / 4, kOpThreads, 8), kOpThreads, 0, c->stream>>>(v, c->d_overflow, ov);
+        TableView v = view_of(t);
+        v.overflow = d.d_pairs2; v.overflow_cap = d.cap2;
+        replay_pairs_kernel<<<grid_for(c, (ov + 3) / 4, kOpThreads, 8), kOpThreads, 0, c->stream>>>(v, d.d_pairs, ov);
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
         ov = t->h_ctrl->overflow;
-        std::swap(c->d_overflow, c->d_overflow2);
-        std::swap(c->overflow_cap, c->overflow2_cap);
+        std::swap(d.d_pairs, d.d_pairs2);
+        std::swap(d.cap, d.cap2);
     }
+    return OXG_OK;
+}
+
+// The end of a counting launch, or of a group of `launches` of them, begun at ev_t0: read the
+// control block, add the time, the launches and the k-mers counted to the tallies, and tell the
+// time, the keys created and the hash occurrences deferred.
+struct Counting { float ms = 0.f; uint64_t made = 0, ov = 0; };
+oxg_status end_counting(oxg_table *t, uint64_t launches, uint64_t *counted, Counting *out) {
+    DeviceCtx *c = t->ctx;
+    CU(cudaEventRecord(c->ev_t1, c->stream));
+    const uint64_t size_before = t->size;
+    TRY(pull_ctrl(t));
+    CU(cudaEventElapsedTime(&out->ms, c->ev_t0, c->ev_t1));
+    t->last_ms += out->ms; t->last_launches += launches;
+    if (counted) *counted += t->h_ctrl->counted;
+    out->made = t->size - size_before;
+    out->ov = t->h_ctrl->overflow;
     return OXG_OK;
 }
 
@@ -763,9 +844,9 @@ oxg_status presize_for_group(oxg_table *t, const PartPlan &pl, const AggSource *
     if (rounds_left > 1) headroom = est * 4 >= (double)arrivals ? std::max(4.0, 0.5 * (double)rounds_left) : (double)std::min<uint64_t>(4, rounds_left);
     uint64_t expect = (uint64_t)(est * 1.04 * headroom) + unseen + 1024;  // 1.04: three standard errors
     if (headroom > 4.0) {  // a guess that size must not cost more than half of what is free
-        size_t free_b = 0, total_b = 0;
-        CU(cudaMemGetInfo(&free_b, &total_b));
-        while (headroom > 4.0 && std::max(capacity_for_keys(expect), pow2_at_least(expect * 2)) * 16 > free_b / 2) {
+        size_t free_b = 0;
+        TRY(free_device_bytes(&free_b));
+        while (headroom > 4.0 && slots_for(expect) * 16 > free_b / 2) {
             headroom /= 2;
             expect = (uint64_t)(est * 1.04 * std::max(headroom, 4.0)) + unseen + 1024;
         }
@@ -789,21 +870,16 @@ oxg_status flush_pending(oxg_table *t, uint64_t *counted) {
     const bool roomy = t->size != 0 && (t->size + 2 * t->last_made) * 10 <= t->cap * 7;
     const bool sketched = !hint_holds && !roomy;
     if (sketched) TRY(presize_for_group(t, t->pend.pl, &own, 1, c->stream));
-    TRY(launch_part_b(t, view_of(t, true), t->pend.pl, &own, 1, t->pend.windows, c->stream));
-    CU(cudaEventRecord(c->ev_t1, c->stream));
-    const uint64_t size_before = t->size;
-    TRY(pull_ctrl(t));
-    float ms = 0.f, ms_a = 0.f;
-    CU(cudaEventElapsedTime(&ms, c->ev_t0, c->ev_t1));
+    TRY(launch_part_b(t, view_of(t, &c->defer), t->pend.pl, &own, 1, t->pend.windows, c->stream));
+    Counting r;
+    TRY(end_counting(t, t->pend.launches, counted, &r));
+    float ms_a = 0.f;
     CU(cudaEventElapsedTime(&ms_a, c->ev_t0, c->ev_mid));
-    t->last_ms += ms; t->last_launches += t->pend.launches;
-    t->last_ms_a += ms_a; t->last_ms_b += ms - ms_a;
-    if (counted) *counted += t->h_ctrl->counted;
-    const uint64_t ov = t->h_ctrl->overflow;
+    t->last_ms_a += ms_a; t->last_ms_b += r.ms - ms_a;
+    const uint64_t made = r.made;
     // forecast for the next group: what this one created, unless the caller's hint still covers the table
-    const uint64_t made = t->size - size_before;
-    t->last_new = ov ? made + ov : (t->hinted && t->size <= t->hint_keys) ? 0 : made;
-    if (ov) TRY(drain_deferred(t, ov));
+    t->last_new = r.ov ? made + r.ov : (t->hinted && t->size <= t->hint_keys) ? 0 : made;
+    if (r.ov) TRY(drain_deferred(t, c->defer, r.ov));
     t->last_made = made;
     if (sketched) t->sketch_covers = t->size;
     if (!hint_holds) {
@@ -814,12 +890,9 @@ oxg_status flush_pending(oxg_table *t, uint64_t *counted) {
         if (made * 4 >= t->pend.windows && t->part_budget && t->size * 20 >= t->cap * 7) {  // (only a table that is filling up)
             const uint64_t more = (uint64_t)((double)made / (double)t->pend.windows * 0.6 * (double)t->part_budget);
             const uint64_t want = t->size + more;
-            const uint64_t cap_want = std::max(capacity_for_keys(want), pow2_at_least(want * 2));
-            if (cap_want > t->cap) {  // (cudaMemGetInfo is a slow driver call, 10-150 ms at times: only when there is a question)
-                size_t free_b = 0, total_b = 0;
-                CU(cudaMemGetInfo(&free_b, &total_b));
-                if (cap_want * 16 < free_b / 2) TRY(grow_to_fit(t, want));
-            }
+            bool grow = false;
+            TRY(larger_and_fits(want, t->cap, &grow));
+            if (grow) TRY(grow_to_fit(t, want));
         }
     }
     return OXG_OK;
@@ -859,7 +932,7 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
                 if (expect * 10 > t->cap * 7) TRY(grow_to_fit(t, expect));
                 else if (over_loaded(t->size, t->cap)) TRY(grow_to_fit(t, t->size));
             }
-            TRY(ensure_dev(&c->d_overflow, &c->overflow_cap, std::max<uint64_t>(span, t->pend.active ? t->pend.planned : 0)));
+            TRY(ensure_dev(&c->defer.d_pairs, &c->defer.cap, std::max<uint64_t>(span, t->pend.active ? t->pend.planned : 0)));
             // counted, overflow, absorbed, tile and absorb counters -- unless a group of pass A
             // launches is accumulating into them
             if (!t->pend.active) TRY(zero_ctrl_fields(t, kFieldCounted, kLaunchFields));
@@ -869,7 +942,7 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
         ConsumeParams p{};
         p.bases = d_bases; p.g0 = g0; p.w_lo = lo; p.w_hi = hi; p.data_end = data_end;
         p.tile_base = tile_base; p.n_tiles = n_tiles; p.offsets = d_offsets; p.n_off = n_off;
-        p.tile_first = c->d_tile_first; p.table = view_of(t, mode == kModeCount);
+        p.tile_first = c->d_tile_first; p.table = view_of(t, mode == kModeCount ? &c->defer : nullptr);
         p.hashes_out = hashes_out ? hashes_out + (lo - w_lo) : nullptr; p.ksize = t->k;
         tile_first_kernel<<<(unsigned)((n_tiles + 255) / 256), 256, 0, c->stream>>>(d_offsets, n_off, tile_base, n_tiles, tw, c->d_tile_first);
         LAUNCHED();
@@ -899,21 +972,15 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
         if (mode == kModeCount) TRY(launch_consume<kModeCount>(t, p));
         else if (mode == kModeHash) TRY(launch_consume<kModeHash>(t, p));
         else TRY(launch_consume<kModeFirstBad>(t, p));
-        CU(cudaEventRecord(c->ev_t1, c->stream));
         if (mode == kModeCount) {
-            const uint64_t size_before = t->size;
-            TRY(pull_ctrl(t));
-            float ms = 0.f;
-            CU(cudaEventElapsedTime(&ms, c->ev_t0, c->ev_t1));
-            t->last_ms += ms; t->last_launches += 1;
-            if (counted) *counted += t->h_ctrl->counted;
-            uint64_t ov = t->h_ctrl->overflow;
+            Counting r;
+            TRY(end_counting(t, 1, counted, &r));
             // what the next launch of this stream will probably create: the rate of the last
             // quarter of this one (high-coverage input finds its keys early and then stops
             // creating them; the whole-launch count would quadruple the table for nothing),
             // or everything it wanted when it ran into the limit
-            t->last_new = (hi - lo) <= kSmallBatch ? 0 : ov ? (t->size - size_before) + ov : 4 * t->h_ctrl->late_new;
-            if (ov) TRY(drain_deferred(t, ov));  // table hit its load limit: grow, then replay the deferred hashes
+            t->last_new = (hi - lo) <= kSmallBatch ? 0 : r.ov ? r.made + r.ov : 4 * t->h_ctrl->late_new;
+            if (r.ov) TRY(drain_deferred(t, c->defer, r.ov));  // table hit its load limit: grow, then replay the deferred hashes
         }
         lo = hi;
     }
@@ -1032,7 +1099,7 @@ oxg_status oxg_table_create(int device, uint32_t ksize, uint64_t capacity_hint, 
     CU(cudaMemsetAsync(t->d_ctrl, 0, sizeof(Ctrl), c->stream));
     CU(cudaMallocHost(&t->h_ctrl, sizeof(Ctrl)));
     memset(t->h_ctrl, 0, sizeof(Ctrl));
-    TRY(alloc_slots(c, t->cap, &t->slots));
+    TRY(alloc_slots(t.get(), t->cap, &t->slots));
     CU(cudaStreamSynchronize(c->stream));
     *out = t.release();
     return OXG_OK;
@@ -1043,7 +1110,7 @@ oxg_status oxg_table_destroy(oxg_table *t) {
     std::lock_guard<std::mutex> lk(t->ctx->mu);
     cudaSetDevice(t->ctx->dev);
     cudaStreamSynchronize(t->ctx->stream);
-    if (t->pooled) cudaFreeAsync(t->slots, t->ctx->stream); else cudaFree(t->slots);
+    free_slots(t, t->slots);
     cudaFree(t->d_ctrl);
     cudaFreeHost(t->h_ctrl);
     if (t->d_sketch) cudaFree(t->d_sketch);
@@ -1333,21 +1400,16 @@ static oxg_status count_list_device(oxg_table *t, const uint64_t *d_hashes, uint
         if (!optimistic) TRY(reserve_keys(t, m));
         else {
             if (over_loaded(t->size, t->cap)) TRY(grow_to_fit(t, t->size));
-            TRY(ensure_dev(&c->d_overflow, &c->overflow_cap, m));
+            TRY(ensure_dev(&c->defer.d_pairs, &c->defer.cap, m));
         }
         TRY(zero_ctrl_fields(t, kFieldCounted, kLaunchFields));
         CU(cudaEventRecord(c->ev_t0, c->stream));
-        count_hashes_kernel<<<grid_for(c, (m + 7) / 8, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t, optimistic), d_hashes + lo, m, nullptr, skip_zero);
+        count_hashes_kernel<<<grid_for(c, (m + 7) / 8, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t, optimistic ? &c->defer : nullptr), d_hashes + lo, m, nullptr, skip_zero);
         LAUNCHED();
         CU(cudaGetLastError());
-        CU(cudaEventRecord(c->ev_t1, c->stream));
-        TRY(pull_ctrl(t));
-        float ms = 0.f;
-        CU(cudaEventElapsedTime(&ms, c->ev_t0, c->ev_t1));
-        t->last_ms += ms; t->last_launches += 1;
-        if (counted) *counted += t->h_ctrl->counted;
-        const uint64_t ov = t->h_ctrl->overflow;
-        if (ov) TRY(drain_deferred(t, ov));
+        Counting r;
+        TRY(end_counting(t, 1, counted, &r));
+        if (r.ov) TRY(drain_deferred(t, c->defer, r.ov));
     }
     return OXG_OK;
 }
@@ -1369,7 +1431,7 @@ oxg_status oxg_count_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, ui
     TRY(ensure_io(c, 2 * n));
     memcpy(c->h_io, hashes, n * 8);
     CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
-    count_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t, false), c->d_io, n, new_counts ? c->d_io + n : nullptr, 0);
+    count_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, new_counts ? c->d_io + n : nullptr, 0);
     LAUNCHED();
     CU(cudaGetLastError());
     if (new_counts) CU(cudaMemcpyAsync(c->h_io + n, c->d_io + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1387,7 +1449,7 @@ oxg_status oxg_add_pairs(oxg_table *t, const uint64_t *keys, const uint64_t *val
     memcpy(c->h_io, keys, n * 8);
     memcpy(c->h_io + n, vals, n * 8);
     CU(cudaMemcpyAsync(c->d_io, c->h_io, 2 * n * 8, cudaMemcpyHostToDevice, c->stream));
-    add_pairs_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t, false), c->d_io, c->d_io + n, n);
+    add_pairs_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, c->d_io + n, n);
     LAUNCHED();
     CU(cudaGetLastError());
     // the out-of-band key's side entry must exist even when its value is 0
@@ -1403,7 +1465,7 @@ oxg_status oxg_get_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, uint
     TRY(ensure_io(c, 2 * n));
     memcpy(c->h_io, hashes, n * 8);
     CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
-    get_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t, false), c->d_io, n, c->d_io + n);
+    get_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, c->d_io + n);
     LAUNCHED();
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(c->h_io + n, c->d_io + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1415,7 +1477,7 @@ oxg_status oxg_get_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, uint
 oxg_status oxg_set_hash(oxg_table *t, uint64_t hash, uint64_t value) {
     ENTER(t);
     TRY(reserve_keys(t, 1));
-    set_hash_kernel<<<1, 32, 0, c->stream>>>(view_of(t, false), hash, value);
+    set_hash_kernel<<<1, 32, 0, c->stream>>>(view_of(t), hash, value);
     LAUNCHED();
     CU(cudaGetLastError());
     return pull_ctrl(t);
@@ -1431,7 +1493,7 @@ oxg_status oxg_erase_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, ui
     CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
     if (n < 256) {
         // the reference's usage: one key per call (drop / drop_hash, src/lib.rs:197-224)
-        erase_hashes_kernel<<<1, 32, 0, c->stream>>>(view_of(t, false), c->d_io, n);
+        erase_hashes_kernel<<<1, 32, 0, c->stream>>>(view_of(t), c->d_io, n);
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
@@ -1445,27 +1507,12 @@ oxg_status oxg_erase_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, ui
     CU(cudaMalloc(&d_doomed, words * 4));
     CU(cudaMemsetAsync(d_doomed, 0, words * 4, c->stream));
     TRY(zero_ctrl_fields(t, kFieldScratch, 1));
-    erase_mark_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t, false), c->d_io, n, d_doomed);
+    erase_mark_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, d_doomed);
     LAUNCHED();
-    ulonglong2 *fresh = nullptr;
-    TRY(alloc_slots(c, t->cap, &fresh, t->pooled));
-    ulonglong2 *old = t->slots;
-    t->slots = fresh;
-    erase_rebuild_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t, false), d_doomed);
-    LAUNCHED();
-    CU(cudaGetLastError());
-    TRY(pull_ctrl(t));
-    if (t->pooled) CU(cudaFreeAsync(old, c->stream)); else CU(cudaFree(old));
+    TRY(rebuild_slots(t, [&](const ulonglong2 *old) {
+        erase_rebuild_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t), d_doomed);
+    }, [&](uint64_t) { return std::find(hashes, hashes + n, kEmpty) != hashes + n; }, n_removed));
     CU(cudaFree(d_doomed));
-    uint64_t removed = t->h_ctrl->scratch[0];
-    t->h_ctrl->size -= removed;
-    if (t->h_ctrl->side_present && std::find(hashes, hashes + n, kEmpty) != hashes + n) {
-        t->h_ctrl->side_present = 0; t->h_ctrl->side_count = 0; ++removed;
-    }
-    t->size = t->h_ctrl->size;
-    CU(cudaMemcpyAsync(t->d_ctrl, t->h_ctrl, offsetof(Ctrl, counted), cudaMemcpyHostToDevice, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (n_removed) *n_removed = removed;
     return OXG_OK;
 }
 
@@ -1473,28 +1520,10 @@ oxg_status oxg_cut(oxg_table *t, int mode, uint64_t thresh, uint64_t *n_removed)
     ENTER(t);
     if (mode != 0 && mode != 1) return fail(OXG_ERR_INVALID, "mode must be 0 (mincut) or 1 (maxcut)");
     TRY(pull_ctrl(t));
-    uint64_t removed = 0;
-    ulonglong2 *fresh = nullptr;
-    TRY(alloc_slots(c, t->cap, &fresh, t->pooled));
-    ulonglong2 *old = t->slots;
-    t->slots = fresh;
     TRY(zero_ctrl_fields(t, kFieldScratch, 1));
-    cut_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t, false), mode, thresh);
-    LAUNCHED();
-    CU(cudaGetLastError());
-    TRY(pull_ctrl(t));
-    if (t->pooled) CU(cudaFreeAsync(old, c->stream)); else CU(cudaFree(old));
-    removed = t->h_ctrl->scratch[0];
-    t->h_ctrl->size -= removed;
-    if (t->h_ctrl->side_present) {
-        const uint64_t v = t->h_ctrl->side_count;
-        if (mode == 0 ? v < thresh : v > thresh) { t->h_ctrl->side_present = 0; t->h_ctrl->side_count = 0; ++removed; }
-    }
-    t->size = t->h_ctrl->size;
-    CU(cudaMemcpyAsync(t->d_ctrl, t->h_ctrl, offsetof(Ctrl, counted), cudaMemcpyHostToDevice, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (n_removed) *n_removed = removed;
-    return OXG_OK;
+    return rebuild_slots(t, [&](const ulonglong2 *old) {
+        cut_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t), mode, thresh);
+    }, [&](uint64_t v) { return mode == 0 ? v < thresh : v > thresh; }, n_removed);
 }
 
 // ---- scans -------------------------------------------------------------------
@@ -1510,7 +1539,7 @@ static oxg_status run_stats(oxg_table *t, bool histo, oxg_stats *st, uint64_t *n
         init.scratch[2] = ~0ULL;
         memcpy(t->h_ctrl->scratch, init.scratch, sizeof init.scratch);
         CU(cudaMemcpyAsync(t->d_ctrl->scratch, t->h_ctrl->scratch, sizeof init.scratch, cudaMemcpyHostToDevice, c->stream));
-        stats_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t, false), histo ? c->d_dense : nullptr, c->d_big, c->big_cap);
+        stats_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), histo ? c->d_dense : nullptr, c->d_big, c->big_cap);
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
@@ -1583,7 +1612,7 @@ oxg_status oxg_table_digest(oxg_table *t, int n_ranks, int rank, uint64_t out[5]
     int lg = 0;
     while ((1 << lg) < n_ranks) ++lg;
     CU(cudaMemsetAsync(t->d_ctrl->scratch, 0, 5 * 8, c->stream));
-    digest_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t, false), 64 - lg, (uint64_t)rank);
+    digest_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), 64 - lg, (uint64_t)rank);
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(t));
@@ -1733,7 +1762,7 @@ static oxg_status setop_sizes_locked(oxg_table *a, oxg_table *b, uint64_t *inter
     DeviceCtx *c = a->ctx;
     TRY(pull_ctrl(b));
     TRY(zero_ctrl_fields(a, kFieldScratch, 1));
-    setop_count_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a, false), view_of(b, false));
+    setop_count_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b));
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(a));
@@ -1775,7 +1804,7 @@ oxg_status oxg_setop_export(oxg_table *a, oxg_table *b, int op, uint64_t *keys_o
     CU(cudaMalloc(&d_cnt, 8));
     CU(cudaMemsetAsync(d_cnt, 0, 8, c->stream));
     auto pass = [&](oxg_table *x, oxg_table *y, int want) -> oxg_status {
-        setop_export_kernel<<<grid_for(c, x->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(x, false), view_of(y, false), want, d_out, room, d_cnt);
+        setop_export_kernel<<<grid_for(c, x->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(x), view_of(y), want, d_out, room, d_cnt);
         LAUNCHED();
         CU(cudaGetLastError());
         return OXG_OK;
@@ -1819,11 +1848,11 @@ oxg_status oxg_cosine(oxg_table *a, oxg_table *b, double *out) {
     if (na == 0 || nb == 0) { *out = 0.0; return OXG_OK; }  // src/lib.rs:729-731
     CU(cudaMemsetAsync(c->d_f64, 0, 4 * sizeof(double), c->stream));
     TRY(zero_ctrl_fields(a, kFieldScratch, 1));
-    cosine_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a, false), view_of(b, false), c->d_f64);
+    cosine_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b), c->d_f64);
     LAUNCHED();
-    TableView none = view_of(a, false);
+    TableView none = view_of(a);
     none.slots = nullptr;  // norm-only pass over b: adds nothing to any dot product
-    cosine_kernel<<<grid_for(c, b->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b, false), none, c->d_f64 + 1);
+    cosine_kernel<<<grid_for(c, b->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b), none, c->d_f64 + 1);
     LAUNCHED();
     CU(cudaGetLastError());
     double sq[2];
@@ -1849,7 +1878,7 @@ oxg_status oxg_merge(oxg_table *dst, oxg_table *src, uint64_t *counts_added, uin
     TRY(pull_ctrl(src));
     TRY(reserve_keys(dst, src->h_ctrl->size));
     TRY(zero_ctrl_fields(dst, kFieldScratch, 2));
-    merge_kernel<<<grid_for(c, src->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(dst, false), view_of(src, false));
+    merge_kernel<<<grid_for(c, src->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(dst), view_of(src));
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(dst));
