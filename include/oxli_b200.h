@@ -228,6 +228,21 @@ oxg_status oxg_shard_consume_batch_device(oxg_shard *s, const uint8_t *d_bases,
                                           const uint64_t *d_offsets, uint64_t n_reads,
                                           uint64_t total_bases, int skip_bad, uint64_t *counted,
                                           uint64_t *absorbed, int64_t *err_read, uint64_t *err_pos);
+/* get_hash_array on the whole sharded table (src/lib.rs:185-194), COLLECTIVE: every
+ * rank calls it with its own list (n may be 0, and may differ between ranks).
+ * counts_out[i] = count of hashes[i] in the table (0 when absent), in the order of
+ * the queries.  Any u64 is a legal query: 0, 2^64-1 (its owner's side entry), and
+ * duplicates.  Each query goes to the rank that owns it and is answered there: the
+ * queries travel in rounds of round_windows per rank, the same exchange rounds a
+ * consume call runs, so lookups and consume calls may follow each other in any
+ * order.  Plain-table calls on oxg_shard_table(s) made before the call are seen.
+ * A call refused for its arguments (null lists with n > 0, an unconnected shard, a
+ * device list in another device's memory) returns OXG_ERR_INVALID before it takes
+ * part in any exchange. */
+oxg_status oxg_shard_get_hashes(oxg_shard *s, const uint64_t *hashes, uint64_t n, uint64_t *counts_out);
+/* same, with both lists resident in this shard's HBM */
+oxg_status oxg_shard_get_hashes_device(oxg_shard *s, const uint64_t *d_hashes, uint64_t n,
+                                       uint64_t *d_counts_out);
 /* time of the last consume call on this shard's stream (device variant: CUDA events;
  * host variant: wall clock of the call) and its number of exchange rounds */
 oxg_status oxg_shard_last_ms(const oxg_shard *s, float *ms, uint64_t *rounds);

@@ -78,6 +78,8 @@ SIGNATURES = {
     "oxg_shard_connect_local": (C.c_int, [C.POINTER(vp), C.c_int]),
     "oxg_shard_consume_batch": (C.c_int, [vp, vp, vp, u64, C.c_int, u64p, u64p, C.POINTER(C.c_int64), u64p]),
     "oxg_shard_consume_batch_device": (C.c_int, [vp, vp, vp, u64, u64, C.c_int, u64p, u64p, C.POINTER(C.c_int64), u64p]),
+    "oxg_shard_get_hashes": (C.c_int, [vp, vp, u64, vp]),
+    "oxg_shard_get_hashes_device": (C.c_int, [vp, vp, u64, vp]),
     "oxg_shard_last_ms": (C.c_int, [vp, C.POINTER(C.c_float), u64p]),
     "oxg_shard_stats": (C.c_int, [vp, C.POINTER(oxg_stats)]),
     "oxg_shard_histo": (C.c_int, [vp, vp, vp, u64, u64p]),
@@ -419,6 +421,16 @@ class Shard:
         if st not in (OK, ERR_BAD_KMER):
             check(st)
         return st, int(cn.value), int(ab.value), int(er.value), int(ep.value)
+
+    def get_hashes(self, hashes) -> np.ndarray:
+        """Counts of this rank's queries in the whole table (collective)."""
+        h = np.ascontiguousarray(hashes, dtype=np.uint64)
+        out = np.zeros(len(h), dtype=np.uint64)
+        check(lib.oxg_shard_get_hashes(self._h, _ptr(h), len(h), _ptr(out)))
+        return out
+
+    def get_hashes_device(self, d_hashes: int, n: int, d_out: int) -> None:
+        check(lib.oxg_shard_get_hashes_device(self._h, d_hashes, n, d_out))
 
     def last_ms(self) -> tuple[float, int]:
         ms, n = C.c_float(), u64()

@@ -27,6 +27,7 @@
 #include "consume.cuh"
 #include "scatter.cuh"
 #include "klist.h"
+#include "lookup.cuh"
 #include "shard.cuh"
 #include "sortexport.cuh"
 #include "tableops.cuh"

@@ -4,9 +4,11 @@
 The table is sharded by the high bits of the hash -- owner(h) = h >> (64 - log2 N) -- as
 BASELINE.json's north_star prescribes; every rank hashes its own reads, leaves the hashes in
 fragments per (owner, table partition) in its own HBM, and each owner's aggregation kernel
-pulls its fragments from all ranks over NVLink (peer-mapped memory) and counts them.  All of
-that, including the rank-to-rank flags and the reductions (len / sum / min / max, histo,
-|A & B|, jaccard: reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
+pulls its fragments from all ranks over NVLink (peer-mapped memory) and counts them.  Point
+queries (get / get_hash / get_hash_array, src/lib.rs:170-194) take the same route: every rank
+sends its hashes to their owners, which answer them in place.  All of that, including the
+rank-to-rank flags and the reductions (len / sum / min / max, histo, |A & B|, jaccard, digests:
+reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
 
 Nothing here imports torch.  A launcher (bench.py, the tests, a user's torchrun script)
 provides ONE thing: `exchange(blob: bytes) -> list[bytes]`, an all-gather of a 64-byte CUDA IPC
@@ -94,6 +96,27 @@ class ShardedTable:
         if st != 0:
             raise BadKmerError(ep, er)
         return counted
+
+    # -- lookups (collective) ----------------------------------------------------------
+    def get_hash_array(self, hashes) -> np.ndarray:
+        """Counts of this rank's hashes in the whole table (0 when absent), in order
+        (src/lib.rs:185-194).  Every rank calls it with its own list, empty ones included; each
+        hash is answered by the rank that owns it."""
+        return self.engine.get_hashes(hashes)
+
+    def get_hash(self, h: int) -> int:
+        return int(self.get_hash_array([h])[0])
+
+    def get(self, kmer: str) -> int:
+        """Count of a k-mer (src/lib.rs:170-182), hashed through this rank's shard table.  A k-mer
+        of the wrong length or with a non-ACGT base raises before the lookup starts; the other
+        ranks' lookup then fails once the exchange gives up waiting for this one."""
+        if len(kmer) != self.ksize:
+            raise ValueError("kmer size does not match count table ksize")
+        h = self.engine.table.hash_windows(kmer.encode())
+        if h[0] == 0:  # (the reference panics here; the drop-in raises the same error)
+            raise RuntimeError(f"invalid DNA character in input k-mer: {kmer}")
+        return self.get_hash(int(h[0]))
 
     # -- reductions (collective) ------------------------------------------------------
     def stats(self) -> dict:
