@@ -527,6 +527,10 @@ oxg_status rebuild_slots(oxg_table *t, const Rebuild &rebuild, const SideDrops &
 // high-coverage input every new key is deferred many times).  Grow geometrically -- room for
 // at most as many new keys as the table already holds -- and replay; a replay that runs into
 // the limit again defers into the second list, the two swap and the loop goes round once more.
+// A replay that defers again although the table did not grow met a probe run longer than
+// kMaxProbe: keys that share one home at every capacity, which no growth separates.  The last
+// replay then gets room for every deferred key and no deferral list: without one there is no
+// probe limit and no load limit, so it places them all.
 oxg_status drain_deferred(oxg_table *t, DeferLists &d, uint64_t ov) {
     NvtxRange range("oxg:replay deferred");
     DeviceCtx *c = t->ctx;
@@ -536,14 +540,16 @@ oxg_status drain_deferred(oxg_table *t, DeferLists &d, uint64_t ov) {
         const uint64_t room = std::min<uint64_t>(ov, std::max<uint64_t>(t->size, 1ull << 20));
         const uint64_t cap_before = t->cap;
         TRY(grow_to_fit(t, t->size + room));
-        // deferred for a probe run that would not end rather than for load: double regardless
-        if (t->cap == cap_before && ov >= prev) TRY(grow_to_fit(t, t->cap));
+        const bool last = t->cap == cap_before && ov >= prev;
+        if (last) TRY(grow_to_fit(t, t->size + ov));
         prev = ov;
-        if (!d.fixed) TRY(ensure_dev(&d.d_pairs2, &d.cap2, ov));
-        else if (d.cap2 < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
+        if (!last) {
+            if (!d.fixed) TRY(ensure_dev(&d.d_pairs2, &d.cap2, ov));
+            else if (d.cap2 < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
+        }
         TRY(zero_ctrl_fields(t, offsetof(Ctrl, overflow) / 8, 1));
         TableView v = view_of(t);
-        v.overflow = d.d_pairs2; v.overflow_cap = d.cap2;
+        if (!last) { v.overflow = d.d_pairs2; v.overflow_cap = d.cap2; }
         replay_pairs_kernel<<<grid_for(c, (ov + 3) / 4, kOpThreads, 8), kOpThreads, 0, c->stream>>>(v, d.d_pairs, ov);
         LAUNCHED();
         CU(cudaGetLastError());
