@@ -172,8 +172,10 @@ oxg_status oxg_merge(oxg_table *dst, oxg_table *src, uint64_t *counts_added, uin
 /* ---- hash-sharded table across the GPUs of one node ------------------------
  * The north_star's multi-GPU layout: shard r of N owns the hashes with
  * h >> (64 - log2 N) == r; the reference's primitive for combining partial
- * tables is KmerCountTable::add (src/lib.rs:778-837), here replaced by routing
- * every hash to its owner before it is counted.  One oxg_shard per GPU.  The
+ * tables is KmerCountTable::add (src/lib.rs:778-837).  Reads need no such step:
+ * consume routes every hash to its owner before it is counted.  Tables counted
+ * elsewhere (on one GPU, or another sharded table) are added with
+ * oxg_shard_merge_table / oxg_shard_merge below.  One oxg_shard per GPU.  The
  * shards of a table live in one process each (the usual arrangement, connected
  * through CUDA IPC handles that the launcher passes around) or in one process
  * together (oxg_shard_connect_local; also how a single-GPU box tests N > 1).
@@ -243,6 +245,26 @@ oxg_status oxg_shard_get_hashes(oxg_shard *s, const uint64_t *hashes, uint64_t n
 /* same, with both lists resident in this shard's HBM */
 oxg_status oxg_shard_get_hashes_device(oxg_shard *s, const uint64_t *d_hashes, uint64_t n,
                                        uint64_t *d_counts_out);
+/* KmerCountTable::add (src/lib.rs:778-837) into a sharded table, COLLECTIVE: every rank passes its
+ * own plain table `src` on this shard's device, or NULL to add nothing.  counts[h] += src[h] for every
+ * key of every rank's table: keys held with count 0 are created with 0, 2^64-1 included (its
+ * owner's side entry), counts wrap mod 2^64.  src is not modified.  *counts_added and *new_keys
+ * (nullable) are totals over the whole table, identical on every rank; new_keys counts, as
+ * oxg_merge does, contributions to a key whose count was 0 just before them.  When the same key
+ * comes from several ranks in one call, the order of the additions is unspecified: new_keys is
+ * then the sum of what adding the ranks' tables one after another would report when no
+ * contributed count is 0, and what some serial order would report otherwise.  Each pair travels
+ * to the rank that owns its key in exchange rounds of round_windows slots of src, the same rounds
+ * consume and lookups run, so all three may follow each other in any order; every owner grows
+ * once, before the first round, to hold every key it may receive.  Plain-table calls on src and
+ * on oxg_shard_table(dst) made before the call are seen.  Refused before any exchange, with the
+ * table unchanged: an unconnected dst, a src on another device or src == oxg_shard_table(dst)
+ * (OXG_ERR_INVALID), a different ksize (OXG_ERR_WRONG_KSIZE). */
+oxg_status oxg_shard_merge_table(oxg_shard *dst, oxg_table *src, uint64_t *counts_added, uint64_t *new_keys);
+/* the same for a sharded src with the same n_ranks, rank and device on every rank: each rank
+ * merges src's shard into its own, nothing crosses between GPUs except the two totals.  Also
+ * refused (OXG_ERR_INVALID): src == dst, or src sharded another way. */
+oxg_status oxg_shard_merge(oxg_shard *dst, oxg_shard *src, uint64_t *counts_added, uint64_t *new_keys);
 /* time of the last consume call on this shard's stream (device variant: CUDA events;
  * host variant: wall clock of the call) and its number of exchange rounds */
 oxg_status oxg_shard_last_ms(const oxg_shard *s, float *ms, uint64_t *rounds);

@@ -80,6 +80,8 @@ SIGNATURES = {
     "oxg_shard_consume_batch_device": (C.c_int, [vp, vp, vp, u64, u64, C.c_int, u64p, u64p, C.POINTER(C.c_int64), u64p]),
     "oxg_shard_get_hashes": (C.c_int, [vp, vp, u64, vp]),
     "oxg_shard_get_hashes_device": (C.c_int, [vp, vp, u64, vp]),
+    "oxg_shard_merge_table": (C.c_int, [vp, vp, u64p, u64p]),
+    "oxg_shard_merge": (C.c_int, [vp, vp, u64p, u64p]),
     "oxg_shard_last_ms": (C.c_int, [vp, C.POINTER(C.c_float), u64p]),
     "oxg_shard_stats": (C.c_int, [vp, C.POINTER(oxg_stats)]),
     "oxg_shard_histo": (C.c_int, [vp, vp, vp, u64, u64p]),
@@ -431,6 +433,19 @@ class Shard:
 
     def get_hashes_device(self, d_hashes: int, n: int, d_out: int) -> None:
         check(lib.oxg_shard_get_hashes_device(self._h, d_hashes, n, d_out))
+
+    def merge_table(self, table: Table | None) -> tuple[int, int]:
+        """Adds this rank's plain table (None: nothing) into the sharded table (collective).
+        Returns (counts_added, new_keys) over the whole table."""
+        a, n = u64(), u64()
+        check(lib.oxg_shard_merge_table(self._h, None if table is None else table._h, C.byref(a), C.byref(n)))
+        return int(a.value), int(n.value)
+
+    def merge(self, other: "Shard") -> tuple[int, int]:
+        """Adds the other sharded table's shard of this rank into this one (collective)."""
+        a, n = u64(), u64()
+        check(lib.oxg_shard_merge(self._h, other._h, C.byref(a), C.byref(n)))
+        return int(a.value), int(n.value)
 
     def last_ms(self) -> tuple[float, int]:
         ms, n = C.c_float(), u64()

@@ -1,10 +1,16 @@
-// lookup.cuh -- device side of the sharded table's lookup round (oxg_shard_get_hashes*).
+// lookup.cuh -- device side of the sharded table's lookup and merge rounds (oxg_shard_get_hashes*,
+// oxg_shard_merge_table).
 //
-// A round: every rank sorts its queries by owner into the fragment region of its own exchange
-// area (route_*), each owner reads its segment of every rank's queries through the peer mapping,
-// looks the keys up in its table and writes each count over its key (answer_queries_kernel), and
-// every rank reads its answers back in the order of its queries (gather_answers_kernel).  Each key
-// slot is read and rewritten by exactly one owner, so the answers need no memory of their own.
+// A lookup round: every rank sorts its queries by owner into the fragment region of its own
+// exchange area (route_*), each owner reads its segment of every rank's queries through the peer
+// mapping, looks the keys up in its table and writes each count over its key
+// (answer_queries_kernel), and every rank reads its answers back in the order of its queries
+// (gather_answers_kernel).  Each key slot is read and rewritten by exactly one owner, so the
+// answers need no memory of their own.
+//
+// A merge round routes the occupied slots of a range of a plain table instead: keys to the
+// fragment region, their counts to the same positions of the spill region, and each owner adds
+// its segments into its table (apply_pairs_kernel).
 #pragma once
 #include "shard.cuh"
 #include "tableops.cuh"
@@ -22,9 +28,36 @@ __device__ __forceinline__ uint32_t owner_bin(uint64_t h, uint32_t owner_shift) 
     return owner_shift >= 64 ? 0u : (uint32_t)(h >> owner_shift);
 }
 
-// Route, step 1.  CTA c takes the queries [c * chunk, (c + 1) * chunk) of the round and counts
-// them per owner in shared memory: bins[o * gridDim.x + c] (one shared atomic per warp and owner).
-__global__ void __launch_bounds__(kRouteThreads) route_count_kernel(const uint64_t *__restrict__ q, uint64_t m, uint64_t chunk,
+// Where a route's keys come from.  A list of queries (lookups): every entry is a key, and
+// out[i] = the slot query i went to (pos) ...
+struct RouteList {
+    using In = uint64_t;
+    using Out = uint32_t;
+    static __device__ __forceinline__ uint64_t key(const In *q, uint64_t i) { return q[i]; }
+    static __device__ __forceinline__ bool live(uint64_t) { return true; }
+    static __device__ __forceinline__ uint32_t bin(const In *q, uint64_t i, uint32_t owner_shift) { return owner_bin(q[i], owner_shift); }
+    static __device__ __forceinline__ void place(const In *, uint64_t i, uint32_t at, Out *out) { out[i] = at; }
+};
+// ... or a range of table slots (merges): empty slots go nowhere (so the out-of-band key never
+// travels), and each key's count goes to the same position of out (the spill region) as the key
+// goes to in frag.
+struct RouteSlots {
+    using In = ulonglong2;
+    using Out = uint64_t;
+    static __device__ __forceinline__ uint64_t key(const In *q, uint64_t i) { return q[i].x; }
+    static __device__ __forceinline__ bool live(uint64_t h) { return h != kEmpty; }
+    static __device__ __forceinline__ uint32_t bin(const In *q, uint64_t i, uint32_t owner_shift) {
+        const uint64_t h = key(q, i);
+        return live(h) ? owner_bin(h, owner_shift) : kShardMaxRanks;
+    }
+    static __device__ __forceinline__ void place(const In *q, uint64_t i, uint32_t at, Out *out) { out[at] = q[i].y; }
+};
+
+// Route, step 1.  CTA c takes the entries [c * chunk, (c + 1) * chunk) of the round and counts
+// the keys among them per owner in shared memory: bins[o * gridDim.x + c] (one shared atomic per
+// warp and owner).
+template <class Src>
+__global__ void __launch_bounds__(kRouteThreads) route_count_kernel(const typename Src::In *__restrict__ q, uint64_t m, uint64_t chunk,
                                                                     uint32_t owner_shift, uint32_t n_own, uint32_t *__restrict__ bins) {
     __shared__ uint32_t hist[kShardMaxRanks];
     if (threadIdx.x < kShardMaxRanks) hist[threadIdx.x] = 0;
@@ -36,7 +69,7 @@ __global__ void __launch_bounds__(kRouteThreads) route_count_kernel(const uint64
 #pragma unroll
         for (int u = 0; u < kRouteU; ++u) {
             const uint64_t i = t0 + u * kRouteThreads + threadIdx.x;
-            o[u] = i < hi ? owner_bin(q[i], owner_shift) : kShardMaxRanks;
+            o[u] = i < hi ? Src::bin(q, i, owner_shift) : kShardMaxRanks;
         }
 #pragma unroll
         for (int u = 0; u < kRouteU; ++u) {
@@ -50,9 +83,9 @@ __global__ void __launch_bounds__(kRouteThreads) route_count_kernel(const uint64
 
 // Route, step 2 (one CTA of kRouteScanThreads).  bins becomes its exclusive prefix sum in (owner,
 // CTA) order: the slot where CTA c's run of owner o begins.  offs[o] = first slot of owner o's
-// segment, offs[n_own] = m.
+// segment, offs[n_own] = the keys routed (the last thread's run ends at the total).
 __global__ void __launch_bounds__(kRouteScanThreads) route_scan_kernel(uint32_t *__restrict__ bins, uint32_t n_bins, uint32_t grid,
-                                                                       uint32_t n_own, uint64_t m, uint64_t *__restrict__ offs) {
+                                                                       uint32_t n_own, uint64_t *__restrict__ offs) {
     __shared__ uint32_t warp_sum_s[kRouteScanThreads / 32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t per = (n_bins + kRouteScanThreads - 1) / kRouteScanThreads;
@@ -85,16 +118,19 @@ __global__ void __launch_bounds__(kRouteScanThreads) route_scan_kernel(uint32_t 
         run += v;
     }
     __syncthreads();
-    if (threadIdx.x <= n_own) offs[threadIdx.x] = threadIdx.x < n_own ? bins[threadIdx.x * grid] : m;
+    if (threadIdx.x < n_own) offs[threadIdx.x] = bins[threadIdx.x * grid];
+    if (threadIdx.x == kRouteScanThreads - 1) offs[n_own] = run;
 }
 
-// Route, step 3: the same chunks as step 1, tile by tile in index order.  Each query goes to the
-// next slot of its owner's run in frag (stable: slots follow the queries' order), and pos[i]
-// records where.  A tile writes at most one contiguous run per owner.
-__global__ void __launch_bounds__(kRouteThreads) route_queries_kernel(const uint64_t *__restrict__ q, uint64_t m, uint64_t chunk,
+// Route, step 3: the same chunks as step 1, tile by tile in index order.  Each key goes to the
+// next slot of its owner's run in frag (stable: slots follow the entries' order), and Src::place
+// records where (a query's slot) or what (a count) in out.  A tile writes at most one contiguous
+// run per owner.
+template <class Src>
+__global__ void __launch_bounds__(kRouteThreads) route_queries_kernel(const typename Src::In *__restrict__ q, uint64_t m, uint64_t chunk,
                                                                       uint32_t owner_shift, uint32_t n_own,
                                                                       const uint32_t *__restrict__ base, uint64_t *__restrict__ frag,
-                                                                      uint32_t *__restrict__ pos) {
+                                                                      typename Src::Out *__restrict__ out) {
     constexpr int kVW = kRouteU * kRouteWarps;              // (u, warp): 32 queries each, in index order
     __shared__ uint32_t cnt[kVW][kShardMaxRanks];           // queries per (u, warp) and owner
     __shared__ uint32_t first[kVW][kShardMaxRanks];         // ... and the slot of the first of them
@@ -111,8 +147,8 @@ __global__ void __launch_bounds__(kRouteThreads) route_queries_kernel(const uint
 #pragma unroll
         for (int u = 0; u < kRouteU; ++u) {
             const uint64_t i = t0 + u * kRouteThreads + threadIdx.x;
-            h[u] = i < hi ? q[i] : 0;
-            o[u] = i < hi ? owner_bin(h[u], owner_shift) : kShardMaxRanks;
+            h[u] = i < hi ? Src::key(q, i) : 0;
+            o[u] = i < hi && Src::live(h[u]) ? owner_bin(h[u], owner_shift) : kShardMaxRanks;
         }
 #pragma unroll
         for (int u = 0; u < kRouteU; ++u) {
@@ -135,13 +171,13 @@ __global__ void __launch_bounds__(kRouteThreads) route_queries_kernel(const uint
             if (o[u] >= kShardMaxRanks) continue;
             const uint32_t at = first[u * kRouteWarps + warp][o[u]] + __popc(peers[u] & below);
             frag[at] = h[u];
-            pos[t0 + u * kRouteThreads + threadIdx.x] = at;
+            Src::place(q, t0 + u * kRouteThreads + threadIdx.x, at, out);
         }
     }
 }
 
-// Where the owner finds every rank's queries of the round: rank s's routed queries (frag) and
-// its n + 1 owner offsets (offs), both through the peer mapping.
+// Where the owner finds every rank's keys of the round: rank s's routed keys (frag) and its
+// n + 1 owner offsets (offs), both through the peer mapping.
 struct LookupSources {
     uint64_t *frag[kShardMaxRanks];
     const uint64_t *offs[kShardMaxRanks];
@@ -149,11 +185,10 @@ struct LookupSources {
 };
 
 // On the owner `me`: the segments [offs_s[me], offs_s[me + 1]) of every rank s, concatenated into
-// one grid-stride range.  Four keys per thread are loaded (coalesced, over NVLink for a peer's)
-// before table_get_many looks them up; each count is one 8-byte store over its key.
-__global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t, LookupSources src, int me) {
-    __shared__ uint64_t seg_lo[kShardMaxRanks];       // segment s starts at this slot of rank s's frag
-    __shared__ uint64_t seg_at[kShardMaxRanks + 1];   // ... and at this position of the concatenation
+// one range.  seg_lo[s] = where segment s starts in rank s's region, seg_at[s] = where it starts in
+// the concatenation (both in shared memory).  Called by every thread of the block (it
+// synchronises); returns the range's length.
+__device__ __forceinline__ uint64_t load_segments(const LookupSources &src, int me, uint64_t *seg_lo, uint64_t *seg_at) {
     if ((int)threadIdx.x < src.n) {
         const uint64_t lo = __ldcg(src.offs[threadIdx.x] + me), hi = __ldcg(src.offs[threadIdx.x] + me + 1);
         seg_lo[threadIdx.x] = lo;
@@ -165,8 +200,24 @@ __global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t,
         for (int s = 1; s <= src.n; ++s) seg_at[s] += seg_at[s - 1];
     }
     __syncthreads();
+    return seg_at[src.n];
+}
+
+// the rank whose segment holds entry i of that range: the entry is at seg_lo[s] + (i - seg_at[s])
+// of rank s's region
+__device__ __forceinline__ int segment_of(const uint64_t *seg_at, uint64_t i) {
+    int s = 0;
+    while (i >= seg_at[s + 1]) ++s;
+    return s;
+}
+
+// Answers every rank's queries of the round: four keys per thread are loaded (coalesced, over
+// NVLink for a peer's) before table_get_many looks them up; each count is one 8-byte store over
+// its key.
+__global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t, LookupSources src, int me) {
+    __shared__ uint64_t seg_lo[kShardMaxRanks], seg_at[kShardMaxRanks + 1];
     constexpr int U = 4;
-    const uint64_t total = seg_at[src.n], stride = gstride();
+    const uint64_t total = load_segments(src, me, seg_lo, seg_at), stride = gstride();
     for (uint64_t base = gtid(); base < total; base += stride * U) {
         uint64_t *p[U], key[U], cnt[U];
         uint32_t live = 0;
@@ -176,8 +227,7 @@ __global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t,
             p[j] = nullptr;
             key[j] = 0;
             if (i < total) {
-                int s = 0;
-                while (i >= seg_at[s + 1]) ++s;
+                const int s = segment_of(seg_at, i);
                 p[j] = src.frag[s] + seg_lo[s] + (i - seg_at[s]);
                 key[j] = __ldcg(p[j]);
                 live |= 1u << j;
@@ -194,6 +244,57 @@ __global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t,
 __global__ void __launch_bounds__(kOpThreads) gather_answers_kernel(const uint64_t *frag, const uint32_t *__restrict__ pos, uint64_t m,
                                                                     uint64_t *__restrict__ out) {
     for (uint64_t i = gtid(); i < m; i += gstride()) out[i] = __ldcg(frag + pos[i]);
+}
+
+// A merge round's routed pairs: the keys as a lookup's, and rank s's counts at the same positions
+// of its spill region (vals[s]).
+struct PairSources {
+    LookupSources keys;
+    const uint64_t *vals[kShardMaxRanks];
+};
+
+// On the owner `me`: counts[key] += count for every pair of every rank's segment (KmerCountTable::add,
+// src/lib.rs:778-837), four in flight per thread.  Room for every key was reserved before the
+// round (no deferral).  scratch[0] += counts added, scratch[1] += pairs whose key held 0 just
+// before them (the reference's "new keys"), size += keys created; one atomic per warp each.
+__global__ void __launch_bounds__(kOpThreads) apply_pairs_kernel(TableView t, PairSources src, int me) {
+    __shared__ uint64_t seg_lo[kShardMaxRanks], seg_at[kShardMaxRanks + 1];
+    constexpr int U = 4;
+    const uint64_t total = load_segments(src.keys, me, seg_lo, seg_at), stride = gstride();
+    uint64_t added = 0, fresh = 0;
+    uint32_t created = 0;
+    for (uint64_t base = gtid(); base < total; base += stride * U) {
+        uint64_t key[U], val[U], before[U];
+        uint32_t live = 0;
+#pragma unroll
+        for (int j = 0; j < U; ++j) {
+            const uint64_t i = base + j * stride;
+            key[j] = 0;
+            val[j] = 0;
+            if (i < total) {
+                const int s = segment_of(seg_at, i);
+                const uint64_t at = seg_lo[s] + (i - seg_at[s]);
+                key[j] = __ldcg(src.keys.frag[s] + at);
+                val[j] = __ldcg(src.vals[s] + at);
+                live |= 1u << j;
+            }
+        }
+        created += table_add_fetch_many<U>(t, key, val, live, before);
+#pragma unroll
+        for (int j = 0; j < U; ++j)
+            if ((live >> j) & 1) {
+                added += val[j];
+                fresh += before[j] == 0 ? 1 : 0;
+            }
+    }
+    added = warp_sum(added);
+    fresh = warp_sum(fresh);
+    const uint64_t cr = warp_sum(created);
+    if ((threadIdx.x & 31) == 0) {
+        if (added) atomicAdd((unsigned long long *)&t.ctrl->scratch[0], (unsigned long long)added);
+        if (fresh) atomicAdd((unsigned long long *)&t.ctrl->scratch[1], (unsigned long long)fresh);
+        if (cr) atomicAdd((unsigned long long *)&t.ctrl->size, (unsigned long long)cr);
+    }
 }
 
 }  // namespace oxg

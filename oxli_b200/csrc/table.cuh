@@ -198,6 +198,32 @@ __device__ __forceinline__ uint64_t table_add_fetch(const TableView &t, uint64_t
     }
 }
 
+// counts[key[u]] += inc[u] for the lanes' U live entries, as table_add_many, and before[u] = the
+// count the key held just before its increment (0 for a key created here).  Never defers: the
+// caller reserved room.  Returns the number of keys created.
+template <int U>
+__device__ __forceinline__ uint32_t table_add_fetch_many(const TableView &t, const uint64_t (&key)[U], const uint64_t (&inc)[U],
+                                                         uint32_t live, uint64_t (&before)[U]) {
+    uint64_t idx[U];
+    ulonglong2 a[U], b[U];
+    uint32_t created = 0;
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        before[u] = 0;
+        if (((live >> u) & 1u) && key[u] == kEmpty) { before[u] = table_add_fetch(t, key[u], inc[u], &created) - inc[u]; live &= ~(1u << u); }
+        idx[u] = t.home(key[u]);
+        if ((live >> u) & 1u) load_pair(t.slots + idx[u], a[u], b[u]);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        if (!((live >> u) & 1u)) continue;
+        if (a[u].x == key[u]) before[u] = atomicAdd((unsigned long long *)&t.slots[idx[u]].y, (unsigned long long)inc[u]);
+        else if (b[u].x == key[u]) before[u] = atomicAdd((unsigned long long *)&t.slots[idx[u] + 1].y, (unsigned long long)inc[u]);
+        else before[u] = table_add_fetch(t, key[u], inc[u], &created) - inc[u];
+    }
+    return created;
+}
+
 // slot index of key, or -1
 __device__ __forceinline__ int64_t table_find(const TableView &t, uint64_t key) {
     uint64_t i = t.home(key);

@@ -6,7 +6,10 @@ BASELINE.json's north_star prescribes; every rank hashes its own reads, leaves t
 fragments per (owner, table partition) in its own HBM, and each owner's aggregation kernel
 pulls its fragments from all ranks over NVLink (peer-mapped memory) and counts them.  Point
 queries (get / get_hash / get_hash_array, src/lib.rs:170-194) take the same route: every rank
-sends its hashes to their owners, which answer them in place.  All of that, including the
+sends its hashes to their owners, which answer them in place.  So does `add` (KmerCountTable::add,
+src/lib.rs:778-837) of a table counted on one GPU: every (key, count) of each rank's plain table
+goes to its owner and is added there; a second sharded table is added rank by rank, its shards
+already on their owners.  All of that, including the
 rank-to-rank flags and the reductions (len / sum / min / max, histo, |A & B|, jaccard, digests:
 reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
 
@@ -117,6 +120,23 @@ class ShardedTable:
         if h[0] == 0:  # (the reference panics here; the drop-in raises the same error)
             raise RuntimeError(f"invalid DNA character in input k-mer: {kmer}")
         return self.get_hash(int(h[0]))
+
+    # -- merges (collective) -----------------------------------------------------------
+    def add(self, other) -> tuple[int, int]:
+        """KmerCountTable::add (src/lib.rs:778-837): counts[h] += other[h] for every key of
+        `other`.  Every rank calls it: with another ShardedTable (same world, rank by rank; each
+        rank adds that table's shard into its own), or each with its own plain `_capi.Table` on
+        this rank's device, or None to add nothing (each key of a plain table is sent to the rank
+        that owns it).  `other` is not modified.  Returns (counts_added, new_keys) over the whole
+        table, the two numbers the reference prints; this class prints nothing (the drop-in
+        KmerCountTable does)."""
+        if other is self or other is self.engine.table:
+            raise ValueError("cannot add a table to itself")
+        if other is not None and other.ksize != self.ksize:
+            raise ValueError("KmerCountTables must have the same ksize")
+        if isinstance(other, ShardedTable):
+            return self.engine.merge(other.engine)
+        return self.engine.merge_table(other)
 
     # -- reductions (collective) ------------------------------------------------------
     def stats(self) -> dict:
