@@ -175,7 +175,8 @@ oxg_status oxg_merge(oxg_table *dst, oxg_table *src, uint64_t *counts_added, uin
  * tables is KmerCountTable::add (src/lib.rs:778-837).  Reads need no such step:
  * consume routes every hash to its owner before it is counted.  Tables counted
  * elsewhere (on one GPU, or another sharded table) are added with
- * oxg_shard_merge_table / oxg_shard_merge below.  One oxg_shard per GPU.  The
+ * oxg_shard_merge_table / oxg_shard_merge below, and keys are removed with
+ * oxg_shard_erase_hashes* / oxg_shard_cut.  One oxg_shard per GPU.  The
  * shards of a table live in one process each (the usual arrangement, connected
  * through CUDA IPC handles that the launcher passes around) or in one process
  * together (oxg_shard_connect_local; also how a single-GPU box tests N > 1).
@@ -265,6 +266,29 @@ oxg_status oxg_shard_merge_table(oxg_shard *dst, oxg_table *src, uint64_t *count
  * merges src's shard into its own, nothing crosses between GPUs except the two totals.  Also
  * refused (OXG_ERR_INVALID): src == dst, or src sharded another way. */
 oxg_status oxg_shard_merge(oxg_shard *dst, oxg_shard *src, uint64_t *counts_added, uint64_t *new_keys);
+/* drop_hash for a list on the whole sharded table (src/lib.rs:197-224), COLLECTIVE: every rank
+ * passes its own list (n may be 0, and may differ between ranks).  Each hash goes to the rank that
+ * owns it, which removes it.  Any u64 is a legal key: 0, duplicates, and 2^64-1 (its owner's side
+ * entry); absent keys are ignored.  *n_removed (nullable) = distinct keys removed from the whole
+ * table, 2^64-1 included, identical on every rank: a key listed several times, by one rank or by
+ * several, counts once.  The keys travel in exchange rounds of round_windows per rank, the same
+ * rounds consume, lookups and merges run, so all four may follow each other in any order.  Fewer
+ * than 256 keys over all ranks are erased in place, one at a time (the reference's drop /
+ * drop_hash); a longer list marks its keys' slots and each owner rebuilds its table once, at the
+ * same capacity (the call never grows the table).  Plain-table calls on oxg_shard_table(s) made
+ * before the call are seen.  Refused before any exchange, with the table unchanged
+ * (OXG_ERR_INVALID): a null list with n > 0, an unconnected shard, a device list outside this
+ * shard's device memory.  The slot bitmap (cap / 8 bytes) is reserved before the first exchange
+ * too: when that fails the call returns OXG_ERR_NOMEM (OXG_ERR_CUDA for any other CUDA error),
+ * again with the table unchanged. */
+oxg_status oxg_shard_erase_hashes(oxg_shard *s, const uint64_t *hashes, uint64_t n, uint64_t *n_removed);
+/* same, with the list resident in this shard's HBM (left as it was) */
+oxg_status oxg_shard_erase_hashes_device(oxg_shard *s, const uint64_t *d_hashes, uint64_t n, uint64_t *n_removed);
+/* mincut (mode 0: drop counts < thresh) / maxcut (mode 1: drop counts > thresh) on every shard
+ * (src/lib.rs:227-267), COLLECTIVE; *n_removed (nullable) = keys removed from the whole table,
+ * 2^64-1 included, identical on every rank.  Refused before any exchange (OXG_ERR_INVALID): an
+ * unconnected shard, a mode other than 0 / 1. */
+oxg_status oxg_shard_cut(oxg_shard *s, int mode, uint64_t thresh, uint64_t *n_removed);
 /* time of the last consume call on this shard's stream (device variant: CUDA events;
  * host variant: wall clock of the call) and its number of exchange rounds */
 oxg_status oxg_shard_last_ms(const oxg_shard *s, float *ms, uint64_t *rounds);

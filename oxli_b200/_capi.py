@@ -82,6 +82,9 @@ SIGNATURES = {
     "oxg_shard_get_hashes_device": (C.c_int, [vp, vp, u64, vp]),
     "oxg_shard_merge_table": (C.c_int, [vp, vp, u64p, u64p]),
     "oxg_shard_merge": (C.c_int, [vp, vp, u64p, u64p]),
+    "oxg_shard_erase_hashes": (C.c_int, [vp, vp, u64, u64p]),
+    "oxg_shard_erase_hashes_device": (C.c_int, [vp, vp, u64, u64p]),
+    "oxg_shard_cut": (C.c_int, [vp, C.c_int, u64, u64p]),
     "oxg_shard_last_ms": (C.c_int, [vp, C.POINTER(C.c_float), u64p]),
     "oxg_shard_stats": (C.c_int, [vp, C.POINTER(oxg_stats)]),
     "oxg_shard_histo": (C.c_int, [vp, vp, vp, u64, u64p]),
@@ -446,6 +449,25 @@ class Shard:
         a, n = u64(), u64()
         check(lib.oxg_shard_merge(self._h, other._h, C.byref(a), C.byref(n)))
         return int(a.value), int(n.value)
+
+    def erase_hashes(self, hashes) -> int:
+        """Removes this rank's keys from the whole table (collective).  Returns the distinct keys
+        removed over the whole table."""
+        h = np.ascontiguousarray(hashes, dtype=np.uint64)
+        n = u64()
+        check(lib.oxg_shard_erase_hashes(self._h, _ptr(h), len(h), C.byref(n)))
+        return int(n.value)
+
+    def erase_hashes_device(self, d_hashes: int, n: int) -> int:
+        r = u64()
+        check(lib.oxg_shard_erase_hashes_device(self._h, d_hashes, n, C.byref(r)))
+        return int(r.value)
+
+    def cut(self, mode: int, thresh: int) -> int:
+        """mincut (mode 0) / maxcut (mode 1) on every shard (collective); keys removed in all."""
+        n = u64()
+        check(lib.oxg_shard_cut(self._h, mode, thresh, C.byref(n)))
+        return int(n.value)
 
     def last_ms(self) -> tuple[float, int]:
         ms, n = C.c_float(), u64()

@@ -1,5 +1,5 @@
-// lookup.cuh -- device side of the sharded table's lookup and merge rounds (oxg_shard_get_hashes*,
-// oxg_shard_merge_table).
+// lookup.cuh -- device side of the sharded table's lookup, merge and erase rounds
+// (oxg_shard_get_hashes*, oxg_shard_merge_table, oxg_shard_erase_hashes*).
 //
 // A lookup round: every rank sorts its queries by owner into the fragment region of its own
 // exchange area (route_*), each owner reads its segment of every rank's queries through the peer
@@ -11,6 +11,10 @@
 // A merge round routes the occupied slots of a range of a plain table instead: keys to the
 // fragment region, their counts to the same positions of the spill region, and each owner adds
 // its segments into its table (apply_pairs_kernel).
+//
+// An erase round routes a list of keys as a lookup does, and each owner erases its segments from
+// its table: in place for a few keys (erase_walk_segments_kernel), or by marking their slots for
+// one rebuild after the last round (erase_mark_segments_kernel).
 #pragma once
 #include "shard.cuh"
 #include "tableops.cuh"
@@ -295,6 +299,59 @@ __global__ void __launch_bounds__(kOpThreads) apply_pairs_kernel(TableView t, Pa
         if (fresh) atomicAdd((unsigned long long *)&t.ctrl->scratch[1], (unsigned long long)fresh);
         if (cr) atomicAdd((unsigned long long *)&t.ctrl->size, (unsigned long long)cr);
     }
+}
+
+// On the owner `me`, for a few keys over all ranks (drop / drop_hash, src/lib.rs:197-224): erase
+// every key of every rank's segment in place, one at a time, as erase_hashes_kernel does -- no
+// rebuild, so a single drop_hash costs a probe run, not a pass over the table.
+// scratch[0] += keys removed, 2^64-1 included.  One thread walks; the block loads the segments.
+__global__ void __launch_bounds__(32) erase_walk_segments_kernel(TableView t, LookupSources src, int me) {
+    __shared__ uint64_t seg_lo[kShardMaxRanks], seg_at[kShardMaxRanks + 1];
+    const uint64_t total = load_segments(src, me, seg_lo, seg_at);
+    if (gtid() != 0) return;
+    uint64_t removed = 0;
+    for (uint64_t i = 0; i < total; ++i) {
+        const int s = segment_of(seg_at, i);
+        erase_one(t, __ldcg(src.frag[s] + seg_lo[s] + (i - seg_at[s])), removed);
+    }
+    t.ctrl->scratch[0] += removed;
+}
+
+// On the owner `me`, for a list: mark the slot of every key of every rank's segment in doomed (one
+// bit per slot of my table), four keys in flight per thread; the table is rebuilt without them
+// after the call's last round (erase_rebuild_kernel), so nothing may move it in between.
+// scratch[0] += bits newly set (a key listed several times, by any ranks, counts once);
+// scratch[1] = 1 when 2^64-1 is listed (its side entry is dropped on the host, with the rebuild).
+__global__ void __launch_bounds__(kOpThreads) erase_mark_segments_kernel(TableView t, LookupSources src, int me,
+                                                                         uint32_t *__restrict__ doomed) {
+    __shared__ uint64_t seg_lo[kShardMaxRanks], seg_at[kShardMaxRanks + 1];
+    constexpr int U = 4;
+    const uint64_t total = load_segments(src, me, seg_lo, seg_at), stride = gstride();
+    uint64_t found = 0;
+    bool side = false;
+    for (uint64_t base = gtid(); base < total; base += stride * U) {
+        uint64_t key[U];
+        uint32_t live = 0;
+#pragma unroll
+        for (int j = 0; j < U; ++j) {
+            const uint64_t i = base + j * stride;
+            key[j] = 0;
+            if (i < total) {
+                const int s = segment_of(seg_at, i);
+                key[j] = __ldcg(src.frag[s] + seg_lo[s] + (i - seg_at[s]));
+                live |= 1u << j;
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < U; ++j) {
+            if (!((live >> j) & 1)) continue;
+            if (key[j] == kEmpty) side = true;
+            else erase_mark_one(t, key[j], doomed, found);
+        }
+    }
+    found = warp_sum(found);
+    if ((threadIdx.x & 31) == 0 && found) atomicAdd((unsigned long long *)&t.ctrl->scratch[0], (unsigned long long)found);
+    if (side) t.ctrl->scratch[1] = 1;
 }
 
 }  // namespace oxg

@@ -142,38 +142,50 @@ __global__ void set_hash_kernel(TableView t, uint64_t key, uint64_t value) {
     }
 }
 
-// drop_hash (src/lib.rs:213-224): remove, then shift the rest of the probe run
-// back so lookups never need tombstones.  One thread walks the list.
+// drop_hash of one key (src/lib.rs:213-224): remove it, then shift the rest of the probe run back
+// so lookups never need tombstones; 2^64-1 clears the side entry.  ++removed when the key was
+// there.  Only one thread of the grid may erase at a time.
+__device__ __forceinline__ void erase_one(const TableView &t, uint64_t key, uint64_t &removed) {
+    if (key == kEmpty) {
+        if (t.ctrl->side_present) { t.ctrl->side_present = 0; t.ctrl->side_count = 0; ++removed; }
+        return;
+    }
+    int64_t f = table_find(t, key);
+    if (f < 0) return;
+    const uint64_t mask = t.cap - 1;
+    uint64_t hole = (uint64_t)f, j = hole;
+    t.slots[hole] = make_ulonglong2(kEmpty, 0);
+    for (;;) {
+        j = (j + 1) & mask;
+        ulonglong2 s = t.slots[j];
+        if (s.x == kEmpty) break;
+        const uint64_t hm = t.home(s.x);
+        // s may move into the hole iff its home is not cyclically inside (hole, j]
+        if (((j - hm) & mask) >= ((j - hole) & mask)) {
+            t.slots[hole] = s;
+            t.slots[j] = make_ulonglong2(kEmpty, 0);
+            hole = j;
+        }
+    }
+    ++removed;
+    t.ctrl->size -= 1;
+}
+
+// drop_hash for a short list: one thread walks it.
 __global__ void erase_hashes_kernel(TableView t, const uint64_t *__restrict__ hashes, uint64_t n) {
     if (gtid() != 0) return;
     uint64_t removed = 0;
-    const uint64_t mask = t.cap - 1;
-    for (uint64_t q = 0; q < n; ++q) {
-        const uint64_t key = hashes[q];
-        if (key == kEmpty) {
-            if (t.ctrl->side_present) { t.ctrl->side_present = 0; t.ctrl->side_count = 0; ++removed; }
-            continue;
-        }
-        int64_t f = table_find(t, key);
-        if (f < 0) continue;
-        uint64_t hole = (uint64_t)f, j = hole;
-        t.slots[hole] = make_ulonglong2(kEmpty, 0);
-        for (;;) {
-            j = (j + 1) & mask;
-            ulonglong2 s = t.slots[j];
-            if (s.x == kEmpty) break;
-            const uint64_t hm = t.home(s.x);
-            // s may move into the hole iff its home is not cyclically inside (hole, j]
-            if (((j - hm) & mask) >= ((j - hole) & mask)) {
-                t.slots[hole] = s;
-                t.slots[j] = make_ulonglong2(kEmpty, 0);
-                hole = j;
-            }
-        }
-        ++removed;
-        t.ctrl->size -= 1;
-    }
+    for (uint64_t q = 0; q < n; ++q) erase_one(t, hashes[q], removed);
     t.ctrl->scratch[0] = removed;
+}
+
+// Marks the slot of `key` (not 2^64-1) in a bitmap of one bit per slot; ++found when this call set
+// the bit, so a key listed twice counts once.
+__device__ __forceinline__ void erase_mark_one(const TableView &t, uint64_t key, uint32_t *__restrict__ doomed, uint64_t &found) {
+    const int64_t f = table_find(t, key);
+    if (f < 0) return;
+    const uint32_t bit = 1u << (f & 31);
+    if (!(atomicOr(&doomed[f >> 5], bit) & bit)) ++found;
 }
 
 // Bulk form of drop_hash: mark the slots of the listed keys in a bitmap (one bit per slot; a key
@@ -185,10 +197,7 @@ __global__ void erase_mark_kernel(TableView t, const uint64_t *__restrict__ hash
     for (uint64_t q = gtid(); q < n; q += gstride()) {
         const uint64_t key = hashes[q];
         if (key == kEmpty) continue;  // the out-of-band key is handled on the host
-        const int64_t f = table_find(t, key);
-        if (f < 0) continue;
-        const uint32_t bit = 1u << (f & 31);
-        if (!(atomicOr(&doomed[f >> 5], bit) & bit)) ++found;
+        erase_mark_one(t, key, doomed, found);
     }
     found = warp_sum(found);
     if ((threadIdx.x & 31) == 0 && found) atomicAdd((unsigned long long *)&t.ctrl->scratch[0], (unsigned long long)found);

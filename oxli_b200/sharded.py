@@ -9,7 +9,9 @@ queries (get / get_hash / get_hash_array, src/lib.rs:170-194) take the same rout
 sends its hashes to their owners, which answer them in place.  So does `add` (KmerCountTable::add,
 src/lib.rs:778-837) of a table counted on one GPU: every (key, count) of each rank's plain table
 goes to its owner and is added there; a second sharded table is added rank by rank, its shards
-already on their owners.  All of that, including the
+already on their owners.  Removal takes the same route: drop / drop_hash / drop_hash_array
+(src/lib.rs:197-224) send each hash to its owner, which erases it, and mincut / maxcut
+(src/lib.rs:227-267) cut every shard and sum what each removed.  All of that, including the
 rank-to-rank flags and the reductions (len / sum / min / max, histo, |A & B|, jaccard, digests:
 reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
 
@@ -110,16 +112,20 @@ class ShardedTable:
     def get_hash(self, h: int) -> int:
         return int(self.get_hash_array([h])[0])
 
-    def get(self, kmer: str) -> int:
-        """Count of a k-mer (src/lib.rs:170-182), hashed through this rank's shard table.  A k-mer
-        of the wrong length or with a non-ACGT base raises before the lookup starts; the other
-        ranks' lookup then fails once the exchange gives up waiting for this one."""
+    def _hash_kmer(self, kmer: str) -> int:
+        """The k-mer's hash, through this rank's shard table.  A k-mer of the wrong length or with
+        a non-ACGT base raises here, before the caller starts an exchange; the other ranks' call
+        then fails once the exchange gives up waiting for this one."""
         if len(kmer) != self.ksize:
             raise ValueError("kmer size does not match count table ksize")
         h = self.engine.table.hash_windows(kmer.encode())
         if h[0] == 0:  # (the reference panics here; the drop-in raises the same error)
             raise RuntimeError(f"invalid DNA character in input k-mer: {kmer}")
-        return self.get_hash(int(h[0]))
+        return int(h[0])
+
+    def get(self, kmer: str) -> int:
+        """Count of a k-mer (src/lib.rs:170-182)."""
+        return self.get_hash(self._hash_kmer(kmer))
 
     # -- merges (collective) -----------------------------------------------------------
     def add(self, other) -> tuple[int, int]:
@@ -137,6 +143,30 @@ class ShardedTable:
         if isinstance(other, ShardedTable):
             return self.engine.merge(other.engine)
         return self.engine.merge_table(other)
+
+    # -- removal (collective) ---------------------------------------------------------
+    def drop_hash_array(self, hashes) -> int:
+        """drop_hash (src/lib.rs:213-224) for each of this rank's hashes on the whole table: every
+        rank calls it with its own list, empty ones included, and each hash is removed by the rank
+        that owns it.  Returns the distinct keys removed from the whole table."""
+        return self.engine.erase_hashes(hashes)
+
+    def drop_hash(self, h: int) -> None:
+        self.drop_hash_array([h])
+
+    def drop(self, kmer: str) -> None:
+        """drop (src/lib.rs:197-224)."""
+        self.drop_hash(self._hash_kmer(kmer))
+
+    def mincut(self, m: int) -> int:
+        """Removes every key with a count below m from every shard (src/lib.rs:227-267); returns
+        the keys removed from the whole table."""
+        return self.engine.cut(0, m)
+
+    def maxcut(self, m: int) -> int:
+        """Removes every key with a count above m from every shard (src/lib.rs:227-267); returns the
+        keys removed from the whole table."""
+        return self.engine.cut(1, m)
 
     # -- reductions (collective) ------------------------------------------------------
     def stats(self) -> dict:
