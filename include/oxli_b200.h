@@ -39,7 +39,8 @@ typedef enum oxg_status {
     OXG_ERR_BAD_KMER = 3,    /* non-ACGT window met in error mode (src/lib.rs:593-596) */
     OXG_ERR_NOMEM = 4,       /* host or device allocation failed */
     OXG_ERR_WRONG_KSIZE = 5, /* k-mer length != table ksize (src/lib.rs:66-67,146-149) */
-    OXG_ERR_TOO_SMALL = 6    /* caller-provided output buffer too small */
+    OXG_ERR_TOO_SMALL = 6,   /* caller-provided output buffer too small */
+    OXG_ERR_IO = 7           /* a file could not be created, opened or written */
 } oxg_status;
 
 typedef struct oxg_table oxg_table;
@@ -289,6 +290,36 @@ oxg_status oxg_shard_erase_hashes_device(oxg_shard *s, const uint64_t *d_hashes,
  * 2^64-1 included, identical on every rank.  Refused before any exchange (OXG_ERR_INVALID): an
  * unconnected shard, a mode other than 0 / 1. */
 oxg_status oxg_shard_cut(oxg_shard *s, int mode, uint64_t thresh, uint64_t *n_removed);
+/* The whole sharded table in one order, each rank holding its own shard's part (hashes /
+ * dump / __iter__, src/lib.rs:330-381), COLLECTIVE: every rank passes the same sort_mode, that
+ * of oxg_export (0: slot order, 1: by key, 2: by (count, key)).  Every key of rank r is below
+ * every key of rank r + 1, so the order of the whole table is each rank's own export placed at
+ * the right positions; no pair crosses between GPUs.  keys / vals receive min(*n_out, cap) of this
+ * rank's pairs in sort_mode order, 2^64-1 (its owner's side entry) and keys held with count 0
+ * included.  runs receives min(*n_runs_out, runs_cap) pieces (global_start, length), 2 u64 each:
+ * taken in order they cover keys / vals and say where they go in the whole table.  Modes 0 and 1:
+ * one run per rank (the ranks' blocks in rank order); mode 2: one run per distinct count of this
+ * rank.  *total_out = pairs in the whole table, the same on every rank.  Output pointers are
+ * nullable; call with cap = runs_cap = 0 to size the arrays.  Plain-table calls on
+ * oxg_shard_table(s) made before the call are seen.  Refused before any exchange
+ * (OXG_ERR_INVALID): an unconnected shard, a bad sort_mode, null arrays with a nonzero cap.  Any
+ * other failure on one rank (a device reservation among them, OXG_ERR_NOMEM) reaches every rank in
+ * the call's exchange: every rank then returns the status of the first rank that failed. */
+oxg_status oxg_shard_export_pairs(oxg_shard *s, int sort_mode, uint64_t *keys, uint64_t *vals, uint64_t cap,
+                                  uint64_t *n_out, uint64_t *runs, uint64_t runs_cap, uint64_t *n_runs_out,
+                                  uint64_t *total_out);
+/* dump(file, sortcounts, sortkeys) of the whole sharded table (src/lib.rs:330-381), COLLECTIVE:
+ * every rank passes the same path and sort_mode, and the ranks write ONE file together, the lines
+ * "<hash>\t<count>\n" (u64 in decimal) in the order of oxg_shard_export_pairs.  Modes 1 and 2 give
+ * the bytes a plain table holding the same pairs dumps; mode 0 the same lines, each rank's in one
+ * block, the blocks in rank order.  Each rank sorts and formats its shard on its GPU; rank 0
+ * creates the file at its final size, then every rank writes its byte ranges into it.  Refused
+ * before any exchange (OXG_ERR_INVALID): an unconnected shard, a bad sort_mode, a null path.  Any
+ * other failure on one rank reaches every rank in the call's exchange, and every rank returns the
+ * first failing rank's status: ranks that passed different paths (OXG_ERR_INVALID), a device
+ * reservation (OXG_ERR_NOMEM), a file that cannot be created, opened or written (OXG_ERR_IO; the
+ * file may then be left incomplete). */
+oxg_status oxg_shard_dump(oxg_shard *s, const char *path, int sort_mode);
 /* time of the last consume call on this shard's stream (device variant: CUDA events;
  * host variant: wall clock of the call) and its number of exchange rounds */
 oxg_status oxg_shard_last_ms(const oxg_shard *s, float *ms, uint64_t *rounds);

@@ -16,7 +16,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OXLI_B200_LIB") or os.path.join(_HERE, "liboxli_b200.so")
 
-OK, ERR_CUDA, ERR_INVALID, ERR_BAD_KMER, ERR_NOMEM, ERR_WRONG_KSIZE, ERR_TOO_SMALL = range(7)
+OK, ERR_CUDA, ERR_INVALID, ERR_BAD_KMER, ERR_NOMEM, ERR_WRONG_KSIZE, ERR_TOO_SMALL, ERR_IO = range(8)
 
 u64 = C.c_uint64
 u64p = C.POINTER(C.c_uint64)
@@ -31,6 +31,10 @@ class OxliError(RuntimeError):
 
 class OxliCudaError(OxliError):
     pass
+
+
+class OxliIOError(OxliError, OSError):
+    """a file could not be created, opened or written (OXG_ERR_IO)"""
 
 
 class oxg_stats(C.Structure):
@@ -85,6 +89,8 @@ SIGNATURES = {
     "oxg_shard_erase_hashes": (C.c_int, [vp, vp, u64, u64p]),
     "oxg_shard_erase_hashes_device": (C.c_int, [vp, vp, u64, u64p]),
     "oxg_shard_cut": (C.c_int, [vp, C.c_int, u64, u64p]),
+    "oxg_shard_export_pairs": (C.c_int, [vp, C.c_int, vp, vp, u64, u64p, vp, u64, u64p, u64p]),
+    "oxg_shard_dump": (C.c_int, [vp, C.c_char_p, C.c_int]),
     "oxg_shard_last_ms": (C.c_int, [vp, C.POINTER(C.c_float), u64p]),
     "oxg_shard_stats": (C.c_int, [vp, C.POINTER(oxg_stats)]),
     "oxg_shard_histo": (C.c_int, [vp, vp, vp, u64, u64p]),
@@ -132,6 +138,8 @@ def check(status: int) -> None:
     msg = (lib.oxg_last_error() or b"").decode(errors="replace")
     if status == ERR_CUDA:
         raise OxliCudaError(status, msg)
+    if status == ERR_IO:
+        raise OxliIOError(status, msg)
     raise OxliError(status, msg)
 
 
@@ -468,6 +476,24 @@ class Shard:
         n = u64()
         check(lib.oxg_shard_cut(self._h, mode, thresh, C.byref(n)))
         return int(n.value)
+
+    def export_pairs(self, sort_mode: int = 0) -> tuple[np.ndarray, np.ndarray, np.ndarray, int]:
+        """This rank's pairs in sort_mode order (0 slot, 1 key, 2 (count, key)), as oxg_export, with
+        where they go in the whole table (collective): returns (keys, vals, runs, total), runs an
+        (n_runs, 2) array of (global_start, length) covering keys / vals in order."""
+        n, nr, tot = u64(), u64(), u64()
+        check(lib.oxg_shard_export_pairs(self._h, sort_mode, None, None, 0, C.byref(n), None, 0, C.byref(nr), C.byref(tot)))
+        k = np.zeros(max(n.value, 1), dtype=np.uint64)
+        v = np.zeros(max(n.value, 1), dtype=np.uint64)
+        runs = np.zeros((max(nr.value, 1), 2), dtype=np.uint64)
+        # (collective: the sizing call above was one exchange, this is the second)
+        check(lib.oxg_shard_export_pairs(self._h, sort_mode, _ptr(k), _ptr(v), len(k), C.byref(n), _ptr(runs), len(runs),
+                                         C.byref(nr), C.byref(tot)))
+        return k[: n.value], v[: n.value], runs[: nr.value], int(tot.value)
+
+    def dump(self, path: str, sort_mode: int = 0) -> None:
+        """The whole table into one file at `path`, the same path on every rank (collective)."""
+        check(lib.oxg_shard_dump(self._h, os.fsencode(path), sort_mode))
 
     def last_ms(self) -> tuple[float, int]:
         ms, n = C.c_float(), u64()

@@ -4,6 +4,7 @@
 // count table.  Everything is plain CUDA runtime: no torch, no Thrust/CUB.
 #include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <chrono>
 #include <cmath>
 #include <cstdarg>
@@ -12,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -19,12 +21,16 @@
 #include <thread>
 #include <vector>
 
+#include <fcntl.h>
+#include <unistd.h>
+
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 
 #include "../../include/oxli_b200.h"
 #include "aggregate.cuh"
 #include "consume.cuh"
+#include "dump.cuh"
 #include "scatter.cuh"
 #include "klist.h"
 #include "lookup.cuh"
@@ -1636,55 +1642,54 @@ oxg_status oxg_table_digest(oxg_table *t, int n_ranks, int rank, uint64_t out[5]
 
 constexpr uint64_t kBounceBytes = 32ull << 20;
 
-// ordered compaction of the live slots into the context's export arrays [0] (slot order: stable
-// between calls while the table is not modified, so dump() == list(iter), src/lib.rs:330-381,658)
-static oxg_status export_device(oxg_table *t, uint64_t *n_live) {
-    DeviceCtx *c = t->ctx;
-    const uint64_t n_chunks = (t->cap + kExportChunk - 1) / kExportChunk;
-    TRY(ensure_dev(&c->d_exp_counts, &c->exp_counts_cap, n_chunks + 1));
-    export_count_kernel<<<(unsigned)n_chunks, kOpThreads, 0, c->stream>>>(t->slots, t->cap, c->d_exp_counts);
+// Where a table's pairs go on the device: [0] the compaction (size + 1 pairs: the side entry joins
+// them), [1] the radix sort's second pair of arrays (size + 1), chunk counts of the compaction
+// (export_chunks + 1), the sort's histogram (256 per sort tile).  The plain table passes its device
+// context's arrays, a shard its own (shards on one device share the context).
+struct ExportArrays {
+    uint64_t *k[2] = {}, *v[2] = {};
+    uint64_t *chunk_counts = nullptr;
+    uint64_t *sort_hist = nullptr;
+};
+
+static uint64_t export_chunks(const oxg_table *t) { return (t->cap + kExportChunk - 1) / kExportChunk; }
+static uint64_t sort_tiles(uint64_t n) { return (n + kSortTile - 1) / kSortTile; }
+
+// ordered compaction of the live slots into a.k[0] / a.v[0] (room for out_cap pairs) on stream st
+// (slot order: stable between calls while the table is not modified, so dump() == list(iter),
+// src/lib.rs:330-381,658)
+static oxg_status export_device(const oxg_table *t, cudaStream_t st, const ExportArrays &a, uint64_t out_cap, uint64_t *n_live) {
+    const uint64_t n_chunks = export_chunks(t);
+    export_count_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots, t->cap, a.chunk_counts);
     LAUNCHED();
-    export_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_exp_counts, n_chunks, c->d_exp_counts + n_chunks);
+    export_scan_kernel<<<1, 1024, 0, st>>>(a.chunk_counts, n_chunks, a.chunk_counts + n_chunks);
     LAUNCHED();
     CU(cudaGetLastError());
     uint64_t live = 0;
-    CU(cudaMemcpyAsync(&live, c->d_exp_counts + n_chunks, 8, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    if (c->exp_cap[0] < live + 1) {
-        if (c->d_exp_k[0]) { CU(cudaFree(c->d_exp_k[0])); CU(cudaFree(c->d_exp_v[0])); }
-        c->d_exp_k[0] = c->d_exp_v[0] = nullptr; c->exp_cap[0] = 0;
-        CU(cudaMalloc(&c->d_exp_k[0], (live + 1) * 8));
-        CU(cudaMalloc(&c->d_exp_v[0], (live + 1) * 8));
-        c->exp_cap[0] = live + 1;
-    }
-    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, c->stream>>>(t->slots, t->cap, c->d_exp_counts, c->d_exp_k[0], c->d_exp_v[0], live);
+    CU(cudaMemcpyAsync(&live, a.chunk_counts + n_chunks, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (live >= out_cap) return fail(OXG_ERR_INVALID, "internal: %llu live slots, room for %llu", (unsigned long long)live, (unsigned long long)out_cap);
+    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots, t->cap, a.chunk_counts, a.k[0], a.v[0], live);
     LAUNCHED();
     CU(cudaGetLastError());
     *n_live = live;
     return OXG_OK;
 }
 
-// stable LSD radix sort of the n pairs in export arrays [0]; *which = the pair of arrays holding the result
-static oxg_status sort_pairs_device(DeviceCtx *c, uint64_t n, int sort_mode, uint64_t max_count, int *which) {
+// stable LSD radix sort of the n pairs in a.k[0] / a.v[0] on stream st; *which = the pair of arrays
+// holding the result
+static oxg_status sort_pairs_device(cudaStream_t st, const ExportArrays &a, uint64_t n, int sort_mode, uint64_t max_count, int *which) {
     *which = 0;
     if (n < 2) return OXG_OK;
-    if (c->exp_cap[1] < n) {
-        if (c->d_exp_k[1]) { CU(cudaFree(c->d_exp_k[1])); CU(cudaFree(c->d_exp_v[1])); }
-        c->d_exp_k[1] = c->d_exp_v[1] = nullptr; c->exp_cap[1] = 0;
-        CU(cudaMalloc(&c->d_exp_k[1], n * 8));
-        CU(cudaMalloc(&c->d_exp_v[1], n * 8));
-        c->exp_cap[1] = n;
-    }
-    const uint64_t n_tiles = (n + kSortTile - 1) / kSortTile;
-    TRY(ensure_dev(&c->d_sort_hist, &c->sort_hist_cap, 256 * n_tiles));
+    const uint64_t n_tiles = sort_tiles(n);
     int cur = 0;
     auto pass = [&](int shift, int by_count) -> oxg_status {
-        radix_hist_kernel<<<(unsigned)n_tiles, kSortThreads, 0, c->stream>>>(c->d_exp_k[cur], c->d_exp_v[cur], n, shift, by_count, n_tiles, c->d_sort_hist);
+        radix_hist_kernel<<<(unsigned)n_tiles, kSortThreads, 0, st>>>(a.k[cur], a.v[cur], n, shift, by_count, n_tiles, a.sort_hist);
         LAUNCHED();
-        radix_scan_kernel<<<1, 1024, 0, c->stream>>>(c->d_sort_hist, 256 * n_tiles);
+        radix_scan_kernel<<<1, 1024, 0, st>>>(a.sort_hist, 256 * n_tiles);
         LAUNCHED();
-        radix_scatter_kernel<<<(unsigned)n_tiles, kSortThreads, 0, c->stream>>>(c->d_exp_k[cur], c->d_exp_v[cur], c->d_exp_k[cur ^ 1], c->d_exp_v[cur ^ 1],
-                                                                                n, shift, by_count, n_tiles, c->d_sort_hist);
+        radix_scatter_kernel<<<(unsigned)n_tiles, kSortThreads, 0, st>>>(a.k[cur], a.v[cur], a.k[cur ^ 1], a.v[cur ^ 1],
+                                                                         n, shift, by_count, n_tiles, a.sort_hist);
         LAUNCHED();
         CU(cudaGetLastError());
         cur ^= 1;
@@ -1697,30 +1702,61 @@ static oxg_status sort_pairs_device(DeviceCtx *c, uint64_t n, int sort_mode, uin
     return OXG_OK;
 }
 
-// device array -> caller's host array through two pinned bounce buffers (the caller's memory is
-// usually pageable: a plain cudaMemcpy would stage it the same way, but one chunk at a time)
-static oxg_status download(DeviceCtx *c, uint64_t *dst, const uint64_t *d_src, uint64_t n) {
-    if (!dst || n == 0) return OXG_OK;
-    for (int b = 0; b < 2; ++b)
-        if (!c->h_bounce[b]) {
-            CU(cudaMallocHost(&c->h_bounce[b], kBounceBytes));
-            CU(cudaEventCreateWithFlags(&c->ev_bounce[b], cudaEventDisableTiming));
+// A table's n pairs (side entry included: side_count when `side`) in sort_mode order in a.k[*which] /
+// a.v[*which], on stream st.  Returns with st drained.
+static oxg_status export_pairs_device(const oxg_table *t, cudaStream_t st, const ExportArrays &a, uint64_t out_cap, bool side,
+                                      uint64_t side_count, int sort_mode, uint64_t max_count, uint64_t *n_out, int *which) {
+    uint64_t n = 0;
+    TRY(export_device(t, st, a, out_cap, &n));
+    if (side) {  // the out-of-band key 2^64-1 lives outside the slot array: it joins the pairs here
+        const uint64_t kv[2] = {kEmpty, side_count};
+        CU(cudaMemcpyAsync(a.k[0] + n, &kv[0], 8, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(a.v[0] + n, &kv[1], 8, cudaMemcpyHostToDevice, st));
+        ++n;
+    }
+    *which = 0;
+    if (sort_mode != 0) TRY(sort_pairs_device(st, a, n, sort_mode, max_count, which));
+    CU(cudaStreamSynchronize(st));
+    *n_out = n;
+    return OXG_OK;
+}
+
+// two pinned buffers of `bytes` each and an event per buffer, through which device memory reaches the host
+struct Bounce {
+    uint8_t *buf[2];
+    cudaEvent_t ev[2];
+    uint64_t bytes;
+};
+
+// `bytes` of device memory at d_src, piece by piece through the bounce buffers on stream st:
+// sink(at, p, len) receives bytes [at, at + len) while the next piece is on its way
+static oxg_status stream_to_host(cudaStream_t st, const Bounce &b, const uint8_t *d_src, uint64_t bytes,
+                                 const std::function<oxg_status(uint64_t, const uint8_t *, uint64_t)> &sink) {
+    const uint64_t per = b.bytes;
+    const uint64_t n_pieces = (bytes + per - 1) / per;
+    for (uint64_t i = 0; i <= n_pieces; ++i) {
+        if (i < n_pieces) {
+            const uint64_t lo = i * per, cnt = std::min(per, bytes - lo);
+            CU(cudaMemcpyAsync(b.buf[i & 1], d_src + lo, cnt, cudaMemcpyDeviceToHost, st));
+            CU(cudaEventRecord(b.ev[i & 1], st));
         }
-    const uint64_t per = kBounceBytes / 8;
-    const uint64_t n_chunks = (n + per - 1) / per;
-    for (uint64_t i = 0; i <= n_chunks; ++i) {
-        if (i < n_chunks) {
-            const uint64_t lo = i * per, cnt = std::min(per, n - lo);
-            CU(cudaMemcpyAsync(c->h_bounce[i & 1], d_src + lo, cnt * 8, cudaMemcpyDeviceToHost, c->stream));
-            CU(cudaEventRecord(c->ev_bounce[i & 1], c->stream));
-        }
-        if (i > 0) {  // chunk i-1 has landed while chunk i is on its way
-            const uint64_t lo = (i - 1) * per, cnt = std::min(per, n - lo);
-            CU(cudaEventSynchronize(c->ev_bounce[(i - 1) & 1]));
-            memcpy(dst + lo, c->h_bounce[(i - 1) & 1], cnt * 8);
+        if (i > 0) {  // piece i-1 has landed while piece i is on its way
+            const uint64_t lo = (i - 1) * per, cnt = std::min(per, bytes - lo);
+            CU(cudaEventSynchronize(b.ev[(i - 1) & 1]));
+            TRY(sink(lo, b.buf[(i - 1) & 1], cnt));
         }
     }
     return OXG_OK;
+}
+
+// device array -> caller's host array through the bounce buffers (the caller's memory is usually
+// pageable: a plain cudaMemcpy would stage it the same way, but one chunk at a time)
+static oxg_status download(cudaStream_t st, const Bounce &b, uint64_t *dst, const uint64_t *d_src, uint64_t n) {
+    if (!dst || n == 0) return OXG_OK;
+    return stream_to_host(st, b, reinterpret_cast<const uint8_t *>(d_src), n * 8, [&](uint64_t at, const uint8_t *p, uint64_t len) {
+        memcpy(reinterpret_cast<uint8_t *>(dst) + at, p, len);
+        return OXG_OK;
+    });
 }
 
 oxg_status oxg_export(oxg_table *t, uint64_t *keys, uint64_t *vals, uint64_t cap, int sort_mode, uint64_t *n_out) {
@@ -1730,7 +1766,7 @@ oxg_status oxg_export(oxg_table *t, uint64_t *keys, uint64_t *vals, uint64_t cap
     TRY(pull_ctrl(t));
     const bool side = t->h_ctrl->side_present != 0;
     const uint64_t side_count = t->h_ctrl->side_count;
-    const uint64_t total = t->h_ctrl->size + (side ? 1 : 0);
+    const uint64_t live = t->h_ctrl->size, total = live + (side ? 1 : 0);
     *n_out = total;
     if (cap == 0 || total == 0) return OXG_OK;
     uint64_t max_count = 0;
@@ -1739,20 +1775,29 @@ oxg_status oxg_export(oxg_table *t, uint64_t *keys, uint64_t *vals, uint64_t cap
         TRY(run_stats(t, false, &st, nullptr));
         max_count = st.max;
     }
-    uint64_t live = 0;
-    TRY(export_device(t, &live));
-    uint64_t n = live;
-    if (side) {  // the out-of-band key 2^64-1 lives outside the slot array: it joins the pairs here
-        const uint64_t kv[2] = {kEmpty, side_count};
-        CU(cudaMemcpyAsync(c->d_exp_k[0] + n, &kv[0], 8, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(c->d_exp_v[0] + n, &kv[1], 8, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-        ++n;
+    // the context's export arrays, grown as needed
+    TRY(ensure_dev(&c->d_exp_counts, &c->exp_counts_cap, export_chunks(t) + 1));
+    for (int i = 0; i < (sort_mode != 0 && total >= 2 ? 2 : 1); ++i) {
+        if (c->exp_cap[i] >= live + 1) continue;
+        if (c->d_exp_k[i]) { CU(cudaFree(c->d_exp_k[i])); CU(cudaFree(c->d_exp_v[i])); }
+        c->d_exp_k[i] = c->d_exp_v[i] = nullptr; c->exp_cap[i] = 0;
+        CU(cudaMalloc(&c->d_exp_k[i], (live + 1) * 8));
+        CU(cudaMalloc(&c->d_exp_v[i], (live + 1) * 8));
+        c->exp_cap[i] = live + 1;
     }
+    if (sort_mode != 0 && total >= 2) TRY(ensure_dev(&c->d_sort_hist, &c->sort_hist_cap, 256 * sort_tiles(total)));
+    for (int b = 0; b < 2; ++b)
+        if (!c->h_bounce[b]) {
+            CU(cudaMallocHost(&c->h_bounce[b], kBounceBytes));
+            CU(cudaEventCreateWithFlags(&c->ev_bounce[b], cudaEventDisableTiming));
+        }
+    const ExportArrays a{{c->d_exp_k[0], c->d_exp_k[1]}, {c->d_exp_v[0], c->d_exp_v[1]}, c->d_exp_counts, c->d_sort_hist};
+    uint64_t n = 0;
     int which = 0;
-    if (sort_mode != 0) TRY(sort_pairs_device(c, n, sort_mode, max_count, &which));
-    TRY(download(c, keys, c->d_exp_k[which], std::min(n, cap)));
-    TRY(download(c, vals, c->d_exp_v[which], std::min(n, cap)));
+    TRY(export_pairs_device(t, c->stream, a, c->exp_cap[0], side, side_count, sort_mode, max_count, &n, &which));
+    const Bounce b{{c->h_bounce[0], c->h_bounce[1]}, {c->ev_bounce[0], c->ev_bounce[1]}, kBounceBytes};
+    TRY(download(c->stream, b, keys, a.k[which], std::min(n, cap)));
+    TRY(download(c->stream, b, vals, a.v[which], std::min(n, cap)));
     CU(cudaStreamSynchronize(c->stream));
     return OXG_OK;
 }

@@ -11,7 +11,9 @@ src/lib.rs:778-837) of a table counted on one GPU: every (key, count) of each ra
 goes to its owner and is added there; a second sharded table is added rank by rank, its shards
 already on their owners.  Removal takes the same route: drop / drop_hash / drop_hash_array
 (src/lib.rs:197-224) send each hash to its owner, which erases it, and mincut / maxcut
-(src/lib.rs:227-267) cut every shard and sum what each removed.  All of that, including the
+(src/lib.rs:227-267) cut every shard and sum what each removed.  export and dump (src/lib.rs:330-381)
+need no routing at all: every key of rank r is below every key of rank r + 1, so each rank sorts
+and formats its own shard and writes its part of one file.  All of that, including the
 rank-to-rank flags and the reductions (len / sum / min / max, histo, |A & B|, jaccard, digests:
 reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
 
@@ -192,6 +194,30 @@ class ShardedTable:
     def digest(self) -> dict:
         """{n, sum, xor, sum_hc, foreign} of the whole table; foreign must be 0."""
         return self.engine.digest()
+
+    # -- export and dump (collective) ---------------------------------------------------
+    @staticmethod
+    def _sort_mode(sortcounts: bool, sortkeys: bool) -> int:
+        if sortcounts and sortkeys:
+            raise ValueError("Cannot sort by both counts and keys at the same time.")
+        return 1 if sortkeys else 2 if sortcounts else 0
+
+    def export(self, sortcounts: bool = False, sortkeys: bool = False):
+        """This rank's part of the whole table in dump order (src/lib.rs:330-381): by key with
+        sortkeys, by (count, key) with sortcounts, else each rank's shard in table order.  Returns
+        (keys, vals, runs, total): this rank's pairs, an (n_runs, 2) array of (global_start, length)
+        pieces that place keys / vals in the whole table in order, and the whole table's length.
+        Every key of rank r is below every key of rank r + 1, so each rank sorts its own shard on
+        its GPU and no pair crosses between GPUs."""
+        return self.engine.export_pairs(self._sort_mode(sortcounts, sortkeys))
+
+    def dump(self, file: str, sortcounts: bool = False, sortkeys: bool = False) -> None:
+        """dump(file, sortcounts, sortkeys) of the whole table (src/lib.rs:330-381): every rank
+        passes the same path, and the ranks write one file of "<hash>\\t<count>\\n" lines together.
+        With sortkeys or sortcounts it holds the bytes the drop-in KmerCountTable.dump writes for a
+        table of the same pairs; without, the same lines, each rank's shard in one block, the blocks
+        in rank order.  A file that cannot be written raises OSError on every rank."""
+        self.engine.dump(file, self._sort_mode(sortcounts, sortkeys))
 
     # -- this rank's shard only ---------------------------------------------------------
     def local_items_sorted(self):
