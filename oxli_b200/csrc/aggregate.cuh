@@ -217,7 +217,7 @@ __global__ void __launch_bounds__(kAggThreads, 1) aggregate_kernel(const AggPara
         uint32_t live = 0;
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-            bool ok = h[u] != 0;  // (0 pads the last line a launch of pass A wrote, and the block's tail)
+            bool ok = h[u] != 0;  // (0 fills the tail of a block past the fragment's fill count)
             if (filter_owner && p.n_ranks > 1 && ok) ok = (int)(h[u] >> p.owner_shift) == p.self_rank;
             live |= (ok ? 1u : 0u) << u;
         }

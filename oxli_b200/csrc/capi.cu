@@ -388,8 +388,8 @@ struct PartPlan {
     uint32_t n_parts = 0, part_bits = 0;   // partitions of one rank's table
     int n_ranks = 1, self_rank = 0, owner_shift = 64;
     uint32_t grid_a = 0;                   // CTAs of pass A = fragments per destination
-    uint32_t frag_cap = 0;                 // entries per fragment (multiple of the line)
-    uint32_t line_shift = 4;               // entries staged per destination before a line is written: 2^line_shift
+    uint32_t frag_cap = 0;                 // entries per fragment (multiple of four: 32-byte sectors)
+    uint32_t batch_tiles = 1;              // warp tiles per warp that pass A sorts by destination at a time
     uint64_t spill_cap = 0;
     uint32_t groups = 1;
     uint32_t n_dest() const { return n_parts * (uint32_t)n_ranks; }
@@ -668,8 +668,8 @@ bool use_partitioned(const oxg_table *t, uint64_t span) {
 
 // Partition count: 3072-6144 distinct keys per partition, so that the shared-memory table of
 // pass B (16384 slots in buckets of four) holds a partition's keys at load 0.2-0.4 and duplicates
-// meet there; at most max_parts, because pass A stages one line per destination in shared memory
-// (and keeps longer lines with fewer destinations).
+// meet there; at most max_parts (2048 over all ranks), because pass A keeps three words per
+// destination in shared memory next to its batch of hashes.
 uint32_t choose_parts(const oxg_table *t, uint32_t max_parts) {
     const uint32_t forced = g_parts_override.load();
     if (forced >= 2 && !(forced & (forced - 1))) return std::min(forced, std::max(max_parts, 2u));
@@ -680,37 +680,45 @@ uint32_t choose_parts(const oxg_table *t, uint32_t max_parts) {
     return (uint32_t)std::min<uint64_t>(parts, max_parts);
 }
 
-// dynamic shared memory of scatter_kernel<k> (mirrors scatter_smem_bytes<K>)
-size_t scatter_smem_rt(uint32_t k, uint32_t n_dest, uint32_t line_shift) {
+// dynamic shared memory of scatter_kernel<k> (its per-warp tile buffers as ScatWarpBuf<K>)
+size_t scatter_smem_rt(uint32_t k, uint32_t n_dest, uint32_t batch_tiles) {
     const uint32_t q = 8 * ((k + 7 + 7) / 8);
     const uint32_t bl = ((kWarpTile - 8 + q) + 15) / 16 * 16;
-    return (((size_t)n_dest * ((8u << line_shift) + 12) + 16 + 15) & ~(size_t)15) + (size_t)kScatWarps * (2 * bl + 128);
+    return scatter_smem_bytes(n_dest, batch_tiles, (int)(2 * bl + 128));
+}
+
+// CTAs of pass A for a launch of n_tiles warp tiles: kScatCtasPerSm per SM, fewer when the launch
+// has less than one tile per warp of the full grid (scatter_full_grid_tiles).  A launch of fewer
+// tiles than one batch of the grid simply leaves the batch part empty.
+uint64_t scatter_full_grid_tiles(const DeviceCtx *c) { return (uint64_t)c->sms * kScatCtasPerSm * kScatWarps; }
+uint32_t scatter_grid(const DeviceCtx *c, uint64_t n_tiles) {
+    return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_tiles + kScatWarps - 1) / kScatWarps, (uint64_t)c->sms * kScatCtasPerSm));
 }
 
 oxg_status plan_partitioned(oxg_table *t, uint64_t span, uint64_t n_tiles, int n_ranks, int self_rank, PartPlan *out) {
     DeviceCtx *c = t->ctx;
     PartPlan pl;
-    // destinations are (rank, partition): 1024 of them keep full 128-byte lines staged in pass A
+    // destinations are (rank, partition), at most 2048: pass A keeps its largest batch at every k up to there
     pl.n_parts = choose_parts(t, std::max(2u, 2048u / (uint32_t)n_ranks));
     while ((1u << pl.part_bits) < pl.n_parts) ++pl.part_bits;
     pl.n_ranks = n_ranks; pl.self_rank = self_rank;
     int lg = 0;
     while ((1 << lg) < n_ranks) ++lg;
     pl.owner_shift = 64 - lg;
-    // the staged line: as long as the shared memory of kScatCtasPerSm CTAs per SM allows
-    pl.line_shift = 4;
-    while (pl.line_shift > 1 && scatter_smem_rt(t->k, pl.n_dest(), pl.line_shift) * kScatCtasPerSm > 220u * 1024) --pl.line_shift;
-    if (scatter_smem_rt(t->k, pl.n_dest(), pl.line_shift) * kScatCtasPerSm > 220u * 1024) return fail(OXG_ERR_INVALID, "internal: too many scatter destinations");
-    // kScatCtasPerSm CTAs per SM (their staging fills the SM's shared memory); fewer when the launch is small
-    const uint64_t tiles_per_cta = kScatWarps;
-    pl.grid_a = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((n_tiles + tiles_per_cta - 1) / tiles_per_cta, (uint64_t)c->sms * kScatCtasPerSm));
+    // the batch of pass A: as large as the shared memory of kScatCtasPerSm CTAs per SM allows
+    pl.batch_tiles = kScatMaxBatchTiles;
+    while (pl.batch_tiles > 1 && scatter_smem_rt(t->k, pl.n_dest(), pl.batch_tiles) * kScatCtasPerSm > 220u * 1024) --pl.batch_tiles;
+    if (scatter_smem_rt(t->k, pl.n_dest(), pl.batch_tiles) * kScatCtasPerSm > 220u * 1024) return fail(OXG_ERR_INVALID, "internal: too many scatter destinations");
+    pl.grid_a = scatter_grid(c, n_tiles);
+    // pass B reads the fill counts of a partition's fragments into shared memory, at most kAggMaxFrags
+    if (pl.grid_a * (uint64_t)kMaxSources > kAggMaxFrags) return fail(OXG_ERR_INVALID, "internal: more pass A CTAs than pass B can take");
     // a fragment holds its fair share of the launch's windows plus half again plus four standard
     // deviations; what does not fit (skew) goes to the spill list, which can take the whole launch
-    const uint64_t line = 1ull << pl.line_shift;
+    // (rounded up to whole 32-byte sectors, so that every fragment starts on one)
     const uint64_t fair = span / ((uint64_t)pl.n_dest() * pl.grid_a) + 1;
     uint64_t sq = 1;
     while (sq * sq < fair) ++sq;
-    pl.frag_cap = (uint32_t)((fair + fair / 2 + 4 * sq + line + line - 1) & ~(line - 1));
+    pl.frag_cap = (uint32_t)((fair + fair / 2 + 4 * sq + 3) & ~(uint64_t)3);
     pl.spill_cap = span;
     // work items of pass B = partitions x groups: enough of them (four per SM) that the CTAs finish
     // together -- 256 partitions of a shard on 148 SMs would otherwise be two uneven waves
@@ -738,12 +746,13 @@ oxg_status launch_part_a(oxg_table *t, ConsumeParams p, const PartPlan &pl, uint
     DeviceCtx *c = t->ctx;
     const void *fn = specialised_entry(t->k, kModePart);
     TRY(scatter_attr(c, t->k));
-    const size_t dyn = scatter_smem_rt(t->k, pl.n_dest(), pl.line_shift);
+    const size_t dyn = scatter_smem_rt(t->k, pl.n_dest(), pl.batch_tiles);
     p.frag = d_frag; p.frag_cnt = d_frag_cnt; p.frag_cap = pl.frag_cap;
-    p.n_parts = pl.n_parts; p.part_shift = 64 - pl.part_bits; p.n_dest = pl.n_dest(); p.line_shift = pl.line_shift;
+    p.n_parts = pl.n_parts; p.part_shift = 64 - pl.part_bits; p.n_dest = pl.n_dest(); p.batch_tiles = pl.batch_tiles;
     p.n_ranks = pl.n_ranks; p.self_rank = pl.self_rank; p.owner_shift = pl.owner_shift;
     p.spill = d_spill; p.spill_cap = pl.spill_cap; p.spill_n = d_spill_n;
     p.frag_append = append ? 1u : 0u;
+    if (p.n_tiles >> 31) return fail(OXG_ERR_INVALID, "internal: too many tiles for one pass A launch");
     if (!append) CU(cudaMemsetAsync(d_spill_n, 0, 8, stream));
     void *args[] = {&p};
     CU(cudaLaunchKernel(fn, dim3(pl.grid_a), dim3(kScatThreads), args, dyn, stream));

@@ -82,7 +82,7 @@ struct ConsumeParams {
     uint32_t n_parts;        // partitions per rank (power of two, >= 2)
     uint32_t part_shift;     // 64 - log2(n_parts)
     uint32_t n_dest;         // n_ranks * n_parts
-    uint32_t line_shift;     // log2 of the entries staged per destination before a line is written (scatter.cuh)
+    uint32_t batch_tiles;    // warp tiles per warp that scatter_kernel sorts by destination at a time (scatter.cuh)
     uint32_t frag_append;    // != 0: continue the fragments where frag_cnt says an earlier launch left them
     uint64_t *spill;
     uint64_t spill_cap;

@@ -9,27 +9,27 @@
 // costs a B200 SM about seven cycles whatever its width (8, 16 or 32 bytes: 40 G stores/s
 // chip-wide, profiles/r2_microbench_smem_scatter.txt), so "one 8-byte store per hash straight
 // into the destination's fragment" runs at a third of the hashing rate.  Shared-memory atomics
-// and stores, in contrast, cost 0.13-0.45 cycles.  So every destination has a line of
-// 2^line_shift entries (128 bytes at 16) staged in shared memory; hashes are ranked into it
-// with one shared-memory atomic each and a line leaves the SM as ONE full-width coalesced
-// store when it is complete.
+// and stores, in contrast, cost 0.13-0.45 cycles.  So a CTA sorts a large batch of hashes by
+// destination in shared memory first; a destination's run of the sorted batch then leaves the
+// SM as consecutive lanes storing consecutive entries of its fragment.
 //
-// A CTA of 12 warps (two per SM) works in rounds: every warp hashes one tile of 256 window starts
-// (8 per lane), then the CTA
-//   1. ranks:   q = atomicAdd(arrivals[dest], 1) is the hash's position in the fragment | barrier
-//   2. places:  the line that was being filled is completed in shared memory (whoever takes its
-//               last slot lists the destination), entries of further complete lines (rare) go
-//               straight out, what lies beyond the last complete line waits       | barrier
-//   3. flushes: listed lines, 32 bytes per lane                                   | barrier
-//   4. moves the waiting entries in at the front of their line; whoever took a destination's
-//      last position of the round brings its book up to date       (no barrier: step 1 of the
-//      next round touches other words, and its barrier precedes every reader)
-// There is no per-destination loop anywhere: all bookkeeping is done by the threads that hold
-// the hashes.
-// At the end of a launch the last line of every destination goes out padded with zeros (0 is
-// never a hash here, src/lib.rs:589), so fill counts stay multiples of the line and a later
-// launch can continue the same fragments (frag_append): pass B then runs once per several
-// launches and sees more duplicates per key.
+// A CTA is persistent and works in batches of `batch_tiles` warp tiles (256 window starts, 8 per
+// lane) per warp:
+//   1. hash:      every warp hashes its tiles with no CTA barrier into its own slice of the batch
+//                 buffer and counts the hashes per destination (one shared-memory atomic each)
+//                                                                                   | barrier
+//   2. scan:      one warp per 256 destinations turns the counts into the run start of every
+//                 destination in the sorted batch and the offset from there to its fragment's fill
+//                 position; every warp loads its slice into registers              | barrier
+//   3. permute:   every hash goes to its destination's run, start + atomicAdd(cursor)  | barrier
+//   4. write out: warps stride over the sorted batch; the entry at rank r of its run goes to
+//                 position fill + r of its fragment, or to the spill list when that is past
+//                 frag_cap                                                          | barrier
+// The destination is recomputed from the hash wherever it is needed (one multiply and a shift),
+// never stored; order within a run is whatever the atomics made it (pass B adds commutatively).
+// At the end of a launch frag_cnt holds the fill counts exactly, and a later launch can continue
+// the same fragments (frag_append): pass B then runs once per several launches and sees more
+// duplicates per key.
 // A fragment is [dest][cta][frag_cap] as pass B expects; what does not fit a fragment (skew: one
 // k-mer flooding its partition) goes to the spill list exactly as before.
 #pragma once
@@ -37,8 +37,10 @@
 
 namespace oxg {
 
-// Two CTAs of 12 warps per SM rather than one of 24: the phases between barriers are short and
-// serial in nature, and while one CTA is in them the other one hashes.
+// Two CTAs of 12 warps per SM rather than one of 24.  One CTA of 24 warps sorts twice the batch
+// (18432 hashes) per set of barriers and ran pass A 1 ms faster on C2 (18.7 against 19.7 ms per
+// step, one B200) -- but it halves the pass A grid, i.e. the fragments of a partition, and pass B
+// then took 9.6 instead of 8.1 ms: the C2 step was 28.6 ms against 28.0 (DESIGN.md 4.3).
 #ifndef OXG_SCAT_THREADS
 #define OXG_SCAT_THREADS 384
 #endif
@@ -48,6 +50,11 @@ namespace oxg {
 constexpr int kScatThreads = OXG_SCAT_THREADS;
 constexpr int kScatCtasPerSm = OXG_SCAT_CTAS;
 constexpr int kScatWarps = kScatThreads / 32;
+// Warp tiles per warp and batch, at most: step 3 holds a warp's whole slice in registers, 8 hashes
+// per lane and tile, and 80 registers per thread (two CTAs of 384 or one of 768 per SM) leave room
+// for three tiles' 24 hashes and no more.
+constexpr int kScatMaxBatchTiles = 3;
+static_assert(kScatWarps * 256 >= 2048, "step 2 scans 256 destinations per warp, up to 2048 of them");
 
 // per-warp tile buffers: forward bytes, mirrored complement, bad bits, end bits
 template <int K>
@@ -56,39 +63,46 @@ struct ScatWarpBuf {
     static constexpr int kBytes = 2 * BL + 64 + 64;
 };
 
-template <int K>
-inline size_t scatter_smem_bytes(uint32_t n_dest, uint32_t line_shift) {
-    return (((size_t)n_dest * ((8u << line_shift) + 12) + 16 + 15) & ~(size_t)15) + (size_t)kScatWarps * ScatWarpBuf<K>::kBytes;
+// dynamic shared memory: the batch buffer, three words per destination (count, run position,
+// fragment-minus-batch offset), the batch total and launch tally, the per-warp tile buffers
+__host__ __device__ inline size_t scatter_dest_bytes(uint32_t n_dest) { return ((size_t)n_dest * 12 + 15) & ~(size_t)15; }
+__host__ __device__ inline size_t scatter_smem_bytes(uint32_t n_dest, uint32_t batch_tiles, int warp_buf_bytes) {
+    return (size_t)kScatWarps * batch_tiles * kWarpTile * 8 + scatter_dest_bytes(n_dest) + 16 + (size_t)kScatWarps * warp_buf_bytes;
 }
 
 template <int K>
 __global__ void __launch_bounds__(kScatThreads, kScatCtasPerSm) scatter_kernel(const ConsumeParams p) {
     using G = TileGeom<K>;
     constexpr int BL = G::BL, NV = G::NV, NE = G::NE;
+    constexpr int kMaxPerLane = kScatMaxBatchTiles * kWPT;
     static_assert(NV + 8 <= 32 && NE <= 16, "per-warp mask buffers are 64 bytes each");
     extern __shared__ __align__(128) uint8_t sm[];
-    const uint32_t nd = p.n_dest, ls = p.line_shift, line = 1u << ls;
-    uint64_t *stage = reinterpret_cast<uint64_t *>(sm);                       // [nd][line]
-    uint2 *book = reinterpret_cast<uint2 *>(sm + ((size_t)nd << (ls + 3)));  // [nd]
-    uint32_t *flist = reinterpret_cast<uint32_t *>(book + nd);                // [nd] destinations to flush this round
-    uint32_t *s_nflush = flist + nd;                                          // [4]
-    uint8_t *wbuf = sm + ((((size_t)nd * ((8u << ls) + 12) + 16) + 15) & ~(size_t)15) + (size_t)(threadIdx.x >> 5) * ScatWarpBuf<K>::kBytes;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t nd = p.n_dest, slice = p.batch_tiles * kWarpTile;  // entries of a warp's slice
+    uint64_t *batch = reinterpret_cast<uint64_t *>(sm);               // [kScatWarps][slice], then sorted
+    // Per destination: cnt = entries of the batch; pos = run start in the sorted batch, after step 3
+    // the run's end; to_frag = fragment position minus batch position of the run (mod 2^32).  The
+    // fill count of the fragment is never stored: before a batch's scan it is
+    // min(to_frag + pos, frag_cap) -- the previous batch's fill plus its run, or where the launch began.
+    uint32_t *cnt = reinterpret_cast<uint32_t *>(batch + (size_t)kScatWarps * slice);
+    uint32_t *pos = cnt + nd, *to_frag = pos + nd;
+    uint32_t *s_total = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(cnt) + scatter_dest_bytes(nd));  // entries of the batch
+    unsigned long long *s_counted = reinterpret_cast<unsigned long long *>(s_total + 2);  // ... of the launch so far
+    uint8_t *wbuf = reinterpret_cast<uint8_t *>(s_total + 4) + (size_t)warp * ScatWarpBuf<K>::kBytes;
     uint8_t *s_fw = wbuf, *s_rc = wbuf + BL;
     uint16_t *s_bad = reinterpret_cast<uint16_t *>(wbuf + 2 * BL);
     uint32_t *s_end = reinterpret_cast<uint32_t *>(wbuf + 2 * BL + 64);
+    uint64_t *const my_slice = batch + (size_t)warp * slice;
 
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t frag_row = (uint64_t)gridDim.x * p.frag_cap;              // entries between destinations
+    // (the fragment buffer holds fewer than 2^32 entries: plan_partitioned)
+    const uint32_t frag_row = gridDim.x * p.frag_cap;                        // entries between destinations
     uint64_t *const my_frag = p.frag + (uint64_t)blockIdx.x * p.frag_cap;    // + dest * frag_row
-    // book[d] = {x: entries of the fragment accounted for at the start of the round,
-    //            y: arrivals ever (never reset: an arrival's rank IS its position in the fragment)}
-    // A launch may continue fragments an earlier launch began (frag_append): their fill counts are
-    // multiples of the line, because every launch pads its last lines with zeros (pass B skips them).
+    // A launch may continue fragments an earlier launch began (frag_append) at their fill counts.
     for (uint32_t i = threadIdx.x; i < nd; i += kScatThreads) {
-        const uint32_t at = p.frag_append ? p.frag_cnt[(uint64_t)i * gridDim.x + blockIdx.x] : 0u;
-        book[i] = make_uint2(at, at);
+        to_frag[i] = p.frag_append ? p.frag_cnt[(uint64_t)i * gridDim.x + blockIdx.x] : 0u;
+        cnt[i] = 0; pos[i] = 0;
     }
-    if (threadIdx.x == 0) *s_nflush = 0;
+    if (threadIdx.x == 0) *s_counted = 0;
     __syncthreads();
 
     auto dest_of = [&](uint64_t h) {
@@ -97,159 +111,160 @@ __global__ void __launch_bounds__(kScatThreads, kScatCtasPerSm) scatter_kernel(c
         return d;
     };
 
-    uint64_t n_counted = 0, first_bad_unused = ~0ULL;
-    const uint64_t tiles_per_round = (uint64_t)gridDim.x * kScatWarps;
-    const uint64_t n_rounds = (p.n_tiles + tiles_per_round - 1) / tiles_per_round;
-    auto tile_of = [&](uint64_t r) { return (r * gridDim.x + blockIdx.x) * kScatWarps + warp; };
+    uint64_t first_bad_unused = ~0ULL;
+    // tile numbers in 32 bits (launch_part_a: fewer than 2^31 tiles), so that they cost the
+    // hashing one register each
+    const uint32_t n_tiles = (uint32_t)p.n_tiles, tiles_per_round = gridDim.x * kScatWarps;
+    const uint32_t n_rounds = (n_tiles + tiles_per_round - 1) / tiles_per_round;
+    const uint32_t R = p.batch_tiles, n_batches = (n_rounds + R - 1) / R;  // batch b: rounds [b R, b R + R)
+    auto tile_of = [&](uint32_t r) { return (r * gridDim.x + blockIdx.x) * kScatWarps + warp; };
 
-    // software pipeline over rounds: the bytes and read boundaries of the next tile are fetched
-    // into registers while this one is hashed and scattered
+    // software pipeline over tiles: the bytes and read boundaries of the next tile are fetched
+    // into registers while this one is hashed
     uint4 raw = make_uint4(0, 0, 0, 0);
     uint64_t tf = 0, off = ~0ULL;
-    auto fetch = [&](uint64_t t, uint4 &raw_, uint64_t &tf_) {
-        if (t < p.n_tiles) {
-            if (lane < NV) raw_ = load_bases16(p, p.tile_base + t * kWarpTile + 16ull * lane);
+    auto fetch = [&](uint32_t t, uint4 &raw_, uint64_t &tf_) {
+        if (t < n_tiles) {
+            if (lane < NV) raw_ = load_bases16(p, p.tile_base + (uint64_t)t * kWarpTile + 16ull * lane);
             tf_ = __ldg(p.tile_first + t);
         }
     };
-    auto fetch_off = [&](uint64_t t, uint64_t tf_) {
+    auto fetch_off = [&](uint32_t t, uint64_t tf_) {
         const uint64_t rr = tf_ + lane;
-        return (t < p.n_tiles && rr < p.n_off) ? __ldg(p.offsets + rr) : ~0ULL;
+        return (t < n_tiles && rr < p.n_off) ? __ldg(p.offsets + rr) : ~0ULL;
     };
     fetch(tile_of(0), raw, tf);
     off = fetch_off(tile_of(0), tf);
 
-    // a line leaves as 2^(ls-2) lanes x 4 entries: two 128-bit shared loads, one 256-bit store
-    const uint32_t lanes_per_line = ls >= 2 ? (line >> 2) : 1u;
+    for (uint32_t b = 0; b < n_batches; ++b) {
+        const uint32_t r0 = b * R, n_here = min(r0 + R, n_rounds) - r0;
 
-    for (uint64_t r = 0; r < n_rounds; ++r) {
-        const uint64_t t = tile_of(r);
-        uint4 raw_next = make_uint4(0, 0, 0, 0);
-        uint64_t tf_next = 0;
-        fetch(tile_of(r + 1), raw_next, tf_next);
-        uint64_t h[kWPT] = {};
-        if (t < p.n_tiles) {
-            const uint64_t w0 = p.tile_base + t * kWarpTile;
-            if (lane < NE) s_end[lane] = 0;
-            __syncwarp();
-            if (lane < NV) stage16_raw<BL>(p, w0, lane, raw, s_fw, s_rc, s_bad);
-            {
-                const uint64_t e = off - 1 - w0;  // last base of a read, tile-relative (sentinel: huge)
-                if (e < (uint64_t)BL) atomicOr(&s_end[e >> 5], 1u << (e & 31));
-                if (__shfl_sync(0xffffffffu, e < (uint64_t)BL, 31)) {
-                    // more than 32 read boundaries inside one tile (tiny or empty reads): walk the rest
-                    for (uint64_t q = tf + 32 + lane; q < p.n_off; q += 32) {
-                        const uint64_t e2 = p.offsets[q] - 1 - w0;
-                        if (e2 >= (uint64_t)BL) break;
-                        atomicOr(&s_end[e2 >> 5], 1u << (e2 & 31));
+        // 1. hash this warp's tiles of the batch into its slice (tile i, window j of lane l at
+        //    i * 256 + j * 32 + l; 0 where there is no hash), counting per destination
+        for (uint32_t i = 0; i < n_here; ++i) {
+            const uint32_t r = r0 + i, t = tile_of(r);
+            uint4 raw_next = make_uint4(0, 0, 0, 0);
+            uint64_t tf_next = 0;
+            fetch(tile_of(r + 1), raw_next, tf_next);
+            uint64_t h[kWPT] = {};
+            if (t < n_tiles) {
+                const uint64_t w0 = p.tile_base + (uint64_t)t * kWarpTile;
+                if (lane < NE) s_end[lane] = 0;
+                __syncwarp();
+                if (lane < NV) stage16_raw<BL>(p, w0, lane, raw, s_fw, s_rc, s_bad);
+                {
+                    const uint64_t e = off - 1 - w0;  // last base of a read, tile-relative (sentinel: huge)
+                    if (e < (uint64_t)BL) atomicOr(&s_end[e >> 5], 1u << (e & 31));
+                    if (__shfl_sync(0xffffffffu, e < (uint64_t)BL, 31)) {
+                        // more than 32 read boundaries inside one tile (tiny or empty reads): walk the rest
+                        for (uint64_t q = tf + 32 + lane; q < p.n_off; q += 32) {
+                            const uint64_t e2 = p.offsets[q] - 1 - w0;
+                            if (e2 >= (uint64_t)BL) break;
+                            atomicOr(&s_end[e2 >> 5], 1u << (e2 & 31));
+                        }
                     }
                 }
+                __syncwarp();
+                const uint32_t valid = lane_valid_mask<K, kModePart>(p, s_bad, s_end, w0, lane, first_bad_unused);
+                if (valid) lane_hashes<K>(s_fw, s_rc, lane * kWPT, valid, h);
             }
-            __syncwarp();
-            const uint32_t valid = lane_valid_mask<K, kModePart>(p, s_bad, s_end, w0, lane, first_bad_unused);
-            if (valid) lane_hashes<K>(s_fw, s_rc, lane * kWPT, valid, h);
-        }
-        const uint64_t off_next = fetch_off(tile_of(r + 1), tf_next);  // its tile_first entry has arrived by now
-
-        // 1. every hash takes its position q in its destination's fragment
-        uint32_t dst[kWPT], q[kWPT];
+            off = fetch_off(tile_of(r + 1), tf_next);  // its tile_first entry has arrived by now
+            raw = raw_next; tf = tf_next;
 #pragma unroll
-        for (int j = 0; j < kWPT; ++j) {
-            dst[j] = 0; q[j] = 0;
-            if (h[j] != 0) { ++n_counted; dst[j] = dest_of(h[j]); q[j] = atomicAdd(&book[dst[j]].y, 1u); }
+            for (int j = 0; j < kWPT; ++j) {
+                // h = 0: a bad window, or the reference's hash==0 skip (src/lib.rs:589)
+                if (h[j] != 0) atomicAdd(&cnt[dest_of(h[j])], 1u);
+                my_slice[i * kWarpTile + j * 32 + lane] = h[j];
+            }
+            __syncwarp();  // this warp's tile buffers are restaged by its next tile
         }
         __syncthreads();
 
-        // 2. place.  With b.x = entries accounted for before this round and total = what the
-        //    fragment holds after it: positions inside the line that was being filled go into the
-        //    staged line (whoever takes its last slot lists the destination for the flush);
-        //    positions in further complete lines (rare) go straight out; positions beyond the last
-        //    complete line wait for the flush; positions beyond the fragment spill.
-        uint32_t later = 0, spilled = 0, last = 0;
-        uint2 bk[kWPT];  // all books first: the loads are independent, the stores below are not
+        // 2. run starts: an exclusive scan of the counts, warp w taking destinations [256 w, 256 w + 256)
+        //    (what lies before them it adds up itself); every warp loads its slice into registers
+        if (warp * 256u < nd) {
+            const uint32_t lo = warp * 256u;
+            uint32_t carry = 0;
+            for (uint32_t d = lane; d < lo; d += 32) carry += cnt[d];
+            carry = __reduce_add_sync(0xffffffffu, carry);
+            uint32_t v[8], x[8];
 #pragma unroll
-        for (int j = 0; j < kWPT; ++j) bk[j] = book[dst[j]];
+            for (int u = 0; u < 8; ++u) {
+                const uint32_t d = lo + 32 * u + lane;
+                v[u] = d < nd ? cnt[d] : 0u;
+                x[u] = v[u];
+            }
 #pragma unroll
-        for (int j = 0; j < kWPT; ++j) {
-            if (h[j] == 0) continue;
-            const uint2 b = bk[j];
-            const uint32_t total = min(b.y, p.frag_cap), line_end = (b.x & ~(line - 1)) + line;
-            if (q[j] >= total) { spilled |= 1u << j; continue; }
-            if (q[j] + 1 == total) last |= 1u << j;
-            if (q[j] < line_end) {
-                stage[((size_t)dst[j] << ls) + (q[j] & (line - 1))] = h[j];
-                if (q[j] + 1 == line_end) flist[atomicAdd(s_nflush, 1u)] = dst[j];
-            } else if (q[j] < (total & ~(line - 1))) my_frag[dst[j] * frag_row + q[j]] = h[j];
-            else later |= 1u << j;
-        }
-        if (__any_sync(0xffffffffu, spilled != 0)) {
-            // skewed input (one k-mer flooding its partition): one reservation per warp tile
-            const uint32_t mine = __popc(spilled);
-            uint32_t incl = mine;
             for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += v;
-            }
-            const uint32_t tot = __shfl_sync(0xffffffffu, incl, 31);
-            unsigned long long base = 0;
-            if (lane == 0) base = atomicAdd(p.spill_n, (unsigned long long)tot);
-            base = __shfl_sync(0xffffffffu, base, 0) + (incl - mine);
 #pragma unroll
-            for (int j = 0; j < kWPT; ++j)
-                if ((spilled >> j) & 1u) { if (base < p.spill_cap) p.spill[base] = h[j]; ++base; }
-        }
-        __syncthreads();
-
-        // 3. flush the completed lines
-        {
-            const uint32_t n_flush = *s_nflush;
-            if (ls >= 2) {
-                const uint32_t per_warp = 32u / lanes_per_line, sub = lane / lanes_per_line, li = (lane % lanes_per_line) * 4;
-                for (uint32_t e = warp * per_warp + sub; e < n_flush; e += kScatWarps * per_warp) {
-                    const uint32_t d = flist[e];
-                    const uint64_t *src = stage + ((size_t)d << ls) + li;
-                    const ulonglong2 v0 = *reinterpret_cast<const ulonglong2 *>(src), v1 = *reinterpret_cast<const ulonglong2 *>(src + 2);
-                    uint64_t *dstp = my_frag + d * frag_row + (book[d].x & ~(line - 1)) + li;
-                    asm volatile("st.global.v4.u64 [%0], {%1,%2,%3,%4};" ::"l"(dstp), "l"(v0.x), "l"(v0.y), "l"(v1.x), "l"(v1.y) : "memory");
-                }
-            } else {
-                const uint32_t per_warp = 32u >> ls, sub = lane >> ls, li = lane & (line - 1);
-                for (uint32_t e = warp * per_warp + sub; e < n_flush; e += kScatWarps * per_warp) {
-                    const uint32_t d = flist[e];
-                    my_frag[d * frag_row + (book[d].x & ~(line - 1)) + li] = stage[((size_t)d << ls) + li];
+                for (int u = 0; u < 8; ++u) {
+                    const uint32_t y = __shfl_up_sync(0xffffffffu, x[u], o);
+                    if (lane >= o) x[u] += y;
                 }
             }
+#pragma unroll
+            for (int u = 0; u < 8; ++u) {
+                const uint32_t d = lo + 32 * u + lane;
+                if (d < nd) {
+                    const uint32_t start = carry + x[u] - v[u], fill = min(to_frag[d] + pos[d], p.frag_cap);
+                    pos[d] = start; to_frag[d] = fill - start;
+                }
+                carry += __shfl_sync(0xffffffffu, x[u], 31);
+            }
+            if (lane == 0 && lo + 256u >= nd) { *s_total = carry; *s_counted += carry; }
         }
+        uint64_t v[kMaxPerLane];
+#pragma unroll
+        for (int u = 0; u < kMaxPerLane; ++u) v[u] = u < (int)(n_here * kWPT) ? my_slice[u * 32 + lane] : 0ull;
         __syncthreads();
 
-        // 4. what lies beyond the flushed lines moves in at the front of its line; whoever took a
-        //    destination's last position of the round brings its book up to date
+        // 3. permute: every hash to its destination's run; the counts are cleared for the next batch
+        for (uint32_t d = threadIdx.x; d < nd; d += kScatThreads) cnt[d] = 0;
 #pragma unroll
-        for (int j = 0; j < kWPT; ++j) {
-            if ((later >> j) & 1u) stage[((size_t)dst[j] << ls) + (q[j] & (line - 1))] = h[j];
-            if ((last >> j) & 1u) book[dst[j]].x = q[j] + 1;
+        for (int u = 0; u < kMaxPerLane; ++u)
+            if (v[u] != 0) batch[atomicAdd(&pos[dest_of(v[u])], 1u)] = v[u];
+        __syncthreads();
+
+        // 4. write out: consecutive lanes store consecutive entries of a run; four chunks of 32
+        //    entries per warp at a time, so that the loads and stores of one do not wait for another's
+        const uint32_t total = *s_total;
+        for (uint32_t i0 = warp * 128; i0 < total; i0 += kScatThreads * 4) {
+            uint64_t h[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const uint32_t i = i0 + 32 * u + lane;
+                h[u] = i < total ? batch[i] : 0ull;  // (a sorted entry is never 0)
+            }
+            uint32_t spilled = 0;
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                if (h[u] == 0) continue;
+                const uint32_t d = dest_of(h[u]), at = i0 + 32 * u + lane + to_frag[d];
+                if (at < p.frag_cap) my_frag[d * frag_row + at] = h[u];
+                else spilled |= 1u << u;
+            }
+            if (__any_sync(0xffffffffu, spilled != 0)) {
+                // skewed input (one k-mer flooding its partition): one reservation per warp and 128 entries
+                const uint32_t mine = __popc(spilled);
+                uint32_t incl = mine;
+                for (int o = 1; o < 32; o <<= 1) {
+                    const uint32_t y = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += y;
+                }
+                unsigned long long base = 0;
+                if (lane == 31) base = atomicAdd(p.spill_n, (unsigned long long)incl);
+                base = __shfl_sync(0xffffffffu, base, 31) + (incl - mine);
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    if ((spilled >> u) & 1u) { if (base < p.spill_cap) p.spill[base] = h[u]; ++base; }
+            }
         }
-        if (threadIdx.x == 0) *s_nflush = 0;
-        // (no barrier here: the next round's step 1 touches only the arrival counters, and its
-        // barrier comes before anything reads what step 4 wrote)
-        raw = raw_next; tf = tf_next; off = off_next;
+        __syncthreads();
     }
 
-    __syncthreads();
-    // what is still staged: the last line of every destination goes out whole, its unused slots
-    // holding 0 (never a hash: pass A drops it, src/lib.rs:589) so that fill counts stay multiples
-    // of the line and a later launch can continue the fragment
-    {
-        const uint32_t per_warp = 32u >> ls, sub = lane >> ls, li = lane & (line - 1);
-        for (uint32_t d = warp * per_warp + sub; d < nd; d += kScatWarps * per_warp) {
-            const uint32_t pos = book[d].x, part = pos & (line - 1);
-            if (part) my_frag[d * frag_row + (pos - part) + li] = li < part ? stage[((size_t)d << ls) + li] : 0ull;
-        }
-        for (uint32_t d = threadIdx.x; d < nd; d += kScatThreads)
-            p.frag_cnt[(uint64_t)d * gridDim.x + blockIdx.x] = min((book[d].x + line - 1) & ~(line - 1), p.frag_cap);
-    }
-    for (int o = 16; o; o >>= 1) n_counted += __shfl_xor_sync(0xffffffffu, n_counted, o);
-    if (lane == 0 && n_counted) atomicAdd((unsigned long long *)&p.table.ctrl->counted, (unsigned long long)n_counted);
+    for (uint32_t d = threadIdx.x; d < nd; d += kScatThreads)
+        p.frag_cnt[(uint64_t)d * gridDim.x + blockIdx.x] = min(to_frag[d] + pos[d], p.frag_cap);
+    if (threadIdx.x == 0 && *s_counted) atomicAdd((unsigned long long *)&p.table.ctrl->counted, *s_counted);
 }
 
 }  // namespace oxg
