@@ -207,12 +207,12 @@ __device__ __forceinline__ uint64_t load_segments(const LookupSources &src, int 
     return seg_at[src.n];
 }
 
-// the rank whose segment holds entry i of that range: the entry is at seg_lo[s] + (i - seg_at[s])
-// of rank s's region
-__device__ __forceinline__ int segment_of(const uint64_t *seg_at, uint64_t i) {
+// entry i of that range: position `at` of rank `s`'s region
+struct SegEntry { int s; uint64_t at; };
+__device__ __forceinline__ SegEntry entry_of(const uint64_t *seg_lo, const uint64_t *seg_at, uint64_t i) {
     int s = 0;
     while (i >= seg_at[s + 1]) ++s;
-    return s;
+    return SegEntry{s, seg_lo[s] + (i - seg_at[s])};
 }
 
 // Answers every rank's queries of the round: four keys per thread are loaded (coalesced, over
@@ -231,8 +231,8 @@ __global__ void __launch_bounds__(kOpThreads) answer_queries_kernel(TableView t,
             p[j] = nullptr;
             key[j] = 0;
             if (i < total) {
-                const int s = segment_of(seg_at, i);
-                p[j] = src.frag[s] + seg_lo[s] + (i - seg_at[s]);
+                const SegEntry e = entry_of(seg_lo, seg_at, i);
+                p[j] = src.frag[e.s] + e.at;
                 key[j] = __ldcg(p[j]);
                 live |= 1u << j;
             }
@@ -276,10 +276,9 @@ __global__ void __launch_bounds__(kOpThreads) apply_pairs_kernel(TableView t, Pa
             key[j] = 0;
             val[j] = 0;
             if (i < total) {
-                const int s = segment_of(seg_at, i);
-                const uint64_t at = seg_lo[s] + (i - seg_at[s]);
-                key[j] = __ldcg(src.keys.frag[s] + at);
-                val[j] = __ldcg(src.vals[s] + at);
+                const SegEntry e = entry_of(seg_lo, seg_at, i);
+                key[j] = __ldcg(src.keys.frag[e.s] + e.at);
+                val[j] = __ldcg(src.vals[e.s] + e.at);
                 live |= 1u << j;
             }
         }
@@ -311,8 +310,8 @@ __global__ void __launch_bounds__(32) erase_walk_segments_kernel(TableView t, Lo
     if (gtid() != 0) return;
     uint64_t removed = 0;
     for (uint64_t i = 0; i < total; ++i) {
-        const int s = segment_of(seg_at, i);
-        erase_one(t, __ldcg(src.frag[s] + seg_lo[s] + (i - seg_at[s])), removed);
+        const SegEntry e = entry_of(seg_lo, seg_at, i);
+        erase_one(t, __ldcg(src.frag[e.s] + e.at), removed);
     }
     t.ctrl->scratch[0] += removed;
 }
@@ -337,8 +336,8 @@ __global__ void __launch_bounds__(kOpThreads) erase_mark_segments_kernel(TableVi
             const uint64_t i = base + j * stride;
             key[j] = 0;
             if (i < total) {
-                const int s = segment_of(seg_at, i);
-                key[j] = __ldcg(src.frag[s] + seg_lo[s] + (i - seg_at[s]));
+                const SegEntry e = entry_of(seg_lo, seg_at, i);
+                key[j] = __ldcg(src.frag[e.s] + e.at);
                 live |= 1u << j;
             }
         }

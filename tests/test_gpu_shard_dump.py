@@ -235,8 +235,8 @@ def crafted_shards(capi, world, pairs_of_rank, k=21):
 
 def test_crafted_digits_zero_counts_an_empty_rank_and_many_counts(capi, tmp_path):
     """keys and counts of every decimal length (0 and 2^64-1 included), rank 1 owning nothing, more
-    than 65 536 distinct counts on rank 0 (its per-count blocks cross several all-gather pieces) and
-    4 M keys on rank 3 (its text crosses several chunk boundaries)"""
+    than 65 536 distinct counts on rank 0 (its per-count blocks and its histogram cross several
+    all-gather pieces) and 4 M keys on rank 3 (its text crosses several chunk boundaries)"""
     from oxli_b200.sharded import owner_of
 
     world = 4
@@ -263,6 +263,8 @@ def test_crafted_digits_zero_counts_an_empty_rank_and_many_counts(capi, tmp_path
     assert n3 > 4 * (min(rw, 4 << 20) // 1024 * 1024)  # five chunks of text on rank 3 (the fewest pairs a round holds: 0.9 Mi on a B200)
     model = check_export_and_dump(capi, shards, tmp_path, 21)
     assert model[2][1][0] == 0 and model[2][1][-1] == TOP and model[1][0][-1] == TOP
+    freq, n = np.unique(model[2][1], return_counts=True)  # the sparse histogram of every count
+    assert each_rank(shards, lambda r: shards[r].engine.histo()) == [list(zip(freq.tolist(), n.tolist()))] * world
     for s in shards:
         s.close()
 

@@ -176,17 +176,21 @@ def make_list(rng, keys, size, extra=()):
 
 # ---- 1. lists over several rounds (mark and rebuild) --------------------------------------------
 
-@pytest.mark.parametrize("world", [1, 2, 4, 8])
-def test_drop_lists_in_one_process_vs_model(capi, world):
+# "staged": rounds of 2.5 Mi keys, so that rank 0's host list crosses in several pieces of the
+# shard's 1 Mi-entry staging buffer per round, the last of them partly filled
+@pytest.mark.parametrize("world,round_windows", [(1, 1 << 16), (2, 1 << 16), (4, 1 << 16), (8, 1 << 16), (4, 5 << 19)],
+                         ids=["1", "2", "4", "8", "4-staged"])
+def test_drop_lists_in_one_process_vs_model(capi, world, round_windows):
     from oxli_b200.sharded import owner_of
 
     k = 21 if world % 4 else 31
     bases, offs = reads(71, 16_000)
     d = oracle_dict(k, bases, offs)
-    shards = consumed_shards(capi, world, k, bases, offs)
+    shards = consumed_shards(capi, world, k, bases, offs, round_windows)
     shards[world - 1].engine.table.set_hash(TOP, 7)  # 2^64-1 lives in its owner's side entry
     d[TOP] = 7
     Q = shards[0].engine.info()["round_windows"]  # keys per rank and round
+    assert Q >= round_windows
     keys = np.array(sorted(d), dtype=np.uint64)
     rng = np.random.default_rng(world)
     # rank 0 needs three rounds, the others less, rank 1 nothing; 2^64-1 from rank 0 and the last

@@ -104,8 +104,11 @@ def lookup_all(shards, queries):
     return got
 
 
-@pytest.mark.parametrize("world", [1, 2, 4, 8])
-def test_lookups_in_one_process_vs_oracle(capi, world):
+# "staged": rounds of 2.5 Mi queries, so that a host list's round crosses in several pieces of the
+# shard's 1 Mi-entry staging buffer (on ranks 0 and 2), the last of them partly filled
+@pytest.mark.parametrize("world,round_windows", [(1, 1 << 16), (2, 1 << 16), (4, 1 << 16), (8, 1 << 16), (4, 5 << 19)],
+                         ids=["1", "2", "4", "8", "4-staged"])
+def test_lookups_in_one_process_vs_oracle(capi, world, round_windows):
     from oxli_b200.sharded import owner_of
 
     k = 21 if world % 4 else 31
@@ -115,8 +118,9 @@ def test_lookups_in_one_process_vs_oracle(capi, world):
     truth = OracleTable(k)
     truth.consume_batch(bases, offs, True, nthreads=4)
     tk, tv = truth.items_sorted()
-    shards = consumed_shards(capi, world, k, bases, offs)
+    shards = consumed_shards(capi, world, k, bases, offs, round_windows)
     Q = shards[0].engine.info()["round_windows"]  # queries per rank and round
+    assert Q >= round_windows
     # rank 0 needs three rounds; the others ask less, and rank 1 nothing at all
     sizes = [2 * Q + 1] + [0 if r == 1 else Q // r + r for r in range(1, world)]
     rng = np.random.default_rng(world)
