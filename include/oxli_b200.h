@@ -361,6 +361,12 @@ oxg_status oxg_timer_start(oxg_table *t);
 oxg_status oxg_timer_stop(oxg_table *t, float *ms);
 /* kernels launched by this library in this process so far (bench bookkeeping) */
 uint64_t oxg_launch_count(void);
+/* CUDA buffers, events and streams the library holds now (tests: what an error return leaves) */
+uint64_t oxg_live_allocations(void);
+/* tests: the n-th allocation or handle creation of the library from now on fails as if the
+ * device were out of memory (OXG_ERR_NOMEM); 0 = none.  Returns the countdown it replaces:
+ * 0 once the failure it set has happened (or none was set) */
+uint64_t oxg_fail_allocation_after(uint64_t n);
 /* device-time of the consume kernels of the last oxg_consume_* call on `t`, in
  * milliseconds, and their number (CUDA events on the launch stream) */
 oxg_status oxg_last_consume_kernel_ms(oxg_table *t, float *ms, uint64_t *launches);

@@ -110,6 +110,8 @@ SIGNATURES = {
     "oxg_timer_start": (C.c_int, [vp]),
     "oxg_timer_stop": (C.c_int, [vp, C.POINTER(C.c_float)]),
     "oxg_launch_count": (u64, []),
+    "oxg_live_allocations": (u64, []),
+    "oxg_fail_allocation_after": (u64, [u64]),
     "oxg_last_consume_kernel_ms": (C.c_int, [vp, C.POINTER(C.c_float), u64p]),
     "oxg_set_pipeline": (C.c_int, [C.c_int, C.c_uint32, C.c_uint32]),
     "oxg_last_consume_pass_ms": (C.c_int, [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]),

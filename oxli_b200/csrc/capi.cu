@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <deque>
 #include <functional>
 #include <memory>
 #include <mutex>
@@ -37,6 +38,7 @@
 #include "shard.cuh"
 #include "sortexport.cuh"
 #include "tableops.cuh"
+#include "owned.h"
 
 using namespace oxg;
 
@@ -133,66 +135,36 @@ struct HostBatch {
 // source is pageable) and its batch-relative read boundaries; ev_ready[b] marks its copies
 // landed, ev_free[b] (recorded by whoever launches the kernels) the kernels done reading it.
 struct StageRing {
-    cudaStream_t copy = nullptr;  // the H2D copies
-    uint8_t *d_bases[kStageBufs] = {}, *h_bases[kStageBufs] = {};
-    uint64_t d_cap[kStageBufs] = {}, h_cap[kStageBufs] = {};
-    uint64_t *d_offs[kStageBufs] = {}, *h_offs[kStageBufs] = {};
-    uint64_t offs_cap[kStageBufs] = {};
+    DeviceArray<uint8_t> d_bases[kStageBufs];
+    PinnedArray<uint8_t> h_bases[kStageBufs];
+    DeviceArray<uint64_t> d_offs[kStageBufs];
+    PinnedArray<uint64_t> h_offs[kStageBufs];
     uint64_t n_off[kStageBufs] = {};  // boundaries of the chunk staged in buffer b, sentinel included
-    cudaEvent_t ev_ready[kStageBufs] = {}, ev_free[kStageBufs] = {};
+    Event ev_ready[kStageBufs], ev_free[kStageBufs];
+    Stream copy;  // the H2D copies (declared last: drained and gone before the buffers it reads)
 
     oxg_status init() {
-        CU(cudaStreamCreateWithFlags(&copy, cudaStreamNonBlocking));
-        for (int b = 0; b < kStageBufs; ++b) {
-            CU(cudaEventCreateWithFlags(&ev_ready[b], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&ev_free[b], cudaEventDisableTiming));
-        }
+        CU(copy.create(cudaStreamNonBlocking));
+        for (int b = 0; b < kStageBufs; ++b) { CU(ev_ready[b].create(cudaEventDisableTiming)); CU(ev_free[b].create(cudaEventDisableTiming)); }
         return OXG_OK;
-    }
-
-    void release() {
-        cudaStreamSynchronize(copy);
-        for (int b = 0; b < kStageBufs; ++b) {
-            cudaEventDestroy(ev_ready[b]); cudaEventDestroy(ev_free[b]);
-            cudaFree(d_bases[b]); cudaFreeHost(h_bases[b]); cudaFree(d_offs[b]); cudaFreeHost(h_offs[b]);
-        }
-        cudaStreamDestroy(copy);
     }
 
     // Buffers 0..n_bufs-1 take chunks of `bytes`.  A device buffer is replaced once `kernels` has
     // drained, a pinned one (needed for pageable sources only) once the copy stream has.
     oxg_status reserve(int n_bufs, uint64_t bytes, bool src_pinned, cudaStream_t kernels) {
         for (int b = 0; b < n_bufs; ++b) {
-            if (d_cap[b] < bytes) {
-                CU(cudaStreamSynchronize(kernels));
-                if (d_bases[b]) CU(cudaFree(d_bases[b]));
-                d_bases[b] = nullptr; d_cap[b] = 0;
-                CU(cudaMalloc(&d_bases[b], bytes));
-                d_cap[b] = bytes;
-            }
-            if (!src_pinned && h_cap[b] < bytes) {
-                CU(cudaStreamSynchronize(copy));
-                if (h_bases[b]) CU(cudaFreeHost(h_bases[b]));
-                h_bases[b] = nullptr; h_cap[b] = 0;
-                CU(cudaMallocHost(&h_bases[b], bytes));
-                h_cap[b] = bytes;
-            }
+            if (d_bases[b].cap() < bytes) { CU(cudaStreamSynchronize(kernels)); CU(d_bases[b].reserve(bytes)); }
+            if (!src_pinned && h_bases[b].cap() < bytes) { CU(cudaStreamSynchronize(copy)); CU(h_bases[b].reserve(bytes)); }
         }
         return OXG_OK;
     }
 
     // room for n boundaries in buffer b; `kernels` (if any) is drained too before the old ones go
     oxg_status reserve_offs(int b, uint64_t n, cudaStream_t kernels) {
-        if (offs_cap[b] >= n) return OXG_OK;
+        if (d_offs[b].cap() >= n && h_offs[b].cap() >= n) return OXG_OK;
         CU(cudaStreamSynchronize(copy));
         if (kernels) CU(cudaStreamSynchronize(kernels));
-        if (d_offs[b]) CU(cudaFree(d_offs[b]));
-        if (h_offs[b]) CU(cudaFreeHost(h_offs[b]));
-        d_offs[b] = nullptr; h_offs[b] = nullptr; offs_cap[b] = 0;
-        const uint64_t ncap = std::max<uint64_t>(n, 1 << 16);
-        CU(cudaMalloc(&d_offs[b], ncap * 8));
-        CU(cudaMallocHost(&h_offs[b], ncap * 8));
-        offs_cap[b] = ncap;
+        CU(d_offs[b].reserve(n, 1 << 16)); CU(h_offs[b].reserve(n, 1 << 16));
         return OXG_OK;
     }
 
@@ -215,13 +187,13 @@ struct StageRing {
             CU(cudaStreamWaitEvent(copy, ev_free[b], 0));
         }
         TRY(reserve_offs(b, n + 1, kernels));
-        for (uint64_t i = 0; i < n; ++i) h_offs[b][i] = ob[i] - base0;
-        h_offs[b][n] = ~0ULL >> 1;  // sentinel keeps n_off >= 1
+        for (uint64_t i = 0; i < n; ++i) h_offs[b].get()[i] = ob[i] - base0;
+        h_offs[b].get()[n] = ~0ULL >> 1;  // sentinel keeps n_off >= 1
         n_off[b] = n + 1;
         const uint8_t *src = h.bases + base0 + lo;
-        if (!h.pinned) { memcpy(h_bases[b], src, hi - lo); src = h_bases[b]; }
-        CU(cudaMemcpyAsync(d_bases[b], src, hi - lo, cudaMemcpyHostToDevice, copy));
-        CU(cudaMemcpyAsync(d_offs[b], h_offs[b], n_off[b] * 8, cudaMemcpyHostToDevice, copy));
+        if (!h.pinned) { memcpy(h_bases[b].get(), src, hi - lo); src = h_bases[b].get(); }
+        CU(cudaMemcpyAsync(d_bases[b].get(), src, hi - lo, cudaMemcpyHostToDevice, copy));
+        CU(cudaMemcpyAsync(d_offs[b].get(), h_offs[b].get(), n_off[b] * 8, cudaMemcpyHostToDevice, copy));
         CU(cudaEventRecord(ev_ready[b], copy));
         return OXG_OK;
     }
@@ -231,44 +203,42 @@ struct StageRing {
 // list launches defer into, and the one a replay of it defers into.  Fixed lists are allocated
 // once and never enlarged (a shard's: see oxg_table::pooled).
 struct DeferLists {
-    ulonglong2 *d_pairs = nullptr;   uint64_t cap = 0;
-    ulonglong2 *d_pairs2 = nullptr;  uint64_t cap2 = 0;
+    DeviceArray<ulonglong2> pairs, pairs2;
     bool fixed = false;
 };
 
 struct DeviceCtx {
     int dev = -1;
     int sms = 0;
-    cudaStream_t stream = nullptr;
+    Stream stream;
     std::mutex mu;
     StageRing ring;  // host batches
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_mid = nullptr;
-    cudaEvent_t ev_user0 = nullptr, ev_user1 = nullptr;
+    Event ev_t0, ev_t1, ev_mid, ev_user0, ev_user1;
     // scratch
-    uint64_t *d_tile_first = nullptr; uint64_t tile_first_cap = 0;
+    DeviceArray<uint64_t> d_tile_first;
     DeferLists defer;                 // tables of this context that are not shards
-    uint64_t *d_dense = nullptr;      // kHistDense bins
-    uint64_t *d_big = nullptr;        uint64_t big_cap = 0;
-    uint64_t *d_io = nullptr;         uint64_t io_cap = 0;   // generic u64 in/out scratch (device)
-    uint64_t *h_io = nullptr;         uint64_t h_io_cap = 0; // pinned mirror
-    double *d_f64 = nullptr;          // 4 doubles
-    uint8_t *d_seq = nullptr;         uint64_t seq_cap = 0;  // hash_windows input
+    DeviceArray<uint64_t> d_dense;    // kHistDense bins
+    DeviceArray<uint64_t> d_big;
+    DeviceArray<uint64_t> d_io;       // generic u64 in/out scratch (device)
+    PinnedArray<uint64_t> h_io;       // pinned mirror
+    DeviceArray<double> d_f64;        // 4 doubles
+    DeviceArray<uint8_t> d_seq;       // hash_windows input
     // partitioned pipeline (pass A output): fragments, their fill counts, the spill list
-    uint64_t *d_frag = nullptr;       uint64_t frag_cap = 0;
-    uint32_t *d_frag_cnt = nullptr;   uint64_t frag_cnt_cap = 0;
-    uint64_t *d_spill = nullptr;      uint64_t spill_cap = 0;
-    unsigned long long *d_spill_n = nullptr;
+    DeviceArray<uint64_t> d_frag;
+    DeviceArray<uint32_t> d_frag_cnt;
+    DeviceArray<uint64_t> d_spill;
+    DeviceArray<unsigned long long> d_spill_n;
     // export: compacted pairs, the second pair of arrays of the radix sort, its histogram, pinned bounce buffers
-    uint64_t *d_exp_k[2] = {}, *d_exp_v[2] = {};
-    uint64_t exp_cap[2] = {};
-    uint64_t *d_exp_counts = nullptr; uint64_t exp_counts_cap = 0;
-    uint64_t *d_sort_hist = nullptr;  uint64_t sort_hist_cap = 0;
-    uint8_t *h_bounce[2] = {};
-    cudaEvent_t ev_bounce[2] = {};
+    DeviceArray<uint64_t> d_exp_k[2], d_exp_v[2];
+    DeviceArray<uint64_t> d_exp_counts;
+    DeviceArray<uint64_t> d_sort_hist;
+    PinnedArray<uint8_t> h_bounce[2];
+    Event ev_bounce[2];
 };
 
+// never destroyed: their owners would release after the CUDA runtime may have gone at exit
 std::mutex g_ctx_mu;
-std::vector<std::unique_ptr<DeviceCtx>> g_ctx;
+std::vector<DeviceCtx *> g_ctx;
 
 oxg_status get_ctx(int dev, DeviceCtx **out) {
     std::lock_guard<std::mutex> lk(g_ctx_mu);
@@ -289,41 +259,22 @@ oxg_status get_ctx(int dev, DeviceCtx **out) {
             return fail(OXG_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only",
                         dev, prop.major, prop.minor);
         c->sms = prop.multiProcessorCount;
-        CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+        CU(c->stream.create(cudaStreamNonBlocking));
         TRY(c->ring.init());
-        CU(cudaEventCreate(&c->ev_t0));
-        CU(cudaEventCreate(&c->ev_t1));
-        CU(cudaEventCreate(&c->ev_mid));
-        CU(cudaEventCreate(&c->ev_user0));
-        CU(cudaEventCreate(&c->ev_user1));
-        CU(cudaMalloc(&c->d_dense, kHistDense * sizeof(uint64_t)));
-        CU(cudaMalloc(&c->d_f64, 4 * sizeof(double)));
-        g_ctx[dev] = std::move(c);
+        for (Event *e : {&c->ev_t0, &c->ev_t1, &c->ev_mid, &c->ev_user0, &c->ev_user1}) CU(e->create(cudaEventDefault));
+        CU(c->d_dense.reserve(kHistDense));
+        CU(c->d_f64.reserve(4));
+        g_ctx[dev] = c.release();
     }
-    *out = g_ctx[dev].get();
+    *out = g_ctx[dev];
     return OXG_OK;
 }
 
-template <class T>
-oxg_status ensure_dev(T **p, uint64_t *cap, uint64_t want) {
-    if (*cap >= want && *p) return OXG_OK;
-    if (*p) CU(cudaFree(*p));
-    *p = nullptr; *cap = 0;
-    uint64_t ncap = std::max<uint64_t>(want, 1024);
-    CU(cudaMalloc(p, ncap * sizeof(T)));
-    *cap = ncap;
-    return OXG_OK;
-}
+constexpr uint64_t kScratchMin = 1024;  // entries of a scratch array at least
 
 oxg_status ensure_io(DeviceCtx *c, uint64_t n) {
-    TRY(ensure_dev(&c->d_io, &c->io_cap, n));
-    if (c->h_io_cap < n) {
-        if (c->h_io) CU(cudaFreeHost(c->h_io));
-        c->h_io = nullptr; c->h_io_cap = 0;
-        uint64_t ncap = std::max<uint64_t>(n, 1024);
-        CU(cudaMallocHost(&c->h_io, ncap * sizeof(uint64_t)));
-        c->h_io_cap = ncap;
-    }
+    CU(c->d_io.reserve(n, kScratchMin));
+    CU(c->h_io.reserve(n, kScratchMin));
     return OXG_OK;
 }
 
@@ -401,10 +352,9 @@ struct PartPlan {
 struct oxg_table {
     DeviceCtx *ctx = nullptr;
     uint32_t k = 0;
-    ulonglong2 *slots = nullptr;
-    uint64_t cap = 0;
-    Ctrl *d_ctrl = nullptr;
-    Ctrl *h_ctrl = nullptr;  // pinned
+    DeviceArray<ulonglong2> slots;  // (its capacity is the table's)
+    DeviceArray<Ctrl> d_ctrl;
+    PinnedArray<Ctrl> h_ctrl;
     uint64_t size = 0;       // host mirror of ctrl->size as of the last sync
     bool hinted = false;     // the caller said how many distinct keys to expect
     uint64_t hint_keys = 0;  // ... and this many
@@ -421,8 +371,8 @@ struct oxg_table {
     uint64_t part_budget = 0;  // windows the running consume call still has to go (0 = unknown)
     uint32_t group_cap = 0;    // != 0: at most this many pass A launches per pass B in the running call
     // HyperLogLog sketch of the keys that came in through the partitioned pipeline (aggregate.cuh)
-    uint32_t *d_sketch = nullptr;
-    uint32_t *h_sketch = nullptr;  // pinned
+    DeviceArray<uint32_t> d_sketch;
+    PinnedArray<uint32_t> h_sketch;
     uint64_t sketch_covers = 0;    // keys of the table the sketch has seen
     uint64_t est_keys = 0;         // the sketch's last word on how many keys the table is about to hold
     uint64_t last_made = 0;        // keys the previous group of launches created
@@ -436,29 +386,29 @@ namespace {
 // the table as its kernels see it; `defer` (nullptr: none) takes what runs into the load limit
 TableView view_of(const oxg_table *t, const DeferLists *defer = nullptr) {
     TableView v;
-    v.slots = t->slots;
-    v.cap = t->cap;
+    v.slots = t->slots.get();
+    v.cap = t->slots.cap();
     uint32_t lg = 0;
-    while ((1ull << lg) < t->cap) ++lg;
+    while ((1ull << lg) < t->slots.cap()) ++lg;
     v.shift = 64 - lg;
-    v.limit = t->cap - t->cap / 5;  // stop creating keys at 80 % load
-    v.ctrl = t->d_ctrl;
-    v.overflow = defer ? defer->d_pairs : nullptr;
-    v.overflow_cap = defer ? defer->cap : 0;
+    v.limit = t->slots.cap() - t->slots.cap() / 5;  // stop creating keys at 80 % load
+    v.ctrl = t->d_ctrl.get();
+    v.overflow = defer ? defer->pairs.get() : nullptr;
+    v.overflow_cap = defer ? defer->pairs.cap() : 0;
     return v;
 }
 
 oxg_status pull_ctrl(oxg_table *t) {
     DeviceCtx *c = t->ctx;
-    CU(cudaMemcpyAsync(t->h_ctrl, t->d_ctrl, sizeof(Ctrl), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(t->h_ctrl.get(), t->d_ctrl.get(), sizeof(Ctrl), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    t->size = t->h_ctrl->size;
+    t->size = t->h_ctrl.get()->size;
     return OXG_OK;
 }
 
 // zero the ctrl fields [first, first+n) (in uint64 units)
 oxg_status zero_ctrl_fields(oxg_table *t, size_t first_field, size_t n_fields) {
-    CU(cudaMemsetAsync(reinterpret_cast<uint64_t *>(t->d_ctrl) + first_field, 0, n_fields * 8, t->ctx->stream));
+    CU(cudaMemsetAsync(reinterpret_cast<uint64_t *>(t->d_ctrl.get()) + first_field, 0, n_fields * 8, t->ctx->stream));
     return OXG_OK;
 }
 constexpr size_t kFieldCounted = offsetof(Ctrl, counted) / 8;
@@ -466,39 +416,32 @@ constexpr size_t kFieldTile = offsetof(Ctrl, tile_counter) / 8;
 constexpr size_t kLaunchFields = (offsetof(Ctrl, scratch) - offsetof(Ctrl, counted)) / 8;
 constexpr size_t kFieldScratch = offsetof(Ctrl, scratch) / 8;
 
-oxg_status alloc_slots(const oxg_table *t, uint64_t cap, ulonglong2 **out) {
+// a fresh slot array of cap slots, stream-ordered for a pooled table
+oxg_status alloc_slots(const oxg_table *t, uint64_t cap, DeviceArray<ulonglong2> *out) {
     DeviceCtx *c = t->ctx;
-    if (t->pooled) CU(cudaMallocAsync(out, cap * sizeof(ulonglong2), c->stream));
-    else CU(cudaMalloc(out, cap * sizeof(ulonglong2)));  // (cudaMallocAsync pools were 2x slower for growing multi-GB tables)
-    init_slots_kernel<<<grid_for(c, cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(*out, cap);
+    if (t->pooled) *out = DeviceArray<ulonglong2>(c->stream);  // (pools were 2x slower for growing multi-GB plain tables)
+    CU(out->reserve(cap));
+    init_slots_kernel<<<grid_for(c, cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(out->get(), cap);
     LAUNCHED();
     CU(cudaGetLastError());
-    return OXG_OK;
-}
-
-oxg_status free_slots(const oxg_table *t, ulonglong2 *p) {
-    if (t->pooled) CU(cudaFreeAsync(p, t->ctx->stream)); else CU(cudaFree(p));
     return OXG_OK;
 }
 
 // grow so that `keys` distinct keys sit at <= 50 % load
 oxg_status grow_to_fit(oxg_table *t, uint64_t keys) {
     const uint64_t want = slots_for(keys);
-    if (want <= t->cap) return OXG_OK;
+    if (want <= t->slots.cap()) return OXG_OK;
     DeviceCtx *c = t->ctx;
-    ulonglong2 *fresh = nullptr;
-    TRY(alloc_slots(t, want, &fresh));
-    ulonglong2 *old = t->slots;
-    const uint64_t old_cap = t->cap;
-    t->slots = fresh;
-    t->cap = want;
+    DeviceArray<ulonglong2> old;
+    TRY(alloc_slots(t, want, &old));
+    std::swap(t->slots, old);
     if (t->size) {
-        rehash_kernel<<<grid_for(c, old_cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, old_cap, view_of(t));
+        rehash_kernel<<<grid_for(c, old.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(old.get(), old.cap(), view_of(t));
         LAUNCHED();
         CU(cudaGetLastError());
     }
     CU(cudaStreamSynchronize(c->stream));
-    return free_slots(t, old);
+    return OXG_OK;
 }
 
 oxg_status reserve_keys(oxg_table *t, uint64_t extra) { return grow_to_fit(t, t->size + extra); }
@@ -509,21 +452,20 @@ oxg_status reserve_keys(oxg_table *t, uint64_t extra) { return grow_to_fit(t, t-
 // key goes too.  *removed (if given): the keys dropped, the out-of-band one included.
 template <class Rebuild, class SideDrops>
 oxg_status rebuild_slots(oxg_table *t, const Rebuild &rebuild, const SideDrops &side_drops, uint64_t *removed) {
-    ulonglong2 *fresh = nullptr;
-    TRY(alloc_slots(t, t->cap, &fresh));
-    ulonglong2 *old = t->slots;
-    t->slots = fresh;
-    rebuild(old);
+    DeviceArray<ulonglong2> old;
+    TRY(alloc_slots(t, t->slots.cap(), &old));
+    std::swap(t->slots, old);
+    rebuild(old.get());
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(t));
-    TRY(free_slots(t, old));
-    Ctrl *h = t->h_ctrl;
+    old.reset();
+    Ctrl *h = t->h_ctrl.get();
     uint64_t n = h->scratch[0];
     h->size -= n;
     if (h->side_present && side_drops(h->side_count)) { h->side_present = 0; h->side_count = 0; ++n; }
     t->size = h->size;
-    CU(cudaMemcpyAsync(t->d_ctrl, h, offsetof(Ctrl, counted), cudaMemcpyHostToDevice, t->ctx->stream));
+    CU(cudaMemcpyAsync(t->d_ctrl.get(), h, offsetof(Ctrl, counted), cudaMemcpyHostToDevice, t->ctx->stream));
     CU(cudaStreamSynchronize(t->ctx->stream));
     if (removed) *removed = n;
     return OXG_OK;
@@ -540,29 +482,28 @@ oxg_status rebuild_slots(oxg_table *t, const Rebuild &rebuild, const SideDrops &
 oxg_status drain_deferred(oxg_table *t, DeferLists &d, uint64_t ov) {
     NvtxRange range("oxg:replay deferred");
     DeviceCtx *c = t->ctx;
-    if (ov > d.cap) return fail(OXG_ERR_CUDA, "internal: overflow list overrun");
+    if (ov > d.pairs.cap()) return fail(OXG_ERR_CUDA, "internal: overflow list overrun");
     uint64_t prev = ~0ULL;
     while (ov) {
         const uint64_t room = std::min<uint64_t>(ov, std::max<uint64_t>(t->size, 1ull << 20));
-        const uint64_t cap_before = t->cap;
+        const uint64_t cap_before = t->slots.cap();
         TRY(grow_to_fit(t, t->size + room));
-        const bool last = t->cap == cap_before && ov >= prev;
+        const bool last = t->slots.cap() == cap_before && ov >= prev;
         if (last) TRY(grow_to_fit(t, t->size + ov));
         prev = ov;
         if (!last) {
-            if (!d.fixed) TRY(ensure_dev(&d.d_pairs2, &d.cap2, ov));
-            else if (d.cap2 < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
+            if (!d.fixed) CU(d.pairs2.reserve(ov, kScratchMin));
+            else if (d.pairs2.cap() < ov) return fail(OXG_ERR_NOMEM, "deferral list too small for the replay");
         }
         TRY(zero_ctrl_fields(t, offsetof(Ctrl, overflow) / 8, 1));
         TableView v = view_of(t);
-        if (!last) { v.overflow = d.d_pairs2; v.overflow_cap = d.cap2; }
-        replay_pairs_kernel<<<grid_for(c, (ov + 3) / 4, kOpThreads, 8), kOpThreads, 0, c->stream>>>(v, d.d_pairs, ov);
+        if (!last) { v.overflow = d.pairs2.get(); v.overflow_cap = d.pairs2.cap(); }
+        replay_pairs_kernel<<<grid_for(c, (ov + 3) / 4, kOpThreads, 8), kOpThreads, 0, c->stream>>>(v, d.pairs.get(), ov);
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
-        ov = t->h_ctrl->overflow;
-        std::swap(d.d_pairs, d.d_pairs2);
-        std::swap(d.cap, d.cap2);
+        ov = t->h_ctrl.get()->overflow;
+        std::swap(d.pairs, d.pairs2);
     }
     return OXG_OK;
 }
@@ -578,9 +519,9 @@ oxg_status end_counting(oxg_table *t, uint64_t launches, uint64_t *counted, Coun
     TRY(pull_ctrl(t));
     CU(cudaEventElapsedTime(&out->ms, c->ev_t0, c->ev_t1));
     t->last_ms += out->ms; t->last_launches += launches;
-    if (counted) *counted += t->h_ctrl->counted;
+    if (counted) *counted += t->h_ctrl.get()->counted;
     out->made = t->size - size_before;
-    out->ov = t->h_ctrl->overflow;
+    out->ov = t->h_ctrl.get()->overflow;
     return OXG_OK;
 }
 
@@ -733,10 +674,10 @@ oxg_status plan_partitioned(oxg_table *t, uint64_t span, uint64_t n_tiles, int n
 oxg_status scatter_attr(DeviceCtx *c, uint32_t k) { return max_dyn_smem(specialised_entry(k, kModePart), c->dev, 227 * 1024); }
 
 oxg_status ensure_part_buffers(DeviceCtx *c, const PartPlan &pl) {
-    TRY(ensure_dev(&c->d_frag, &c->frag_cap, pl.frag_entries()));
-    TRY(ensure_dev(&c->d_frag_cnt, &c->frag_cnt_cap, (uint64_t)pl.n_dest() * pl.grid_a));
-    TRY(ensure_dev(&c->d_spill, &c->spill_cap, pl.spill_cap));
-    if (!c->d_spill_n) CU(cudaMalloc(&c->d_spill_n, 8));
+    CU(c->d_frag.reserve(pl.frag_entries(), kScratchMin));
+    CU(c->d_frag_cnt.reserve((uint64_t)pl.n_dest() * pl.grid_a, kScratchMin));
+    CU(c->d_spill.reserve(pl.spill_cap, kScratchMin));
+    CU(c->d_spill_n.reserve(1));
     return OXG_OK;
 }
 
@@ -810,7 +751,7 @@ oxg_status launch_part_b(oxg_table *t, const TableView &v, const PartPlan &pl, c
                          uint64_t windows, cudaStream_t stream) {
     DeviceCtx *c = t->ctx;
     AggParams a = agg_params(v, pl, src, n_src);
-    a.work_counter = (unsigned long long *)&t->d_ctrl->absorb_counter;
+    a.work_counter = (unsigned long long *)&t->d_ctrl.get()->absorb_counter;
     a.use_cache = use_cache_for(t, pl, windows);
     a.groups = aggregate_groups(pl, a.use_cache, windows);
     const void *fn = a.use_cache ? kAggCached : kAggDirect;
@@ -825,6 +766,15 @@ oxg_status launch_part_b(oxg_table *t, const TableView &v, const PartPlan &pl, c
     CU(cudaLaunchKernel(fn, dim3(grid), dim3(threads), args, smem, stream));
     LAUNCHED();
     CU(cudaGetLastError());
+    return OXG_OK;
+}
+
+// the table's sketch, zeroed on stream st when it is new
+oxg_status ensure_sketch(oxg_table *t, cudaStream_t st) {
+    if (t->h_sketch.get()) return OXG_OK;  // (allocated last)
+    CU(t->d_sketch.reserve(kSketchRegs));
+    CU(cudaMemsetAsync(t->d_sketch.get(), 0, kSketchRegs * 4, st));
+    CU(t->h_sketch.reserve(kSketchRegs));
     return OXG_OK;
 }
 
@@ -845,18 +795,14 @@ double sketch_estimate(const uint32_t *regs) {
 oxg_status presize_for_group(oxg_table *t, const PartPlan &pl, const AggSource *src, int n_src, cudaStream_t stream,
                              uint64_t arrivals = 0, uint64_t rounds_left = 1) {
     DeviceCtx *c = t->ctx;
-    if (!t->d_sketch) {
-        CU(cudaMalloc(&t->d_sketch, kSketchRegs * 4));
-        CU(cudaMallocHost(&t->h_sketch, kSketchRegs * 4));
-        CU(cudaMemsetAsync(t->d_sketch, 0, kSketchRegs * 4, stream));
-    }
-    sketch_kernel<<<c->sms * 2, 512, 0, stream>>>(agg_params(TableView{}, pl, src, n_src), t->d_sketch);
+    TRY(ensure_sketch(t, stream));
+    sketch_kernel<<<c->sms * 2, 512, 0, stream>>>(agg_params(TableView{}, pl, src, n_src), t->d_sketch.get());
     LAUNCHED();
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(t->h_sketch, t->d_sketch, kSketchRegs * 4, cudaMemcpyDeviceToHost, stream));
+    CU(cudaMemcpyAsync(t->h_sketch.get(), t->d_sketch.get(), kSketchRegs * 4, cudaMemcpyDeviceToHost, stream));
     CU(cudaStreamSynchronize(stream));
     const uint64_t unseen = t->size > t->sketch_covers ? t->size - t->sketch_covers : 0;  // keys that came in another way
-    const double est = sketch_estimate(t->h_sketch);
+    const double est = sketch_estimate(t->h_sketch.get());
     t->est_keys = (uint64_t)est + unseen;
     // sharded tables call this in the first round only, with more rounds of the same size to come:
     // where nearly everything that arrives is new (a quarter or more), room for half that rate over
@@ -873,7 +819,7 @@ oxg_status presize_for_group(oxg_table *t, const PartPlan &pl, const AggSource *
             expect = (uint64_t)(est * 1.04 * std::max(headroom, 4.0)) + unseen + 1024;
         }
     }
-    if (expect * 10 > t->cap * 7) TRY(grow_to_fit(t, expect));
+    if (expect * 10 > t->slots.cap() * 7) TRY(grow_to_fit(t, expect));
     return OXG_OK;
 }
 
@@ -884,12 +830,12 @@ oxg_status flush_pending(oxg_table *t, uint64_t *counted) {
     DeviceCtx *c = t->ctx;
     t->pend.active = false;
     CU(cudaEventRecord(c->ev_mid, c->stream));
-    const AggSource own{c->d_frag, c->d_frag_cnt, c->d_spill, c->d_spill_n};
+    const AggSource own{c->d_frag.get(), c->d_frag_cnt.get(), c->d_spill.get(), c->d_spill_n.get()};
     // The sketch costs a pass over the group's hashes (0.8 ms per 209 M): taken when the table's
     // size is anybody's guess -- no hint (or the hint is used up), and either nothing is known yet
     // or the room left would not take twice what the previous group created.
     const bool hint_holds = t->hinted && t->size <= t->hint_keys;
-    const bool roomy = t->size != 0 && (t->size + 2 * t->last_made) * 10 <= t->cap * 7;
+    const bool roomy = t->size != 0 && (t->size + 2 * t->last_made) * 10 <= t->slots.cap() * 7;
     const bool sketched = !hint_holds && !roomy;
     if (sketched) TRY(presize_for_group(t, t->pend.pl, &own, 1, c->stream));
     TRY(launch_part_b(t, view_of(t, &c->defer), t->pend.pl, &own, 1, t->pend.windows, c->stream));
@@ -909,11 +855,11 @@ oxg_status flush_pending(oxg_table *t, uint64_t *counted) {
         // the call will bring them at no more than this rate: make the room now, in one step,
         // rather than by doubling under load.  0.6: the rate of a read set falls as coverage builds
         // up (C3-shaped input: 0.39 new keys per window in the first group, 0.22 over the whole set).
-        if (made * 4 >= t->pend.windows && t->part_budget && t->size * 20 >= t->cap * 7) {  // (only a table that is filling up)
+        if (made * 4 >= t->pend.windows && t->part_budget && t->size * 20 >= t->slots.cap() * 7) {  // (only a table that is filling up)
             const uint64_t more = (uint64_t)((double)made / (double)t->pend.windows * 0.6 * (double)t->part_budget);
             const uint64_t want = t->size + more;
             bool grow = false;
-            TRY(larger_and_fits(want, t->cap, &grow));
+            TRY(larger_and_fits(want, t->slots.cap(), &grow));
             if (grow) TRY(grow_to_fit(t, want));
         }
     }
@@ -937,7 +883,7 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
         uint64_t hi = std::min<uint64_t>(w_hi, tile_base + kLaunchWindows);
         const uint32_t tw = tile_width(t->k);
         const uint64_t n_tiles = (hi - tile_base + tw - 1) / tw;
-        TRY(ensure_dev(&c->d_tile_first, &c->tile_first_cap, n_tiles));
+        CU(c->d_tile_first.reserve(n_tiles, kScratchMin));
         if (mode == kModeCount) {
             const uint64_t span = hi - lo;
             // a launch that will not join the group of pass A launches in flight (too small for the
@@ -949,12 +895,12 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
                 // sized gets at least one slot per 8 windows of a full launch (128 MiB for 64 Mi
                 // windows: enough for high-coverage data, cheap if it is not), and if the
                 // previous launch created keys at a rate that would cross the limit, grow now.
-                if (!t->hinted && t->cap < pow2_at_least(span / 8)) TRY(grow_to_fit(t, span / 16));
+                if (!t->hinted && t->slots.cap() < pow2_at_least(span / 8)) TRY(grow_to_fit(t, span / 16));
                 const uint64_t expect = t->size + t->last_new + t->last_new / 4;
-                if (expect * 10 > t->cap * 7) TRY(grow_to_fit(t, expect));
-                else if (over_loaded(t->size, t->cap)) TRY(grow_to_fit(t, t->size));
+                if (expect * 10 > t->slots.cap() * 7) TRY(grow_to_fit(t, expect));
+                else if (over_loaded(t->size, t->slots.cap())) TRY(grow_to_fit(t, t->size));
             }
-            TRY(ensure_dev(&c->defer.d_pairs, &c->defer.cap, std::max<uint64_t>(span, t->pend.active ? t->pend.planned : 0)));
+            CU(c->defer.pairs.reserve(std::max<uint64_t>(span, t->pend.active ? t->pend.planned : 0), kScratchMin));
             // counted, overflow, absorbed, tile and absorb counters -- unless a group of pass A
             // launches is accumulating into them
             if (!t->pend.active) TRY(zero_ctrl_fields(t, kFieldCounted, kLaunchFields));
@@ -964,9 +910,9 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
         ConsumeParams p{};
         p.bases = d_bases; p.g0 = g0; p.w_lo = lo; p.w_hi = hi; p.data_end = data_end;
         p.tile_base = tile_base; p.n_tiles = n_tiles; p.offsets = d_offsets; p.n_off = n_off;
-        p.tile_first = c->d_tile_first; p.table = view_of(t, mode == kModeCount ? &c->defer : nullptr);
+        p.tile_first = c->d_tile_first.get(); p.table = view_of(t, mode == kModeCount ? &c->defer : nullptr);
         p.hashes_out = hashes_out ? hashes_out + (lo - w_lo) : nullptr; p.ksize = t->k;
-        tile_first_kernel<<<(unsigned)((n_tiles + 255) / 256), 256, 0, c->stream>>>(d_offsets, n_off, tile_base, n_tiles, tw, c->d_tile_first);
+        tile_first_kernel<<<(unsigned)((n_tiles + 255) / 256), 256, 0, c->stream>>>(d_offsets, n_off, tile_base, n_tiles, tw, c->d_tile_first.get());
         LAUNCHED();
         CU(cudaGetLastError());
         const bool part = mode == kModeCount && use_partitioned(t, hi - lo);
@@ -982,7 +928,7 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
                 t->pend.active = true; t->pend.launches = 0; t->pend.windows = 0; t->pend.planned = planned;
                 CU(cudaEventRecord(c->ev_t0, c->stream));
             }
-            TRY(launch_part_a(t, p, t->pend.pl, c->d_frag, c->d_frag_cnt, c->d_spill, c->d_spill_n, c->stream, t->pend.launches > 0));
+            TRY(launch_part_a(t, p, t->pend.pl, c->d_frag.get(), c->d_frag_cnt.get(), c->d_spill.get(), c->d_spill_n.get(), c->stream, t->pend.launches > 0));
             t->pend.launches += 1; t->pend.windows += span;
             t->part_budget = t->part_budget > span ? t->part_budget - span : 0;
             if (t->pend.launches >= group_launches(t) || t->pend.windows >= t->pend.planned) TRY(flush_pending(t, counted));
@@ -1001,7 +947,7 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
             // quarter of this one (high-coverage input finds its keys early and then stops
             // creating them; the whole-launch count would quadruple the table for nothing),
             // or everything it wanted when it ran into the limit
-            t->last_new = (hi - lo) <= kSmallBatch ? 0 : r.ov ? r.made + r.ov : 4 * t->h_ctrl->late_new;
+            t->last_new = (hi - lo) <= kSmallBatch ? 0 : r.ov ? r.made + r.ov : 4 * t->h_ctrl.get()->late_new;
             if (r.ov) TRY(drain_deferred(t, c->defer, r.ov));  // table hit its load limit: grow, then replay the deferred hashes
         }
         lo = hi;
@@ -1015,11 +961,11 @@ oxg_status run_span(oxg_table *t, int mode, const uint8_t *d_bases, uint64_t g0,
 // `span` (see consume_batch), and return the first bad window (~0: none).
 template <class Span>
 oxg_status first_bad_window(oxg_table *t, const Span &span, uint64_t n_win, uint64_t total, uint64_t *fb) {
-    t->h_ctrl->first_bad = ~0ULL;
-    CU(cudaMemcpyAsync(&t->d_ctrl->first_bad, &t->h_ctrl->first_bad, 8, cudaMemcpyHostToDevice, t->ctx->stream));
+    t->h_ctrl.get()->first_bad = ~0ULL;
+    CU(cudaMemcpyAsync(&t->d_ctrl.get()->first_bad, &t->h_ctrl.get()->first_bad, 8, cudaMemcpyHostToDevice, t->ctx->stream));
     TRY(span(kModeFirstBad, 0, n_win, total, nullptr));
     TRY(pull_ctrl(t));
-    *fb = t->h_ctrl->first_bad;
+    *fb = t->h_ctrl.get()->first_bad;
     return OXG_OK;
 }
 
@@ -1103,6 +1049,8 @@ int oxg_device_count(void) {
     return n;
 }
 uint64_t oxg_launch_count(void) { return g_launches.load(); }
+uint64_t oxg_live_allocations(void) { return g_owned_live.load(); }
+uint64_t oxg_fail_allocation_after(uint64_t n) { return g_owned_fail_in.exchange(n); }
 
 oxg_status oxg_table_create(int device, uint32_t ksize, uint64_t capacity_hint, oxg_table **out) {
     if (!out) return fail(OXG_ERR_INVALID, "out is null");
@@ -1114,14 +1062,13 @@ oxg_status oxg_table_create(int device, uint32_t ksize, uint64_t capacity_hint, 
     CU(cudaSetDevice(c->dev));
     auto t = std::make_unique<oxg_table>();
     t->ctx = c; t->k = ksize;
-    t->cap = capacity_for_keys(capacity_hint);
     t->hinted = capacity_hint != 0;
     t->hint_keys = capacity_hint;
-    CU(cudaMalloc(&t->d_ctrl, sizeof(Ctrl)));
-    CU(cudaMemsetAsync(t->d_ctrl, 0, sizeof(Ctrl), c->stream));
-    CU(cudaMallocHost(&t->h_ctrl, sizeof(Ctrl)));
-    memset(t->h_ctrl, 0, sizeof(Ctrl));
-    TRY(alloc_slots(t.get(), t->cap, &t->slots));
+    CU(t->d_ctrl.reserve(1));
+    CU(cudaMemsetAsync(t->d_ctrl.get(), 0, sizeof(Ctrl), c->stream));
+    CU(t->h_ctrl.reserve(1));
+    memset(t->h_ctrl.get(), 0, sizeof(Ctrl));
+    TRY(alloc_slots(t.get(), capacity_for_keys(capacity_hint), &t->slots));
     CU(cudaStreamSynchronize(c->stream));
     *out = t.release();
     return OXG_OK;
@@ -1132,11 +1079,6 @@ oxg_status oxg_table_destroy(oxg_table *t) {
     std::lock_guard<std::mutex> lk(t->ctx->mu);
     cudaSetDevice(t->ctx->dev);
     cudaStreamSynchronize(t->ctx->stream);
-    free_slots(t, t->slots);
-    cudaFree(t->d_ctrl);
-    cudaFreeHost(t->h_ctrl);
-    if (t->d_sketch) cudaFree(t->d_sketch);
-    if (t->h_sketch) cudaFreeHost(t->h_sketch);
     delete t;
     return OXG_OK;
 }
@@ -1149,11 +1091,11 @@ oxg_status oxg_table_destroy(oxg_table *t) {
 
 oxg_status oxg_table_clear(oxg_table *t) {
     ENTER(t);
-    init_slots_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(t->slots, t->cap);
+    init_slots_kernel<<<grid_for(c, t->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(t->slots.get(), t->slots.cap());
     LAUNCHED();
     CU(cudaGetLastError());
-    CU(cudaMemsetAsync(t->d_ctrl, 0, sizeof(Ctrl), c->stream));
-    if (t->d_sketch) CU(cudaMemsetAsync(t->d_sketch, 0, kSketchRegs * 4, c->stream));
+    CU(cudaMemsetAsync(t->d_ctrl.get(), 0, sizeof(Ctrl), c->stream));
+    if (t->d_sketch.get()) CU(cudaMemsetAsync(t->d_sketch.get(), 0, kSketchRegs * 4, c->stream));
     t->sketch_covers = 0;
     t->est_keys = 0;
     t->last_made = 0;
@@ -1175,7 +1117,7 @@ oxg_status oxg_table_ksize(const oxg_table *t, uint32_t *ksize) {
 
 oxg_status oxg_table_capacity(const oxg_table *t, uint64_t *slots) {
     if (!t || !slots) return fail(OXG_ERR_INVALID, "null argument");
-    *slots = t->cap;
+    *slots = t->slots.cap();
     return OXG_OK;
 }
 
@@ -1236,17 +1178,17 @@ oxg_status oxg_hash_windows(oxg_table *t, const uint8_t *seq, uint64_t len, uint
     // piecewise so the device-side output stays bounded; scratch lives in the device context
     // (hash_kmer / count / get call this once per k-mer)
     const uint64_t piece = 4ull << 20;
-    TRY(ensure_dev(&c->d_seq, &c->seq_cap, std::min(len, piece + k - 1) + 32));
+    CU(c->d_seq.reserve(std::min(len, piece + k - 1) + 32, kScratchMin));
     TRY(ensure_io(c, std::min(n_win, piece) + 2));
-    uint64_t *d_off = c->d_io + std::min(n_win, piece);
-    c->h_io[0] = 0; c->h_io[1] = len;
-    CU(cudaMemcpyAsync(d_off, c->h_io, 16, cudaMemcpyHostToDevice, c->stream));
+    uint64_t *d_off = c->d_io.get() + std::min(n_win, piece);
+    c->h_io.get()[0] = 0; c->h_io.get()[1] = len;
+    CU(cudaMemcpyAsync(d_off, c->h_io.get(), 16, cudaMemcpyHostToDevice, c->stream));
     for (uint64_t lo = 0; lo < n_win; lo += piece) {
         const uint64_t hi = std::min(n_win, lo + piece);
         const uint64_t bytes = hi - lo + k - 1;
-        CU(cudaMemcpyAsync(c->d_seq, seq + lo, bytes, cudaMemcpyHostToDevice, c->stream));
-        TRY(run_span(t, kModeHash, c->d_seq, lo, lo, hi, lo + bytes, d_off, 2, c->d_io, nullptr));
-        CU(cudaMemcpyAsync(hashes_out + lo, c->d_io, (hi - lo) * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(c->d_seq.get(), seq + lo, bytes, cudaMemcpyHostToDevice, c->stream));
+        TRY(run_span(t, kModeHash, c->d_seq.get(), lo, lo, hi, lo + bytes, d_off, 2, c->d_io.get(), nullptr));
+        CU(cudaMemcpyAsync(hashes_out + lo, c->d_io.get(), (hi - lo) * 8, cudaMemcpyDeviceToHost, c->stream));
         CU(cudaStreamSynchronize(c->stream));
     }
     return OXG_OK;
@@ -1308,8 +1250,8 @@ static oxg_status stream_span(oxg_table *t, int mode, const HostBatch &h, uint64
         const int b = (int)(ci % kStageBufs);
         const uint64_t lo = chunk_lo(ci);
         CU(cudaStreamWaitEvent(c->stream, ring.ev_ready[b], 0));
-        TRY(run_span(t, mode, ring.d_bases[b], lo, std::max(lo, w_lo), std::min(w_hi, lo + kChunkBytes), chunk_hi(ci),
-                     ring.d_offs[b], ring.n_off[b], nullptr, counted));
+        TRY(run_span(t, mode, ring.d_bases[b].get(), lo, std::max(lo, w_lo), std::min(w_hi, lo + kChunkBytes), chunk_hi(ci),
+                     ring.d_offs[b].get(), ring.n_off[b], nullptr, counted));
         CU(cudaEventRecord(ring.ev_free[b], c->stream));
         return OXG_OK;
     };
@@ -1350,7 +1292,7 @@ static oxg_status stream_span(oxg_table *t, int mode, const HostBatch &h, uint64
             TRY(run_chunk(ci));
             if (mode != kModeCount) {
                 TRY(pull_ctrl(t));
-                if (mode == kModeFirstBad && t->h_ctrl->first_bad != ~0ULL) break;
+                if (mode == kModeFirstBad && t->h_ctrl.get()->first_bad != ~0ULL) break;
             }
         }
         return OXG_OK;
@@ -1369,7 +1311,7 @@ static oxg_status stream_span(oxg_table *t, int mode, const HostBatch &h, uint64
             // refilled before this chunk's kernel has read it.  A pre-scan that has found its
             // bad window needs no later chunk.
             st = pull_ctrl(t);
-            found = st == OXG_OK && mode == kModeFirstBad && t->h_ctrl->first_bad != ~0ULL;
+            found = st == OXG_OK && mode == kModeFirstBad && t->h_ctrl.get()->first_bad != ~0ULL;
         }
         std::lock_guard<std::mutex> lk(mu);
         done = ci + 1;
@@ -1421,8 +1363,8 @@ static oxg_status count_list_device(oxg_table *t, const uint64_t *d_hashes, uint
         const bool optimistic = m > kSmallBatch;
         if (!optimistic) TRY(reserve_keys(t, m));
         else {
-            if (over_loaded(t->size, t->cap)) TRY(grow_to_fit(t, t->size));
-            TRY(ensure_dev(&c->defer.d_pairs, &c->defer.cap, m));
+            if (over_loaded(t->size, t->slots.cap())) TRY(grow_to_fit(t, t->size));
+            CU(c->defer.pairs.reserve(m, kScratchMin));
         }
         TRY(zero_ctrl_fields(t, kFieldCounted, kLaunchFields));
         CU(cudaEventRecord(c->ev_t0, c->stream));
@@ -1451,14 +1393,14 @@ oxg_status oxg_count_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, ui
     if (!hashes) return fail(OXG_ERR_INVALID, "null argument");
     TRY(reserve_keys(t, n));
     TRY(ensure_io(c, 2 * n));
-    memcpy(c->h_io, hashes, n * 8);
-    CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
-    count_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, new_counts ? c->d_io + n : nullptr, 0);
+    memcpy(c->h_io.get(), hashes, n * 8);
+    CU(cudaMemcpyAsync(c->d_io.get(), c->h_io.get(), n * 8, cudaMemcpyHostToDevice, c->stream));
+    count_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io.get(), n, new_counts ? c->d_io.get() + n : nullptr, 0);
     LAUNCHED();
     CU(cudaGetLastError());
-    if (new_counts) CU(cudaMemcpyAsync(c->h_io + n, c->d_io + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (new_counts) CU(cudaMemcpyAsync(c->h_io.get() + n, c->d_io.get() + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
     TRY(pull_ctrl(t));
-    if (new_counts) memcpy(new_counts, c->h_io + n, n * 8);
+    if (new_counts) memcpy(new_counts, c->h_io.get() + n, n * 8);
     return OXG_OK;
 }
 
@@ -1468,15 +1410,15 @@ oxg_status oxg_add_pairs(oxg_table *t, const uint64_t *keys, const uint64_t *val
     if (!keys || !vals) return fail(OXG_ERR_INVALID, "null argument");
     TRY(reserve_keys(t, n));
     TRY(ensure_io(c, 2 * n));
-    memcpy(c->h_io, keys, n * 8);
-    memcpy(c->h_io + n, vals, n * 8);
-    CU(cudaMemcpyAsync(c->d_io, c->h_io, 2 * n * 8, cudaMemcpyHostToDevice, c->stream));
-    add_pairs_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, c->d_io + n, n);
+    memcpy(c->h_io.get(), keys, n * 8);
+    memcpy(c->h_io.get() + n, vals, n * 8);
+    CU(cudaMemcpyAsync(c->d_io.get(), c->h_io.get(), 2 * n * 8, cudaMemcpyHostToDevice, c->stream));
+    add_pairs_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io.get(), c->d_io.get() + n, n);
     LAUNCHED();
     CU(cudaGetLastError());
     // the out-of-band key's side entry must exist even when its value is 0
     for (uint64_t i = 0; i < n; ++i)
-        if (keys[i] == kEmpty) { const uint64_t one = 1; CU(cudaMemcpyAsync(&t->d_ctrl->side_present, &one, 8, cudaMemcpyHostToDevice, c->stream)); break; }
+        if (keys[i] == kEmpty) { const uint64_t one = 1; CU(cudaMemcpyAsync(&t->d_ctrl.get()->side_present, &one, 8, cudaMemcpyHostToDevice, c->stream)); break; }
     return pull_ctrl(t);
 }
 
@@ -1485,14 +1427,14 @@ oxg_status oxg_get_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, uint
     if (n == 0) return OXG_OK;
     if (!hashes || !counts_out) return fail(OXG_ERR_INVALID, "null argument");
     TRY(ensure_io(c, 2 * n));
-    memcpy(c->h_io, hashes, n * 8);
-    CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
-    get_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, c->d_io + n);
+    memcpy(c->h_io.get(), hashes, n * 8);
+    CU(cudaMemcpyAsync(c->d_io.get(), c->h_io.get(), n * 8, cudaMemcpyHostToDevice, c->stream));
+    get_hashes_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io.get(), n, c->d_io.get() + n);
     LAUNCHED();
     CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(c->h_io + n, c->d_io + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(c->h_io.get() + n, c->d_io.get() + n, n * 8, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    memcpy(counts_out, c->h_io + n, n * 8);
+    memcpy(counts_out, c->h_io.get() + n, n * 8);
     return OXG_OK;
 }
 
@@ -1511,30 +1453,29 @@ oxg_status oxg_erase_hashes(oxg_table *t, const uint64_t *hashes, uint64_t n, ui
     if (n == 0) return OXG_OK;
     if (!hashes) return fail(OXG_ERR_INVALID, "null argument");
     TRY(ensure_io(c, n));
-    memcpy(c->h_io, hashes, n * 8);
-    CU(cudaMemcpyAsync(c->d_io, c->h_io, n * 8, cudaMemcpyHostToDevice, c->stream));
+    memcpy(c->h_io.get(), hashes, n * 8);
+    CU(cudaMemcpyAsync(c->d_io.get(), c->h_io.get(), n * 8, cudaMemcpyHostToDevice, c->stream));
     if (n < 256) {
         // the reference's usage: one key per call (drop / drop_hash, src/lib.rs:197-224)
-        erase_hashes_kernel<<<1, 32, 0, c->stream>>>(view_of(t), c->d_io, n);
+        erase_hashes_kernel<<<1, 32, 0, c->stream>>>(view_of(t), c->d_io.get(), n);
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
-        if (n_removed) *n_removed = t->h_ctrl->scratch[0];
+        if (n_removed) *n_removed = t->h_ctrl.get()->scratch[0];
         return OXG_OK;
     }
     // a list: mark in parallel, rebuild once
     TRY(pull_ctrl(t));
-    uint32_t *d_doomed = nullptr;
-    const uint64_t words = (t->cap + 31) / 32;
-    CU(cudaMalloc(&d_doomed, words * 4));
-    CU(cudaMemsetAsync(d_doomed, 0, words * 4, c->stream));
+    DeviceArray<uint32_t> doomed;
+    const uint64_t words = (t->slots.cap() + 31) / 32;
+    CU(doomed.reserve(words));
+    CU(cudaMemsetAsync(doomed.get(), 0, words * 4, c->stream));
     TRY(zero_ctrl_fields(t, kFieldScratch, 1));
-    erase_mark_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io, n, d_doomed);
+    erase_mark_kernel<<<grid_for(c, n, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(t), c->d_io.get(), n, doomed.get());
     LAUNCHED();
     TRY(rebuild_slots(t, [&](const ulonglong2 *old) {
-        erase_rebuild_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t), d_doomed);
+        erase_rebuild_kernel<<<grid_for(c, t->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->slots.cap(), view_of(t), doomed.get());
     }, [&](uint64_t) { return std::find(hashes, hashes + n, kEmpty) != hashes + n; }, n_removed));
-    CU(cudaFree(d_doomed));
     return OXG_OK;
 }
 
@@ -1544,7 +1485,7 @@ oxg_status oxg_cut(oxg_table *t, int mode, uint64_t thresh, uint64_t *n_removed)
     TRY(pull_ctrl(t));
     TRY(zero_ctrl_fields(t, kFieldScratch, 1));
     return rebuild_slots(t, [&](const ulonglong2 *old) {
-        cut_kernel<<<grid_for(c, t->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->cap, view_of(t), mode, thresh);
+        cut_kernel<<<grid_for(c, t->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(old, t->slots.cap(), view_of(t), mode, thresh);
     }, [&](uint64_t v) { return mode == 0 ? v < thresh : v > thresh; }, n_removed);
 }
 
@@ -1553,24 +1494,24 @@ oxg_status oxg_cut(oxg_table *t, int mode, uint64_t thresh, uint64_t *n_removed)
 static oxg_status run_stats(oxg_table *t, bool histo, oxg_stats *st, uint64_t *n_big) {
     DeviceCtx *c = t->ctx;
     if (histo) {
-        CU(cudaMemsetAsync(c->d_dense, 0, kHistDense * 8, c->stream));
-        if (!c->d_big) TRY(ensure_dev(&c->d_big, &c->big_cap, 1 << 16));
+        CU(cudaMemsetAsync(c->d_dense.get(), 0, kHistDense * 8, c->stream));
+        if (!c->d_big.get()) CU(c->d_big.reserve(1 << 16));
     }
     for (int attempt = 0; attempt < 2; ++attempt) {
         Ctrl init{};
         init.scratch[2] = ~0ULL;
-        memcpy(t->h_ctrl->scratch, init.scratch, sizeof init.scratch);
-        CU(cudaMemcpyAsync(t->d_ctrl->scratch, t->h_ctrl->scratch, sizeof init.scratch, cudaMemcpyHostToDevice, c->stream));
-        stats_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), histo ? c->d_dense : nullptr, c->d_big, c->big_cap);
+        memcpy(t->h_ctrl.get()->scratch, init.scratch, sizeof init.scratch);
+        CU(cudaMemcpyAsync(t->d_ctrl.get()->scratch, t->h_ctrl.get()->scratch, sizeof init.scratch, cudaMemcpyHostToDevice, c->stream));
+        stats_kernel<<<grid_for(c, t->slots.cap(), kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), histo ? c->d_dense.get() : nullptr, c->d_big.get(), c->d_big.cap());
         LAUNCHED();
         CU(cudaGetLastError());
         TRY(pull_ctrl(t));
-        if (!histo || t->h_ctrl->scratch[4] <= c->big_cap) break;
+        if (!histo || t->h_ctrl.get()->scratch[4] <= c->d_big.cap()) break;
         // more huge counts than the list holds: enlarge and redo
-        TRY(ensure_dev(&c->d_big, &c->big_cap, t->h_ctrl->scratch[4]));
-        CU(cudaMemsetAsync(c->d_dense, 0, kHistDense * 8, c->stream));
+        CU(c->d_big.reserve(t->h_ctrl.get()->scratch[4], kScratchMin));
+        CU(cudaMemsetAsync(c->d_dense.get(), 0, kHistDense * 8, c->stream));
     }
-    const Ctrl *h = t->h_ctrl;
+    const Ctrl *h = t->h_ctrl.get();
     st->len = h->scratch[0]; st->sum = h->scratch[1];
     st->min = h->scratch[0] ? h->scratch[2] : ~0ULL; st->max = h->scratch[3];
     if (h->side_present) {
@@ -1586,7 +1527,7 @@ oxg_status oxg_table_len(oxg_table *t, uint64_t *len) {
     ENTER(t);
     if (!len) return fail(OXG_ERR_INVALID, "null argument");
     TRY(pull_ctrl(t));
-    *len = t->h_ctrl->size + (t->h_ctrl->side_present ? 1 : 0);
+    *len = t->h_ctrl.get()->size + (t->h_ctrl.get()->side_present ? 1 : 0);
     return OXG_OK;
 }
 
@@ -1603,11 +1544,11 @@ oxg_status oxg_histo(oxg_table *t, uint64_t *freq, uint64_t *n, uint64_t cap, ui
     uint64_t n_big = 0;
     TRY(run_stats(t, true, &st, &n_big));
     std::vector<uint64_t> dense(kHistDense), big(n_big);
-    CU(cudaMemcpyAsync(dense.data(), c->d_dense, kHistDense * 8, cudaMemcpyDeviceToHost, c->stream));
-    if (n_big) CU(cudaMemcpyAsync(big.data(), c->d_big, n_big * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(dense.data(), c->d_dense.get(), kHistDense * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (n_big) CU(cudaMemcpyAsync(big.data(), c->d_big.get(), n_big * 8, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    if (t->h_ctrl->side_present) {
-        const uint64_t v = t->h_ctrl->side_count;
+    if (t->h_ctrl.get()->side_present) {
+        const uint64_t v = t->h_ctrl.get()->side_count;
         if (v < kHistDense) dense[v] += 1; else big.push_back(v);
     }
     std::sort(big.begin(), big.end());
@@ -1633,12 +1574,12 @@ oxg_status oxg_table_digest(oxg_table *t, int n_ranks, int rank, uint64_t out[5]
     if (n_ranks < 1 || (n_ranks & (n_ranks - 1)) || rank < 0 || rank >= n_ranks) return fail(OXG_ERR_INVALID, "bad rank / n_ranks");
     int lg = 0;
     while ((1 << lg) < n_ranks) ++lg;
-    CU(cudaMemsetAsync(t->d_ctrl->scratch, 0, 5 * 8, c->stream));
-    digest_kernel<<<grid_for(c, t->cap, kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), 64 - lg, (uint64_t)rank);
+    CU(cudaMemsetAsync(t->d_ctrl.get()->scratch, 0, 5 * 8, c->stream));
+    digest_kernel<<<grid_for(c, t->slots.cap(), kOpThreads, 8), kOpThreads, 0, c->stream>>>(view_of(t), 64 - lg, (uint64_t)rank);
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(t));
-    const Ctrl *h = t->h_ctrl;
+    const Ctrl *h = t->h_ctrl.get();
     for (int i = 0; i < 5; ++i) out[i] = h->scratch[i];
     if (h->side_present) {  // the out-of-band key 2^64-1 (owner: the last rank)
         out[0] += 1; out[1] += h->side_count; out[2] ^= kEmpty; out[3] += kEmpty * h->side_count;
@@ -1661,7 +1602,7 @@ struct ExportArrays {
     uint64_t *sort_hist = nullptr;
 };
 
-static uint64_t export_chunks(const oxg_table *t) { return (t->cap + kExportChunk - 1) / kExportChunk; }
+static uint64_t export_chunks(const oxg_table *t) { return (t->slots.cap() + kExportChunk - 1) / kExportChunk; }
 static uint64_t sort_tiles(uint64_t n) { return (n + kSortTile - 1) / kSortTile; }
 
 // ordered compaction of the live slots into a.k[0] / a.v[0] (room for out_cap pairs) on stream st
@@ -1669,7 +1610,7 @@ static uint64_t sort_tiles(uint64_t n) { return (n + kSortTile - 1) / kSortTile;
 // src/lib.rs:330-381,658)
 static oxg_status export_device(const oxg_table *t, cudaStream_t st, const ExportArrays &a, uint64_t out_cap, uint64_t *n_live) {
     const uint64_t n_chunks = export_chunks(t);
-    export_count_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots, t->cap, a.chunk_counts);
+    export_count_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots.get(), t->slots.cap(), a.chunk_counts);
     LAUNCHED();
     export_scan_kernel<<<1, 1024, 0, st>>>(a.chunk_counts, n_chunks, a.chunk_counts + n_chunks);
     LAUNCHED();
@@ -1678,7 +1619,7 @@ static oxg_status export_device(const oxg_table *t, cudaStream_t st, const Expor
     CU(cudaMemcpyAsync(&live, a.chunk_counts + n_chunks, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (live >= out_cap) return fail(OXG_ERR_INVALID, "internal: %llu live slots, room for %llu", (unsigned long long)live, (unsigned long long)out_cap);
-    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots, t->cap, a.chunk_counts, a.k[0], a.v[0], live);
+    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots.get(), t->slots.cap(), a.chunk_counts, a.k[0], a.v[0], live);
     LAUNCHED();
     CU(cudaGetLastError());
     *n_live = live;
@@ -1773,9 +1714,9 @@ oxg_status oxg_export(oxg_table *t, uint64_t *keys, uint64_t *vals, uint64_t cap
     if (!n_out) return fail(OXG_ERR_INVALID, "null argument");
     if (sort_mode < 0 || sort_mode > 2) return fail(OXG_ERR_INVALID, "sort_mode must be 0, 1 or 2");
     TRY(pull_ctrl(t));
-    const bool side = t->h_ctrl->side_present != 0;
-    const uint64_t side_count = t->h_ctrl->side_count;
-    const uint64_t live = t->h_ctrl->size, total = live + (side ? 1 : 0);
+    const bool side = t->h_ctrl.get()->side_present != 0;
+    const uint64_t side_count = t->h_ctrl.get()->side_count;
+    const uint64_t live = t->h_ctrl.get()->size, total = live + (side ? 1 : 0);
     *n_out = total;
     if (cap == 0 || total == 0) return OXG_OK;
     uint64_t max_count = 0;
@@ -1785,26 +1726,15 @@ oxg_status oxg_export(oxg_table *t, uint64_t *keys, uint64_t *vals, uint64_t cap
         max_count = st.max;
     }
     // the context's export arrays, grown as needed
-    TRY(ensure_dev(&c->d_exp_counts, &c->exp_counts_cap, export_chunks(t) + 1));
-    for (int i = 0; i < (sort_mode != 0 && total >= 2 ? 2 : 1); ++i) {
-        if (c->exp_cap[i] >= live + 1) continue;
-        if (c->d_exp_k[i]) { CU(cudaFree(c->d_exp_k[i])); CU(cudaFree(c->d_exp_v[i])); }
-        c->d_exp_k[i] = c->d_exp_v[i] = nullptr; c->exp_cap[i] = 0;
-        CU(cudaMalloc(&c->d_exp_k[i], (live + 1) * 8));
-        CU(cudaMalloc(&c->d_exp_v[i], (live + 1) * 8));
-        c->exp_cap[i] = live + 1;
-    }
-    if (sort_mode != 0 && total >= 2) TRY(ensure_dev(&c->d_sort_hist, &c->sort_hist_cap, 256 * sort_tiles(total)));
-    for (int b = 0; b < 2; ++b)
-        if (!c->h_bounce[b]) {
-            CU(cudaMallocHost(&c->h_bounce[b], kBounceBytes));
-            CU(cudaEventCreateWithFlags(&c->ev_bounce[b], cudaEventDisableTiming));
-        }
-    const ExportArrays a{{c->d_exp_k[0], c->d_exp_k[1]}, {c->d_exp_v[0], c->d_exp_v[1]}, c->d_exp_counts, c->d_sort_hist};
+    CU(c->d_exp_counts.reserve(export_chunks(t) + 1, kScratchMin));
+    for (int i = 0; i < (sort_mode != 0 && total >= 2 ? 2 : 1); ++i) { CU(c->d_exp_k[i].reserve(live + 1)); CU(c->d_exp_v[i].reserve(live + 1)); }
+    if (sort_mode != 0 && total >= 2) CU(c->d_sort_hist.reserve(256 * sort_tiles(total), kScratchMin));
+    for (int b = 0; b < 2; ++b) { CU(c->h_bounce[b].reserve(kBounceBytes)); if (!c->ev_bounce[b]) CU(c->ev_bounce[b].create(cudaEventDisableTiming)); }
+    const ExportArrays a{{c->d_exp_k[0].get(), c->d_exp_k[1].get()}, {c->d_exp_v[0].get(), c->d_exp_v[1].get()}, c->d_exp_counts.get(), c->d_sort_hist.get()};
     uint64_t n = 0;
     int which = 0;
-    TRY(export_pairs_device(t, c->stream, a, c->exp_cap[0], side, side_count, sort_mode, max_count, &n, &which));
-    const Bounce b{{c->h_bounce[0], c->h_bounce[1]}, {c->ev_bounce[0], c->ev_bounce[1]}, kBounceBytes};
+    TRY(export_pairs_device(t, c->stream, a, std::min(c->d_exp_k[0].cap(), c->d_exp_v[0].cap()), side, side_count, sort_mode, max_count, &n, &which));
+    const Bounce b{{c->h_bounce[0].get(), c->h_bounce[1].get()}, {c->ev_bounce[0], c->ev_bounce[1]}, kBounceBytes};
     TRY(download(c->stream, b, keys, a.k[which], std::min(n, cap)));
     TRY(download(c->stream, b, vals, a.v[which], std::min(n, cap)));
     CU(cudaStreamSynchronize(c->stream));
@@ -1823,14 +1753,14 @@ static oxg_status setop_sizes_locked(oxg_table *a, oxg_table *b, uint64_t *inter
     DeviceCtx *c = a->ctx;
     TRY(pull_ctrl(b));
     TRY(zero_ctrl_fields(a, kFieldScratch, 1));
-    setop_count_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b));
+    setop_count_kernel<<<grid_for(c, a->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b));
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(a));
-    uint64_t both = a->h_ctrl->scratch[0];
-    if (a->h_ctrl->side_present && b->h_ctrl->side_present) both += 1;
-    const uint64_t na = a->h_ctrl->size + (a->h_ctrl->side_present ? 1 : 0);
-    const uint64_t nb = b->h_ctrl->size + (b->h_ctrl->side_present ? 1 : 0);
+    uint64_t both = a->h_ctrl.get()->scratch[0];
+    if (a->h_ctrl.get()->side_present && b->h_ctrl.get()->side_present) both += 1;
+    const uint64_t na = a->h_ctrl.get()->size + (a->h_ctrl.get()->side_present ? 1 : 0);
+    const uint64_t nb = b->h_ctrl.get()->size + (b->h_ctrl.get()->side_present ? 1 : 0);
     if (inter) *inter = both;
     if (uni) *uni = na + nb - both;
     return OXG_OK;
@@ -1859,13 +1789,13 @@ oxg_status oxg_setop_export(oxg_table *a, oxg_table *b, int op, uint64_t *keys_o
     if (op < 0 || op > 3) return fail(OXG_ERR_INVALID, "unknown set operation %d", op);
     TRY(pull_ctrl(a));
     TRY(pull_ctrl(b));
-    const uint64_t room = a->h_ctrl->size + b->h_ctrl->size + 2;
-    uint64_t *d_out = nullptr, *d_cnt = nullptr;
-    CU(cudaMalloc(&d_out, room * 8));
-    CU(cudaMalloc(&d_cnt, 8));
+    const uint64_t room = a->h_ctrl.get()->size + b->h_ctrl.get()->size + 2;
+    DeviceArray<uint64_t> out, cnt;
+    CU(out.reserve(room)); CU(cnt.reserve(1));
+    uint64_t *d_out = out.get(), *d_cnt = cnt.get();
     CU(cudaMemsetAsync(d_cnt, 0, 8, c->stream));
     auto pass = [&](oxg_table *x, oxg_table *y, int want) -> oxg_status {
-        setop_export_kernel<<<grid_for(c, x->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(x), view_of(y), want, d_out, room, d_cnt);
+        setop_export_kernel<<<grid_for(c, x->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(x), view_of(y), want, d_out, room, d_cnt);
         LAUNCHED();
         CU(cudaGetLastError());
         return OXG_OK;
@@ -1881,10 +1811,8 @@ oxg_status oxg_setop_export(oxg_table *a, oxg_table *b, int op, uint64_t *keys_o
     CU(cudaStreamSynchronize(c->stream));
     std::vector<uint64_t> host(n + 1);
     if (n) CU(cudaMemcpy(host.data(), d_out, n * 8, cudaMemcpyDeviceToHost));
-    CU(cudaFree(d_out));
-    CU(cudaFree(d_cnt));
     // the out-of-band key
-    const bool sa = a->h_ctrl->side_present, sb = b->h_ctrl->side_present;
+    const bool sa = a->h_ctrl.get()->side_present, sb = b->h_ctrl.get()->side_present;
     bool side = false;
     switch (op) {
     case OXG_UNION: side = sa || sb; break;
@@ -1904,27 +1832,27 @@ oxg_status oxg_cosine(oxg_table *a, oxg_table *b, double *out) {
     if (!out) return fail(OXG_ERR_INVALID, "null argument");
     TRY(pull_ctrl(a));
     TRY(pull_ctrl(b));
-    const uint64_t na = a->h_ctrl->size + (a->h_ctrl->side_present ? 1 : 0);
-    const uint64_t nb = b->h_ctrl->size + (b->h_ctrl->side_present ? 1 : 0);
+    const uint64_t na = a->h_ctrl.get()->size + (a->h_ctrl.get()->side_present ? 1 : 0);
+    const uint64_t nb = b->h_ctrl.get()->size + (b->h_ctrl.get()->side_present ? 1 : 0);
     if (na == 0 || nb == 0) { *out = 0.0; return OXG_OK; }  // src/lib.rs:729-731
-    CU(cudaMemsetAsync(c->d_f64, 0, 4 * sizeof(double), c->stream));
+    CU(cudaMemsetAsync(c->d_f64.get(), 0, 4 * sizeof(double), c->stream));
     TRY(zero_ctrl_fields(a, kFieldScratch, 1));
-    cosine_kernel<<<grid_for(c, a->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b), c->d_f64);
+    cosine_kernel<<<grid_for(c, a->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b), c->d_f64.get());
     LAUNCHED();
     TableView none = view_of(a);
     none.slots = nullptr;  // norm-only pass over b: adds nothing to any dot product
-    cosine_kernel<<<grid_for(c, b->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b), none, c->d_f64 + 1);
+    cosine_kernel<<<grid_for(c, b->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b), none, c->d_f64.get() + 1);
     LAUNCHED();
     CU(cudaGetLastError());
     double sq[2];
-    CU(cudaMemcpyAsync(sq, c->d_f64, 16, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(sq, c->d_f64.get(), 16, cudaMemcpyDeviceToHost, c->stream));
     TRY(pull_ctrl(a));
-    uint64_t dot = a->h_ctrl->scratch[0];
-    if (a->h_ctrl->side_present) {
-        sq[0] += (double)a->h_ctrl->side_count * (double)a->h_ctrl->side_count;
-        if (b->h_ctrl->side_present) dot += a->h_ctrl->side_count * b->h_ctrl->side_count;
+    uint64_t dot = a->h_ctrl.get()->scratch[0];
+    if (a->h_ctrl.get()->side_present) {
+        sq[0] += (double)a->h_ctrl.get()->side_count * (double)a->h_ctrl.get()->side_count;
+        if (b->h_ctrl.get()->side_present) dot += a->h_ctrl.get()->side_count * b->h_ctrl.get()->side_count;
     }
-    if (b->h_ctrl->side_present) sq[1] += (double)b->h_ctrl->side_count * (double)b->h_ctrl->side_count;
+    if (b->h_ctrl.get()->side_present) sq[1] += (double)b->h_ctrl.get()->side_count * (double)b->h_ctrl.get()->side_count;
     const double ma = sqrt(sq[0]), mb = sqrt(sq[1]);
     *out = (ma == 0.0 || mb == 0.0) ? 0.0 : (double)dot / (ma * mb);
     return OXG_OK;
@@ -1937,20 +1865,20 @@ oxg_status oxg_merge(oxg_table *dst, oxg_table *src, uint64_t *counts_added, uin
     ENTER(dst);
     TRY(pull_ctrl(dst));
     TRY(pull_ctrl(src));
-    TRY(reserve_keys(dst, src->h_ctrl->size));
+    TRY(reserve_keys(dst, src->h_ctrl.get()->size));
     TRY(zero_ctrl_fields(dst, kFieldScratch, 2));
-    merge_kernel<<<grid_for(c, src->cap, kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(dst), view_of(src));
+    merge_kernel<<<grid_for(c, src->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(dst), view_of(src));
     LAUNCHED();
     CU(cudaGetLastError());
     TRY(pull_ctrl(dst));
-    uint64_t added = dst->h_ctrl->scratch[0], fresh = dst->h_ctrl->scratch[1];
-    if (src->h_ctrl->side_present) {
-        Ctrl *h = dst->h_ctrl;
+    uint64_t added = dst->h_ctrl.get()->scratch[0], fresh = dst->h_ctrl.get()->scratch[1];
+    if (src->h_ctrl.get()->side_present) {
+        Ctrl *h = dst->h_ctrl.get();
         if (!h->side_present || h->side_count == 0) ++fresh;
         h->side_present = 1;
-        h->side_count += src->h_ctrl->side_count;
-        added += src->h_ctrl->side_count;
-        CU(cudaMemcpyAsync(&dst->d_ctrl->side_present, &h->side_present, 16, cudaMemcpyHostToDevice, c->stream));
+        h->side_count += src->h_ctrl.get()->side_count;
+        added += src->h_ctrl.get()->side_count;
+        CU(cudaMemcpyAsync(&dst->d_ctrl.get()->side_present, &h->side_present, 16, cudaMemcpyHostToDevice, c->stream));
         CU(cudaStreamSynchronize(c->stream));
     }
     if (counts_added) *counts_added = added;
