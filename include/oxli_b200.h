@@ -331,6 +331,30 @@ oxg_status oxg_shard_stats(oxg_shard *s, oxg_stats *out);
 oxg_status oxg_shard_histo(oxg_shard *s, uint64_t *freq, uint64_t *n, uint64_t cap, uint64_t *n_out);
 oxg_status oxg_shard_setop_sizes(oxg_shard *a, oxg_shard *b, uint64_t *inter, uint64_t *uni);
 oxg_status oxg_shard_jaccard(oxg_shard *a, oxg_shard *b, double *out);
+/* union / intersection / difference / symmetric_difference of two tables sharded the same way
+ * (src/lib.rs:610-655), COLLECTIVE: every rank passes the same op (an oxg_setop).  A key is a
+ * member when it is present, held with count 0 too.  A key of A owned by rank r can only be in B's
+ * shard on rank r, so each rank computes its own part on its GPU and no key crosses between GPUs.
+ * keys receives min(*n_out, cap) of the keys of the result that this rank owns, in ascending key
+ * order (2^64-1, its owner's side entry, last on the last rank); *start_out (nullable) = the sum of
+ * *n_out over the ranks below this one, *total_out (nullable) = the size of the whole result, the
+ * same on every rank.  So the parts in rank order are the whole result sorted.  cap >= the lengths
+ * of both shard tables of this rank (oxg_table_len on oxg_shard_table, not collective) always
+ * suffices.  a == b is allowed.  Plain-table calls on either shard's table made before the call are
+ * seen.  Refused before any exchange (OXG_ERR_INVALID), both tables unchanged: a null or
+ * unconnected shard, a null n_out, keys == NULL with cap > 0, an op outside 0..3, a and b sharded
+ * differently or on different devices.  Any other failure on one rank (ranks that passed different
+ * ops: OXG_ERR_INVALID; a device reservation: OXG_ERR_NOMEM) reaches every rank in the call's
+ * exchange, and every rank returns the status of the first rank that failed. */
+oxg_status oxg_shard_setop_export(oxg_shard *a, oxg_shard *b, int op, uint64_t *keys, uint64_t cap, uint64_t *n_out,
+                                  uint64_t *start_out, uint64_t *total_out);
+/* cosine similarity of the count vectors of two tables sharded the same way (src/lib.rs:727-765),
+ * COLLECTIVE: each rank computes the terms of its shards (dot product as wrapping u64, the sums of
+ * squares as doubles, side entries included), one exchange carries them, and every rank sums them
+ * in rank order: *out is the same double on every rank.  0.0 when the whole of A or of B is empty
+ * or a norm is 0.  Refused before any exchange (OXG_ERR_INVALID) as oxg_shard_setop_export, and
+ * for a null out. */
+oxg_status oxg_shard_cosine(oxg_shard *a, oxg_shard *b, double *out);
 /* order-independent digests of the whole table: out = {len, sum c, xor h,
  * sum h*c mod 2^64, keys found on a rank that does not own them (must be 0)} */
 oxg_status oxg_shard_digest(oxg_shard *s, uint64_t out[5]);

@@ -96,6 +96,8 @@ SIGNATURES = {
     "oxg_shard_histo": (C.c_int, [vp, vp, vp, u64, u64p]),
     "oxg_shard_setop_sizes": (C.c_int, [vp, vp, u64p, u64p]),
     "oxg_shard_jaccard": (C.c_int, [vp, vp, C.POINTER(C.c_double)]),
+    "oxg_shard_setop_export": (C.c_int, [vp, vp, C.c_int, vp, u64, u64p, u64p, u64p]),
+    "oxg_shard_cosine": (C.c_int, [vp, vp, C.POINTER(C.c_double)]),
     "oxg_shard_digest": (C.c_int, [vp, vp]),
     "oxg_shard_allgather": (C.c_int, [vp, vp, C.c_uint32, vp]),
     "oxg_table_digest": (C.c_int, [vp, C.c_int, C.c_int, vp]),
@@ -524,6 +526,21 @@ class Shard:
     def jaccard(self, other: "Shard") -> float:
         d = C.c_double()
         check(lib.oxg_shard_jaccard(self._h, other._h, C.byref(d)))
+        return float(d.value)
+
+    def setop(self, other: "Shard", op: int) -> tuple[np.ndarray, int, int]:
+        """This rank's part of union (0), intersection (1), difference (2) or symmetric difference (3)
+        with the other sharded table, in key order (collective): returns (keys, start, total), start
+        the position of keys in the whole sorted result and total its size."""
+        cap = len(self.table) + len(other.table)  # (plain calls, not collective)
+        out = np.zeros(max(cap, 1), dtype=np.uint64)
+        n, start, total = u64(), u64(), u64()
+        check(lib.oxg_shard_setop_export(self._h, other._h, op, _ptr(out), cap, C.byref(n), C.byref(start), C.byref(total)))
+        return out[: n.value], int(start.value), int(total.value)
+
+    def cosine(self, other: "Shard") -> float:
+        d = C.c_double()
+        check(lib.oxg_shard_cosine(self._h, other._h, C.byref(d)))
         return float(d.value)
 
     def digest(self) -> dict:

@@ -1619,7 +1619,7 @@ static oxg_status export_device(const oxg_table *t, cudaStream_t st, const Expor
     CU(cudaMemcpyAsync(&live, a.chunk_counts + n_chunks, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (live >= out_cap) return fail(OXG_ERR_INVALID, "internal: %llu live slots, room for %llu", (unsigned long long)live, (unsigned long long)out_cap);
-    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots.get(), t->slots.cap(), a.chunk_counts, a.k[0], a.v[0], live);
+    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(t->slots.get(), t->slots.cap(), a.chunk_counts, a.k[0], a.v[0], live, nullptr);
     LAUNCHED();
     CU(cudaGetLastError());
     *n_live = live;
@@ -1782,6 +1782,62 @@ oxg_status oxg_jaccard(oxg_table *a, oxg_table *b, double *out) {
     return OXG_OK;
 }
 
+// Where the keys of a set operation go on the device: the mask of a pass (one bit per slot of the
+// larger table), its chunk counts (export_chunks of the larger table + 1), the keys.
+struct SetopArrays {
+    uint16_t *mask = nullptr;
+    uint64_t *chunk_counts = nullptr;
+    uint64_t *keys = nullptr;
+};
+
+static uint64_t setop_chunks(const oxg_table *a, const oxg_table *b) { return std::max(export_chunks(a), export_chunks(b)); }
+
+// One compaction on stream st: the live slots of x -- all of them (y == nullptr, the export's count)
+// or those whose membership in y equals want_in_y -- in slot order at keys[*n ..), *n advanced.
+static oxg_status setop_pass(const oxg_table *x, const oxg_table *y, int want_in_y, cudaStream_t st, const SetopArrays &a,
+                             uint64_t out_cap, uint64_t *n) {
+    const uint64_t n_chunks = export_chunks(x);
+    if (y) setop_mask_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(view_of(x), view_of(y), want_in_y, a.mask, a.chunk_counts);
+    else export_count_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(x->slots.get(), x->slots.cap(), a.chunk_counts);
+    LAUNCHED();
+    export_scan_kernel<<<1, 1024, 0, st>>>(a.chunk_counts, n_chunks, a.chunk_counts + n_chunks);
+    LAUNCHED();
+    CU(cudaGetLastError());
+    uint64_t got = 0;
+    CU(cudaMemcpyAsync(&got, a.chunk_counts + n_chunks, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (*n + got > out_cap) return fail(OXG_ERR_INVALID, "internal: %llu set keys, room for %llu", (unsigned long long)(*n + got), (unsigned long long)out_cap);
+    export_write_kernel<<<(unsigned)n_chunks, kOpThreads, 0, st>>>(x->slots.get(), x->slots.cap(), a.chunk_counts, a.keys + *n, nullptr,
+                                                                   out_cap - *n, y ? a.mask : nullptr);
+    LAUNCHED();
+    CU(cudaGetLastError());
+    *n += got;
+    return OXG_OK;
+}
+
+// The slot keys of a op b (an oxg_setop) in a.keys, each pass's in slot order, on stream st: *n of
+// them.  2^64-1 lives outside the slot arrays: see setop_side.
+static oxg_status setop_keys_device(const oxg_table *a, const oxg_table *b, int op, cudaStream_t st, const SetopArrays &arr,
+                                    uint64_t out_cap, uint64_t *n) {
+    *n = 0;
+    switch (op) {
+    case OXG_UNION: TRY(setop_pass(a, nullptr, 0, st, arr, out_cap, n)); return setop_pass(b, a, 0, st, arr, out_cap, n);
+    case OXG_INTERSECTION: return setop_pass(a, b, 1, st, arr, out_cap, n);
+    case OXG_DIFFERENCE: return setop_pass(a, b, 0, st, arr, out_cap, n);
+    default: TRY(setop_pass(a, b, 0, st, arr, out_cap, n)); return setop_pass(b, a, 0, st, arr, out_cap, n);
+    }
+}
+
+// whether the out-of-band key 2^64-1 is in a op b, given whether each table holds it
+static bool setop_side(int op, bool sa, bool sb) {
+    switch (op) {
+    case OXG_UNION: return sa || sb;
+    case OXG_INTERSECTION: return sa && sb;
+    case OXG_DIFFERENCE: return sa && !sb;
+    default: return sa != sb;
+    }
+}
+
 oxg_status oxg_setop_export(oxg_table *a, oxg_table *b, int op, uint64_t *keys_out, uint64_t cap, uint64_t *n_out) {
     TRY(two_tables(a, b));
     ENTER(a);
@@ -1789,72 +1845,79 @@ oxg_status oxg_setop_export(oxg_table *a, oxg_table *b, int op, uint64_t *keys_o
     if (op < 0 || op > 3) return fail(OXG_ERR_INVALID, "unknown set operation %d", op);
     TRY(pull_ctrl(a));
     TRY(pull_ctrl(b));
-    const uint64_t room = a->h_ctrl.get()->size + b->h_ctrl.get()->size + 2;
-    DeviceArray<uint64_t> out, cnt;
-    CU(out.reserve(room)); CU(cnt.reserve(1));
-    uint64_t *d_out = out.get(), *d_cnt = cnt.get();
-    CU(cudaMemsetAsync(d_cnt, 0, 8, c->stream));
-    auto pass = [&](oxg_table *x, oxg_table *y, int want) -> oxg_status {
-        setop_export_kernel<<<grid_for(c, x->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(x), view_of(y), want, d_out, room, d_cnt);
+    const uint64_t room = a->h_ctrl.get()->size + b->h_ctrl.get()->size;
+    const uint64_t n_chunks = setop_chunks(a, b);
+    DeviceArray<uint16_t> mask;
+    DeviceArray<uint64_t> counts, out;
+    CU(mask.reserve(n_chunks * kOpThreads));
+    CU(counts.reserve(n_chunks + 1));
+    CU(out.reserve(room, 1));
+    for (int i = 0; i < 2; ++i) { CU(c->h_bounce[i].reserve(kBounceBytes)); if (!c->ev_bounce[i]) CU(c->ev_bounce[i].create(cudaEventDisableTiming)); }
+    uint64_t n = 0;
+    TRY(setop_keys_device(a, b, op, c->stream, SetopArrays{mask.get(), counts.get(), out.get()}, room, &n));
+    const bool side = setop_side(op, a->h_ctrl.get()->side_present != 0, b->h_ctrl.get()->side_present != 0);
+    *n_out = n + (side ? 1 : 0);
+    const Bounce bb{{c->h_bounce[0].get(), c->h_bounce[1].get()}, {c->ev_bounce[0], c->ev_bounce[1]}, kBounceBytes};
+    TRY(download(c->stream, bb, keys_out, out.get(), std::min(n, cap)));
+    if (keys_out && side && n < cap) keys_out[n] = kEmpty;  // the out-of-band key comes last
+    return OXG_OK;
+}
+
+// The raw terms of cosine(a, b) (src/lib.rs:727-765), side entries included: the dot product over
+// A & B (wrapping u64), sum a^2 and sum b^2 as doubles, |A| and |B|.  Locks a's context.
+struct CosineTerms {
+    uint64_t dot = 0;
+    double sq_a = 0.0, sq_b = 0.0;
+    uint64_t n_a = 0, n_b = 0;
+};
+
+static oxg_status cosine_terms(oxg_table *a, oxg_table *b, CosineTerms *out) {
+    ENTER(a);
+    TRY(pull_ctrl(a));
+    TRY(pull_ctrl(b));
+    const Ctrl ha = *a->h_ctrl.get(), hb = *b->h_ctrl.get();
+    CosineTerms t;
+    t.n_a = ha.size + (ha.side_present ? 1 : 0);
+    t.n_b = hb.size + (hb.side_present ? 1 : 0);
+    double sq[2] = {0.0, 0.0};
+    if (ha.size || hb.size) {
+        CU(cudaMemsetAsync(c->d_f64.get(), 0, 4 * sizeof(double), c->stream));
+        TRY(zero_ctrl_fields(a, kFieldScratch, 1));
+        cosine_kernel<<<grid_for(c, a->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b), c->d_f64.get());
+        LAUNCHED();
+        TableView none = view_of(a);
+        none.slots = nullptr;  // norm-only pass over b: adds nothing to any dot product
+        cosine_kernel<<<grid_for(c, b->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b), none, c->d_f64.get() + 1);
         LAUNCHED();
         CU(cudaGetLastError());
-        return OXG_OK;
-    };
-    switch (op) {
-    case OXG_UNION: TRY(pass(a, b, 2)); TRY(pass(b, a, 0)); break;
-    case OXG_INTERSECTION: TRY(pass(a, b, 1)); break;
-    case OXG_DIFFERENCE: TRY(pass(a, b, 0)); break;
-    default: TRY(pass(a, b, 0)); TRY(pass(b, a, 0)); break;
+        CU(cudaMemcpyAsync(sq, c->d_f64.get(), 16, cudaMemcpyDeviceToHost, c->stream));
+        TRY(pull_ctrl(a));
+        t.dot = a->h_ctrl.get()->scratch[0];
     }
-    uint64_t n = 0;
-    CU(cudaMemcpyAsync(&n, d_cnt, 8, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    std::vector<uint64_t> host(n + 1);
-    if (n) CU(cudaMemcpy(host.data(), d_out, n * 8, cudaMemcpyDeviceToHost));
-    // the out-of-band key
-    const bool sa = a->h_ctrl.get()->side_present, sb = b->h_ctrl.get()->side_present;
-    bool side = false;
-    switch (op) {
-    case OXG_UNION: side = sa || sb; break;
-    case OXG_INTERSECTION: side = sa && sb; break;
-    case OXG_DIFFERENCE: side = sa && !sb; break;
-    default: side = sa != sb; break;
+    if (ha.side_present) {
+        sq[0] += (double)ha.side_count * (double)ha.side_count;
+        if (hb.side_present) t.dot += ha.side_count * hb.side_count;
     }
-    if (side) host[n++] = kEmpty;
-    *n_out = n;
-    if (keys_out) memcpy(keys_out, host.data(), std::min(n, cap) * 8);
+    if (hb.side_present) sq[1] += (double)hb.side_count * (double)hb.side_count;
+    t.sq_a = sq[0];
+    t.sq_b = sq[1];
+    *out = t;
     return OXG_OK;
+}
+
+// cosine from its terms: 0.0 when either table is empty (src/lib.rs:729-731) or a norm is 0
+static double cosine_of(const CosineTerms &t) {
+    if (t.n_a == 0 || t.n_b == 0) return 0.0;
+    const double ma = sqrt(t.sq_a), mb = sqrt(t.sq_b);
+    return (ma == 0.0 || mb == 0.0) ? 0.0 : (double)t.dot / (ma * mb);
 }
 
 oxg_status oxg_cosine(oxg_table *a, oxg_table *b, double *out) {
     TRY(two_tables(a, b));
-    ENTER(a);
     if (!out) return fail(OXG_ERR_INVALID, "null argument");
-    TRY(pull_ctrl(a));
-    TRY(pull_ctrl(b));
-    const uint64_t na = a->h_ctrl.get()->size + (a->h_ctrl.get()->side_present ? 1 : 0);
-    const uint64_t nb = b->h_ctrl.get()->size + (b->h_ctrl.get()->side_present ? 1 : 0);
-    if (na == 0 || nb == 0) { *out = 0.0; return OXG_OK; }  // src/lib.rs:729-731
-    CU(cudaMemsetAsync(c->d_f64.get(), 0, 4 * sizeof(double), c->stream));
-    TRY(zero_ctrl_fields(a, kFieldScratch, 1));
-    cosine_kernel<<<grid_for(c, a->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(a), view_of(b), c->d_f64.get());
-    LAUNCHED();
-    TableView none = view_of(a);
-    none.slots = nullptr;  // norm-only pass over b: adds nothing to any dot product
-    cosine_kernel<<<grid_for(c, b->slots.cap(), kOpThreads, 16), kOpThreads, 0, c->stream>>>(view_of(b), none, c->d_f64.get() + 1);
-    LAUNCHED();
-    CU(cudaGetLastError());
-    double sq[2];
-    CU(cudaMemcpyAsync(sq, c->d_f64.get(), 16, cudaMemcpyDeviceToHost, c->stream));
-    TRY(pull_ctrl(a));
-    uint64_t dot = a->h_ctrl.get()->scratch[0];
-    if (a->h_ctrl.get()->side_present) {
-        sq[0] += (double)a->h_ctrl.get()->side_count * (double)a->h_ctrl.get()->side_count;
-        if (b->h_ctrl.get()->side_present) dot += a->h_ctrl.get()->side_count * b->h_ctrl.get()->side_count;
-    }
-    if (b->h_ctrl.get()->side_present) sq[1] += (double)b->h_ctrl.get()->side_count * (double)b->h_ctrl.get()->side_count;
-    const double ma = sqrt(sq[0]), mb = sqrt(sq[1]);
-    *out = (ma == 0.0 || mb == 0.0) ? 0.0 : (double)dot / (ma * mb);
+    CosineTerms t;
+    TRY(cosine_terms(a, b, &t));
+    *out = cosine_of(t);
     return OXG_OK;
 }
 

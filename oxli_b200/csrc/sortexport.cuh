@@ -23,6 +23,9 @@ constexpr int kSortThreads = 256;
 constexpr int kSortRounds = 16;
 constexpr int kSortTile = kSortThreads * kSortRounds;  // 4096 pairs per CTA
 
+// Key mode (by_count == 0) also sorts keys alone: vals (and vals_out) == nullptr, and no value is
+// loaded or stored.
+
 // sort digit of pair i: bits [shift, shift+8) of the hash (by_count == 0) or of the count
 __device__ __forceinline__ uint32_t sort_digit(const uint64_t *keys, const uint64_t *vals, uint64_t i, int shift, int by_count) {
     return (uint32_t)(((by_count ? vals[i] : keys[i]) >> shift) & 0xffu);
@@ -76,7 +79,7 @@ static __global__ void __launch_bounds__(kSortThreads) radix_scatter_kernel(cons
         __syncthreads();
         const uint64_t i = base + (uint64_t)r * kSortThreads + threadIdx.x;
         const bool valid = i < n;
-        const uint64_t k = valid ? keys[i] : 0, v = valid ? vals[i] : 0;
+        const uint64_t k = valid ? keys[i] : 0, v = valid && vals ? vals[i] : 0;
         const uint32_t d = valid ? (uint32_t)(((by_count ? v : k) >> shift) & 0xffu) : 0x100u + (uint32_t)lane;  // pairs past the end match nobody
         const unsigned peers = __match_any_sync(0xffffffffu, d);
         const uint32_t rank_in_warp = __popc(peers & ((1u << lane) - 1));
@@ -87,7 +90,7 @@ static __global__ void __launch_bounds__(kSortThreads) radix_scatter_kernel(cons
             for (int w = 0; w < warp; ++w) before += warp_cnt[w][d];
             const uint64_t at = run_base[d] + before + rank_in_warp;
             keys_out[at] = k;
-            vals_out[at] = v;
+            if (vals_out) vals_out[at] = v;
         }
         __syncthreads();
         uint32_t tot = 0;

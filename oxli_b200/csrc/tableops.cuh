@@ -331,19 +331,22 @@ __global__ void export_scan_kernel(uint64_t *__restrict__ chunk_counts, uint64_t
     for (uint64_t i = lo; i < hi; ++i) { uint64_t v = chunk_counts[i]; chunk_counts[i] = run; run += v; }
 }
 
-// pass 2: write (key,count) of live slots in slot order
+// pass 2: write (key,count) of live slots in slot order; with a mask (setop_mask_kernel), only the
+// slots whose bit is set
 __global__ void export_write_kernel(const ulonglong2 *__restrict__ slots, uint64_t cap,
                                     const uint64_t *__restrict__ chunk_offsets,
                                     uint64_t *__restrict__ keys, uint64_t *__restrict__ vals,
-                                    uint64_t out_cap) {
+                                    uint64_t out_cap, const uint16_t *__restrict__ mask) {
     constexpr int PER = kExportChunk / kOpThreads;  // consecutive slots per thread
     __shared__ uint32_t pre[kOpThreads];
     const uint64_t base = blockIdx.x * (uint64_t)kExportChunk + threadIdx.x * (uint64_t)PER;
+    const uint32_t keep = mask ? mask[blockIdx.x * (uint64_t)kOpThreads + threadIdx.x] : ~0u;
     ulonglong2 s[PER];
     uint32_t c = 0;
 #pragma unroll
     for (int i = 0; i < PER; ++i) {
         s[i] = base + i < cap ? slots[base + i] : make_ulonglong2(kEmpty, 0);
+        if (!((keep >> i) & 1u)) s[i].x = kEmpty;
         c += s[i].x != kEmpty;
     }
     pre[threadIdx.x] = c;
@@ -382,23 +385,38 @@ __global__ void setop_count_kernel(TableView a, TableView b) {
     if ((threadIdx.x & 31) == 0 && both) atomicAdd((unsigned long long *)&a.ctrl->scratch[0], (unsigned long long)both);
 }
 
-// keys of A whose membership in B equals want_in_b (2 = don't care); unordered append
-__global__ void setop_export_kernel(TableView a, TableView b, int want_in_b, uint64_t *__restrict__ out,
-                                    uint64_t out_cap, uint64_t *out_count) {
-    const uint64_t n = (a.cap + 31) / 32 * 32;  // keep warps whole for the ballots
-    for (uint64_t i = gtid(); i < n; i += gstride()) {
-        const uint64_t k = i < a.cap ? a.slots[i].x : kEmpty;
-        bool emit = k != kEmpty;
-        if (emit && want_in_b != 2) emit = (table_find(b, k) >= 0) == (want_in_b == 1);
-        const unsigned m = __ballot_sync(0xffffffffu, emit);
-        if (!m) continue;
-        const int lane = threadIdx.x & 31;
-        uint64_t base = 0;
-        if (lane == 0) base = atomicAdd((unsigned long long *)out_count, (unsigned long long)__popc(m));
-        base = __shfl_sync(0xffffffffu, base, 0);
-        const uint64_t at = base + __popc(m & ((1u << lane) - 1));
-        if (emit && at < out_cap) out[at] = k;
+// union / intersection / difference / symmetric_difference (src/lib.rs:610-655): the live slots of x
+// whose key's membership in y equals want_in_y, as one bit per slot of x -- the export's chunks, each
+// thread's kExportChunk / kOpThreads consecutive slots in one u16 -- and their number per chunk, for
+// export_scan_kernel and the masked export_write_kernel.  Four probes of y in flight per thread.
+__global__ void __launch_bounds__(kOpThreads) setop_mask_kernel(TableView x, TableView y, int want_in_y,
+                                                                uint16_t *__restrict__ mask, uint64_t *__restrict__ chunk_counts) {
+    constexpr int PER = kExportChunk / kOpThreads, U = 4;
+    static_assert(PER == 16, "one u16 of mask bits per thread");
+    __shared__ uint32_t total;
+    if (threadIdx.x == 0) total = 0;
+    __syncthreads();
+    const uint64_t base = blockIdx.x * (uint64_t)kExportChunk + threadIdx.x * (uint64_t)PER;
+    uint32_t bits = 0;
+#pragma unroll
+    for (int g = 0; g < PER; g += U) {
+        uint64_t key[U], cnt[U];
+        uint32_t live = 0;
+#pragma unroll
+        for (int j = 0; j < U; ++j) {
+            const uint64_t i = base + g + j;
+            key[j] = i < x.cap ? __ldcs(&x.slots[i].x) : kEmpty;
+            live |= (key[j] != kEmpty ? 1u : 0u) << j;
+        }
+        if (!live) continue;
+        const uint32_t found = table_get_many<U>(y, key, live, cnt);
+        bits |= (want_in_y ? found : ~found & live) << g;
     }
+    mask[blockIdx.x * (uint64_t)kOpThreads + threadIdx.x] = (uint16_t)bits;
+    const uint32_t c = (uint32_t)warp_sum(__popc(bits));
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(&total, c);
+    __syncthreads();
+    if (threadIdx.x == 0) chunk_counts[blockIdx.x] = total;
 }
 
 // cosine (src/lib.rs:727-765): scratch[0] = sum_{k in A&B} a_k*b_k (wrapping u64),

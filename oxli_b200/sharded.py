@@ -13,7 +13,9 @@ already on their owners.  Removal takes the same route: drop / drop_hash / drop_
 (src/lib.rs:197-224) send each hash to its owner, which erases it, and mincut / maxcut
 (src/lib.rs:227-267) cut every shard and sum what each removed.  export and dump (src/lib.rs:330-381)
 need no routing at all: every key of rank r is below every key of rank r + 1, so each rank sorts
-and formats its own shard and writes its part of one file.  All of that, including the
+and formats its own shard and writes its part of one file.  Neither do union, intersection,
+difference, symmetric_difference and cosine of two tables sharded the same way (src/lib.rs:610-655,
+727-765): a key of rank r can only meet keys of rank r, so each rank computes its own part.  All of that, including the
 rank-to-rank flags and the reductions (len / sum / min / max, histo, |A & B|, jaccard, digests:
 reference src/lib.rs:464-539, 610-638, 708-722), lives in the C library.
 
@@ -52,6 +54,23 @@ class BadKmerError(ValueError):
     def __init__(self, position: int, read: int):
         super().__init__(f"bad k-mer encountered at position {position}")
         self.position, self.read = position, read
+
+
+_ERR_INVALID, _ERR_NOMEM = 2, 4  # oxg_status (include/oxli_b200.h)
+
+
+def _engine_call(fn, *args):
+    """fn(*args), with the engine's refusals raised as ValueError and its failed device reservations
+    as MemoryError (the engine's error stays chained)"""
+    try:
+        return fn(*args)
+    except RuntimeError as e:
+        status = getattr(e, "status", None)
+        if status == _ERR_INVALID:
+            raise ValueError(str(e)) from e
+        if status == _ERR_NOMEM:
+            raise MemoryError(str(e)) from e
+        raise
 
 
 class ShardedTable:
@@ -190,6 +209,39 @@ class ShardedTable:
 
     def jaccard(self, other: "ShardedTable") -> float:
         return self.engine.jaccard(other.engine)
+
+    # -- set operations and cosine (collective) ------------------------------------------
+    def _setop(self, other: "ShardedTable", op: int) -> tuple[np.ndarray, int, int]:
+        if not isinstance(other, ShardedTable):
+            raise TypeError(f"expected a ShardedTable, got {type(other).__name__}")
+        return _engine_call(self.engine.setop, other.engine, op)
+
+    def union(self, other: "ShardedTable") -> tuple[np.ndarray, int, int]:
+        """union (src/lib.rs:610-655) with a table sharded the same way.  Returns (keys, start, total):
+        the keys of the result that this rank owns in ascending order, their position in the whole
+        sorted result and its size.  A key of A owned by rank r can only be in B's shard on rank r,
+        so each rank computes its part on its GPU and no key crosses between GPUs; the parts in rank
+        order are the whole result sorted.  A key held with count 0 is a member."""
+        return self._setop(other, 0)
+
+    def intersection(self, other: "ShardedTable") -> tuple[np.ndarray, int, int]:
+        """intersection (src/lib.rs:610-655); returns this rank's (keys, start, total) as union."""
+        return self._setop(other, 1)
+
+    def difference(self, other: "ShardedTable") -> tuple[np.ndarray, int, int]:
+        """difference (src/lib.rs:610-655); returns this rank's (keys, start, total) as union."""
+        return self._setop(other, 2)
+
+    def symmetric_difference(self, other: "ShardedTable") -> tuple[np.ndarray, int, int]:
+        """symmetric_difference (src/lib.rs:610-655); returns this rank's (keys, start, total) as union."""
+        return self._setop(other, 3)
+
+    def cosine(self, other: "ShardedTable") -> float:
+        """cosine similarity of the count vectors (src/lib.rs:727-765) with a table sharded the same
+        way: the same float on every rank; 0.0 when either whole table is empty or a norm is 0."""
+        if not isinstance(other, ShardedTable):
+            raise TypeError(f"expected a ShardedTable, got {type(other).__name__}")
+        return _engine_call(self.engine.cosine, other.engine)
 
     def digest(self) -> dict:
         """{n, sum, xor, sum_hc, foreign} of the whole table; foreign must be 0."""
