@@ -804,7 +804,7 @@ oxg_status presize_for_group(oxg_table *t, const PartPlan &pl, const AggSource *
     const uint64_t unseen = t->size > t->sketch_covers ? t->size - t->sketch_covers : 0;  // keys that came in another way
     const double est = sketch_estimate(t->h_sketch.get());
     t->est_keys = (uint64_t)est + unseen;
-    // sharded tables call this in the first round only, with more rounds of the same size to come:
+    // sharded tables call this with a sketch of one round (shard_round), with more rounds to come:
     // where nearly everything that arrives is new (a quarter or more), room for half that rate over
     // the whole batch, in one step (the rate falls as coverage builds up); else for the rounds in
     // flight before the host monitor catches up
