@@ -37,7 +37,8 @@ constexpr uint32_t kLocalSlots = 1u << kLocalBits;  // 16384 x (8-byte key + 4-b
 constexpr int kLocalProbe = 2;                      // buckets of four slots examined before bypassing
 constexpr uint32_t kSpillSlice = 1u << 16;          // spill-list entries per work item
 constexpr int kMaxSources = 16;
-constexpr uint32_t kAggMaxFrags = 296 * kMaxSources;  // fragments of one partition: pass A CTAs x sources
+constexpr uint32_t kAggMaxFrags = 296 * kMaxSources;  // fragments of one partition: pass A CTAs (up to two per
+                                                      // SM of a B200) x sources
 
 struct AggSource {
     const uint64_t *frag;                 // [n_dest_total][n_ctas][frag_cap]
@@ -150,12 +151,14 @@ __global__ void __launch_bounds__(kAggThreads, 1) aggregate_kernel(const AggPara
     extern __shared__ __align__(16) uint8_t agg_smem[];
     uint64_t *lk = reinterpret_cast<uint64_t *>(agg_smem);                    // keys
     uint32_t *ld = reinterpret_cast<uint32_t *>(agg_smem + kLocalSlots * 8);  // occurrences
-    uint32_t *s_cnt = kCache ? ld + kLocalSlots : reinterpret_cast<uint32_t *>(agg_smem);  // fill counts of the item's fragments
+    uint32_t *s_end = kCache ? ld + kLocalSlots : reinterpret_cast<uint32_t *>(agg_smem);  // the item's fragments, where their hashes end
     __shared__ unsigned long long s_item;
-    __shared__ uint32_t s_next;                          // next fragment (or spill run) of the item to hand out
+    __shared__ uint32_t s_next;                          // next run of blocks past the ranges (or spill block) of the item
+    __shared__ uint32_t s_blocks;                        // blocks of the item
+    __shared__ uint32_t s_warp_sum[kAggThreads / 32];
     __shared__ uint64_t s_spill_first[kMaxSources + 1];  // work-item index of each source's first spill slice
 
-    const int lane = threadIdx.x & 31;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const TableView &tv = p.table;
 
     if (threadIdx.x == 0) {
@@ -242,45 +245,107 @@ __global__ void __launch_bounds__(kAggThreads, 1) aggregate_kernel(const AggPara
 
         if (item < (uint64_t)p.n_parts * p.groups) {
             // A partition of this rank's table: its fragments from every source and pass-A CTA
-            // (with groups > 1, one share of them).  Fill counts first, all at once; then the
-            // warps take fragments as they come free, always one block of hashes ahead.
+            // (with groups > 1, one share of them: fragments g, g + groups, ...).  Laid end to end,
+            // each padded to whole blocks of kBlk hashes, they are the item's blocks; the warps take
+            // them in that order, always one block ahead.  Only filled blocks are handed out: a fragment is planned for every window position of its share plus some
+            // margin (plan_partitioned) and is typically half full.
             const uint64_t dest = p.dest0 + item / p.groups;
             const uint32_t g = (uint32_t)(item % p.groups);
             const uint32_t n_frag = min(p.n_ctas * (uint32_t)p.n_src, kAggMaxFrags);
-            for (uint32_t f = threadIdx.x; f < n_frag; f += kAggThreads) {
-                const uint32_t s = f / p.n_ctas;
-                s_cnt[f] = min(__ldg(p.src[s].frag_cnt + dest * p.n_ctas + (f - s * p.n_ctas)), p.frag_cap);
+            const uint32_t n_mine = g < n_frag ? (n_frag - g + p.groups - 1) / p.groups : 0;
+            auto row_of = [&](uint32_t i, int &s) {  // fragment i of the item: its source and row
+                const uint32_t f = g + i * p.groups;
+                s = (int)(f / p.n_ctas);
+                return dest * p.n_ctas + (f - (uint32_t)s * p.n_ctas);
+            };
+            // s_end[i] = where fragment i's hashes end in the item's blocks: kBlk x (blocks of the
+            // fragments before it) + its fill count.  A scan over contiguous runs of fragments per
+            // thread.  (Below 2^32: a partition's fragments from all sources hold at most half of
+            // what one source's do, under 2^31 entries -- plan_partitioned -- and padding adds < kBlk
+            // per fragment.)
+            const uint32_t per = (n_mine + kAggThreads - 1) / kAggThreads;
+            const uint32_t i0 = min(threadIdx.x * per, n_mine), i1 = min(i0 + per, n_mine);
+            uint32_t mine = 0;
+            for (uint32_t i = i0; i < i1; ++i) {
+                int s;
+                const uint64_t row = row_of(i, s);
+                const uint32_t fill = min(__ldg(p.src[s].frag_cnt + row), p.frag_cap);
+                s_end[i] = fill;
+                mine += (fill + kBlk - 1) / kBlk * kBlk;
+            }
+            uint32_t before = mine;
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t y = __shfl_up_sync(0xffffffffu, before, o);
+                if (lane >= o) before += y;
+            }
+            if (lane == 31) s_warp_sum[warp] = before;
+            before -= mine;
+            __syncthreads();
+            if (warp == 0) {
+                const uint32_t v = lane < kAggThreads / 32 ? s_warp_sum[lane] : 0u;
+                uint32_t x = v;
+                for (int o = 1; o < 32; o <<= 1) {
+                    const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
+                    if (lane >= o) x += y;
+                }
+                if (lane < kAggThreads / 32) s_warp_sum[lane] = x - v;
+                if (lane == 31) s_blocks = x / kBlk;
             }
             __syncthreads();
-            // Work inside the item: whole fragments per warp when the item has plenty (eight per warp
-            // or more: the warps stay level anyway, and a warp streams its fragment front to back);
-            // else in blocks of kBlk hashes, block b of every fragment of the item before block b + 1
-            // of any -- a load is still 1 KB in one piece, and no warp idles however few fragments
-            // there are (with two fragments per item, 22 of 24 warps had nothing to do).
-            const uint32_t n_mine = g < n_frag ? (n_frag - g + p.groups - 1) / p.groups : 0;  // fragments g, g + groups, ...
-            const bool by_block = n_mine < 8u * (kAggThreads / 32);
-            const uint32_t n_units = by_block ? n_mine * ((p.frag_cap + kBlk - 1) / kBlk) : n_mine;
-            const uint64_t *cur = nullptr;  // (whole fragments) rest of the fragment in hand
-            uint32_t left = 0;
-            auto next_blk = [&](const uint64_t *&ptr, uint32_t &n) {  // warp-uniform; n = 0: nothing left
-                for (;;) {
-                    if (left) {
-                        ptr = cur; n = min(left, kBlk);
-                        cur += n; left -= n;
-                        return;
-                    }
-                    uint32_t u = 0;
-                    if (lane == 0) u = atomicAdd(&s_next, 1u);
-                    u = __shfl_sync(0xffffffffu, u, 0);
-                    if (u >= n_units) { n = 0; return; }
-                    const uint32_t b = by_block ? u / n_mine : 0u, f = g + (u - b * n_mine) * p.groups;
-                    const uint32_t have = s_cnt[f];
-                    if (b * kBlk >= have) continue;
-                    const uint32_t s = f / p.n_ctas;
-                    const uint64_t *at = p.src[s].frag + (dest * p.n_ctas + (f - s * p.n_ctas)) * p.frag_cap + b * kBlk;
-                    if (by_block) { ptr = at; n = min(have - b * kBlk, kBlk); return; }
-                    cur = at; left = have;
+            before += s_warp_sum[warp];
+            for (uint32_t i = i0; i < i1; ++i) {
+                const uint32_t fill = s_end[i];
+                s_end[i] = before + fill;
+                before += (fill + kBlk - 1) / kBlk * kBlk;
+            }
+            __syncthreads();
+            const uint32_t n_blocks = s_blocks;
+            // the fragment holding block blk: the first i with s_end[i] > blk * kBlk (the empty fragments
+            // before it end where it starts), 32 candidates per step
+            auto frag_of = [&](uint32_t blk) {
+                const uint32_t x = blk * kBlk;
+                uint32_t lo = 0, hi = n_mine - 1;  // it is in [lo, hi]
+                while (lo < hi) {
+                    const uint32_t step = (hi - lo + 32) / 32, at = lo + lane * step + step - 1;
+                    lo += step * __popc(__ballot_sync(0xffffffffu, at < hi && s_end[at] <= x));
+                    hi = min(hi, lo + step - 1);
                 }
+                return lo;
+            };
+            // The first seven eighths of the blocks are split evenly among the warps up front, one
+            // contiguous range each; the rest is handed out in runs of a warp's share of what is left
+            // (so that the last runs are short and the warps finish level).  A warp streams each
+            // fragment of a range or run front to back.  Measured per step: runs from the first block
+            // on took 8.42 ms of pass B on C2 against 8.11 (one block per run: 9.85), ranges over all
+            // blocks 35.62 ms on C3-shaped input, whose small items of the cache-less variant need the
+            // level finish, against 34.94.
+            const uint32_t n_ranged = n_blocks - n_blocks / 8;
+            uint32_t b = (uint32_t)((uint64_t)warp * n_ranged / (kAggThreads / 32));                // next block
+            uint32_t b_end = (uint32_t)((uint64_t)(warp + 1) * n_ranged / (kAggThreads / 32));      // end of the range or run
+            uint32_t left = 0;  // hashes of the fragment in hand, up to b_end
+            const uint64_t *cur = nullptr;
+            auto next_blk = [&](const uint64_t *&ptr, uint32_t &n) {  // warp-uniform; n = 0: nothing left
+                if (!left) {
+                    if (b >= b_end) {
+                        uint32_t t = 0, run = 0;
+                        if (lane == 0) {
+                            const uint32_t seen = *(volatile uint32_t *)&s_next;
+                            run = max(1u, (n_blocks - n_ranged - min(seen, n_blocks - n_ranged)) / (kAggThreads / 32));
+                            t = n_ranged + atomicAdd(&s_next, run);
+                        }
+                        b = __shfl_sync(0xffffffffu, t, 0);
+                        if (b >= n_blocks) { n = 0; return; }
+                        b_end = min(b + __shfl_sync(0xffffffffu, run, 0), n_blocks);
+                    }
+                    const uint32_t j = frag_of(b);
+                    const uint32_t first = j ? (s_end[j - 1] + kBlk - 1) / kBlk * kBlk : 0u;  // fragment j's first block, x kBlk
+                    int s;
+                    const uint64_t row = row_of(j, s);
+                    cur = p.src[s].frag + row * p.frag_cap + (b * kBlk - first);
+                    left = min(s_end[j], b_end * kBlk) - b * kBlk;
+                }
+                ptr = cur; n = min(left, kBlk);
+                cur += n; left -= n; ++b;
             };
             const uint64_t *ptr = nullptr, *ptr2 = nullptr;
             uint32_t n = 0, n2 = 0;

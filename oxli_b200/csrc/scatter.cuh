@@ -37,21 +37,22 @@
 
 namespace oxg {
 
-// Two CTAs of 12 warps per SM rather than one of 24.  One CTA of 24 warps sorts twice the batch
-// (18432 hashes) per set of barriers and ran pass A 1 ms faster on C2 (18.7 against 19.7 ms per
-// step, one B200) -- but it halves the pass A grid, i.e. the fragments of a partition, and pass B
-// then took 9.6 instead of 8.1 ms: the C2 step was 28.6 ms against 28.0 (DESIGN.md 4.3).
+// One CTA of 24 warps per SM rather than two of 12: it sorts twice the batch (18432 hashes) per set
+// of barriers, and pass A takes 18.8 instead of 19.7 ms per C2 step and 23.0 instead of 25.2 per
+// C3-shaped step (one B200).  It halves the pass A grid, i.e. the fragments of a partition (148),
+// each twice as long; pass B splits a partition's filled blocks among its warps rather than whole
+// fragments, so that it does not lose what pass A gains (DESIGN.md 4.3).
 #ifndef OXG_SCAT_THREADS
-#define OXG_SCAT_THREADS 384
+#define OXG_SCAT_THREADS 768
 #endif
 #ifndef OXG_SCAT_CTAS
-#define OXG_SCAT_CTAS 2
+#define OXG_SCAT_CTAS 1
 #endif
 constexpr int kScatThreads = OXG_SCAT_THREADS;
 constexpr int kScatCtasPerSm = OXG_SCAT_CTAS;
 constexpr int kScatWarps = kScatThreads / 32;
 // Warp tiles per warp and batch, at most: step 3 holds a warp's whole slice in registers, 8 hashes
-// per lane and tile, and 80 registers per thread (two CTAs of 384 or one of 768 per SM) leave room
+// per lane and tile, and 80 registers per thread (one CTA of 768 or two of 384 per SM) leave room
 // for three tiles' 24 hashes and no more.
 constexpr int kScatMaxBatchTiles = 3;
 static_assert(kScatWarps * 256 >= 2048, "step 2 scans 256 destinations per warp, up to 2048 of them");
